@@ -22,6 +22,13 @@ block 1024, strong scaling over the ranks), --workload c5 = configs[4] (256 x 2^
 
 Launch: `python bench.py --gpus 1` or, for N > 1, under torchrun (one rank per GPU, streams sharded by rank,
 no data-path collective; torch.distributed is used only for the barrier and the max-over-ranks time).
+
+--dump-outputs DIR writes what the last timed step computed as float32 .npy files, so that two builds run with the same
+arguments (same seeded inputs) can be compared output for output: c3 / c4 block_output.npy [streams, B], the output block
+of every stream or, past 48 MB, of a fixed seeded sample of streams in ascending order; c5 impulse_responses.npy
+[captures, 2^20] (impulse_responses_rank<r>.npy per rank, the 48 MB split between the ranks, so at most 12 ranks), likewise
+sampled by capture.  Under the c3 capacity ladder the sample is drawn from every stream held resident and keeps those
+that ran, so on one GPU two runs whose ladders stopped at different counts share the leading rows.
 """
 import argparse
 import json
@@ -67,7 +74,12 @@ def parse():
     ap.add_argument("--captures", type=int, default=256, help="c5: captures per batch (per GPU)")
     ap.add_argument("--smoothing", action="store_true", help="c5: with the plug-in's default 3 x 1/13-octave smoothing (not the headline c5 line)")
     ap.add_argument("--sample-ms", type=float, default=20.0, help="period of the NVML clock / power sampler during the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32, at most 48 MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times the CPU code and keeps no outputs")
     if a.workload == "c4":
         a.block, a.ir_seconds = 1024, 10.0
     return a
@@ -190,6 +202,23 @@ def measured_peak_gbs():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_BYTES = 48 << 20
+
+
+def dump_rows(n_rows, row_bytes, budget=DUMP_BYTES):
+    """Indices of the rows (streams or captures) --dump-outputs writes: all of them when they fit the budget, else a fixed
+    seeded sample, ascending."""
+    if n_rows * row_bytes <= budget:
+        return np.arange(n_rows)
+    return np.sort(np.random.default_rng(0).choice(n_rows, budget // row_bytes, replace=False))
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
 
 def workload(args):
@@ -476,6 +505,12 @@ def run_b200(args):
             return R.max(np.percentile(sm_, 99)), R.max(np.percentile(sm_, 50))
         S, ladder_log, ladder_failed = capacity_search(p99_at, S_alloc, period_ms, args.ladder_steps)
         e.set_active_channels(S)
+        # the rungs leave each stream's history and the input cycle wherever the search stopped: start again from silence
+        # and refill the FDL, so that the timed steps compute the same outputs on every run with these arguments
+        e.reset()
+        counter[0] = 0
+        for _ in range(P):
+            step()
     for _ in range(3):
         step()
 
@@ -504,6 +539,13 @@ def run_b200(args):
     # cross-rank data movement of the whole job)
     total_streams = args.streams_total if per_stream_ir else world * S
     gathered = sharding.gather_streams(d_out[:S].cpu().numpy(), total_streams, device="cuda")
+    if args.dump_outputs and rank == 0:
+        if ladder:                                     # stream c of rank r is row r*S + c of the gather when it ran (c < S)
+            r, c = np.divmod(dump_rows(world * S_alloc, B * 4), S_alloc)
+            rows = (r * S + c)[c < S]
+        else:
+            rows = dump_rows(total_streams, B * 4)
+        write_outputs(args.dump_outputs, {"block_output": gathered[rows]})
     throughput_channels = total_streams * B / (ms_per_step * 1e-3) / SR
     lat = percentiles(step_ms, period_ms)
     lat["p99_ms"] = R.max(lat["p99_ms"])
@@ -755,6 +797,8 @@ def run_c5(args, R, eng):
     from irbaboon_b200 import synth
     torch = R.torch
     n, nb = 1 << 20, args.captures
+    if args.dump_outputs and DUMP_BYTES // R.world < n * 4:
+        raise SystemExit("bench.py: --dump-outputs fits one 2^20-sample capture per rank for at most %d ranks" % (DUMP_BYTES // (n * 4)))
     eng.set_device(R.local)
     sweep, base = c5_inputs(4)
     caps = eng.pinned_empty((nb, n))
@@ -781,6 +825,9 @@ def run_c5(args, R, eng):
     clocks = sampler.summary() if R.rank == 0 else None
     sampler.stop()
     res_dev = d_res.cpu().numpy()
+    if args.dump_outputs:                                  # every rank deconvolves its own batch
+        rows = dump_rows(nb, n * 4, DUMP_BYTES // R.world)
+        write_outputs(args.dump_outputs, {"impulse_responses" + ("_rank%d" % R.rank if R.world > 1 else ""): res_dev[rows]})
     for _ in range(2):                                     # e2e: pinned host captures in, pinned host IRs out
         eng.deconvolve_batch(caps, sweep, SR, args.smoothing, out=res)
     R.barrier()

@@ -1,5 +1,6 @@
-"""CPU: the parts of bench.py's contract that do not need a GPU -- the reference arm prints ONE JSON line with the
-agreed keys, and the product arm refuses to run without a CUDA device (no CPU fallback)."""
+"""bench.py's contract.  CPU: the reference arm prints ONE JSON line with the agreed keys, the product arm refuses to run
+without a CUDA device (no CPU fallback), arguments are checked and --dump-outputs samples a fixed set of rows.  GPU: the
+dumped outputs repeat from run to run."""
 import json
 import os
 import subprocess
@@ -91,6 +92,45 @@ def test_capacity_ladder_never_aborts():
     p99_at, calls = _fake_gpu(4.0e-4, 0.0)                                 # a GPU four times slower: jumps to the estimate, then verifies
     S, log, failed = b.capacity_search(p99_at, 98304, period, 300)
     assert not failed and 22528 <= S <= 26624 and len(calls) <= 6
+
+
+def test_bench_rejects_zero_steps_and_dumps_from_the_reference_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert p.returncode == 2 and "error:" in p.stderr, (extra, p.stderr[-2000:])
+
+
+def test_dump_rows_fixed_sample_within_budget():
+    import numpy as np
+    b = _bench_module()
+    assert np.array_equal(b.dump_rows(8192, 4096), np.arange(8192))                     # c4 at one GPU: 32 MB, every stream
+    rows = b.dump_rows(98304, 2048)
+    assert len(rows) * 2048 <= b.DUMP_BYTES < 64 << 20 and len(rows) == b.DUMP_BYTES // 2048
+    assert np.all(np.diff(rows) > 0) and rows[-1] < 98304 and np.array_equal(rows, b.dump_rows(98304, 2048))
+    # the capacity ladder keeps the sampled streams below the count it stopped at: two stops share the leading rows
+    a, c = rows[rows < 94208], rows[rows < 92160]
+    assert np.array_equal(a[:len(c)], c)
+    assert len(b.dump_rows(256, 4 << 20)) == 12                                             # c5: 12 of 256 captures
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_repeat_across_runs(tmp_path):
+    """Two runs with the same arguments, capacity ladder included, time exactly --steps block steps and dump the same outputs."""
+    import numpy as np
+    args = ["--steps", "5", "--warmup", "2", "--streams-max", "4096", "--ladder-steps", "20", "--no-cpu-baseline", "--no-e2e", "--no-selfcheck"]
+    outs = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args + ["--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert p.returncode == 0, p.stderr[-2000:]
+        line = json.loads(p.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 5 and line["gpu_launches"] == 5
+        y = np.load(d / "block_output.npy")
+        assert y.dtype == np.float32 and y.shape == (line["config"]["streams_per_gpu"], 512)
+        outs.append(y)
+    n = min(len(outs[0]), len(outs[1]))
+    assert n >= 2048 and np.isfinite(outs[0]).all() and np.abs(outs[0]).max() > 0
+    assert np.array_equal(outs[0][:n], outs[1][:n])
 
 
 def test_clock_sampler_degrades_without_a_gpu():
