@@ -140,6 +140,20 @@ size_t irb_release_workspace(void);
 /* device time (CUDA events, ms) of the kernels of the calling thread's most recent offline call
  * (irb_convolve_periodic / _nonperiodic / irb_deconvolve*), host<->device copies excluded */
 double irb_last_compute_ms(void);
+/* ---- IR matrix engine ---------------------------------------------------------------------------------
+ * n_groups groups of `ins` consecutive input channels, each producing `outs` consecutive output channels:
+ *   out[g*outs + o] = sum_i conv(in[g*ins + i], IR ir_ids[i*outs + o])
+ * Supported (ins, outs): (1, 2) mono -> stereo, (2, 2) true stereo (IRs LL, LR, RL, RR).  Block sizes whose FFT half size is
+ * 256..1024 (129 <= block_size <= 1024).  Each input channel keeps ONE FDL ring (advanced once per block, read once per block
+ * step for all the IRs it feeds); each output channel keeps its overlap.  n_irs >= ins*outs; until bound, every group uses
+ * ir_ids = {0, 1, ..., ins*outs-1}.  For (1, 2) output o is bit-identical to a plain engine channel bound to ir_ids[o].
+ * in: [n_blocks][n_groups*ins][block_size], out: [n_blocks][n_groups*outs][block_size].
+ * The other irb_engine_* calls keep their meaning on a matrix engine (read_fdl_spectrum: `chan` is an input channel;
+ * mac_plan: slots_kernel = 1 when some kernel unit mixes matrices and every group stages its own IR partitions), except
+ * irb_engine_bind, _process_callback, _set_active_channels, _set_mac_split and _set_fused_step(0): IRB_ERR_STATE. */
+int irb_engine_create_matrix(irb_engine** out, int device, int block_size, int max_partitions, int n_groups, int ins, int outs, int n_irs);
+int irb_engine_bind_matrix(irb_engine* e, int group_begin, int group_end, const int* ir_ids /* [ins*outs] */);
+
 /* ---- several GPUs from one process ---------------------------------------------------------------------
  * Streams never interact (fp/convolution.cpp:160-215 has no cross-channel term), so n_channels are cut into contiguous
  * ranges of whole kernel tiles, one irb_engine per device.  n_irs > 0: shared IRs, replicated on every device, bound with

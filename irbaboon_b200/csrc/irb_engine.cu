@@ -16,6 +16,7 @@
 #include "irb_common.hpp"
 #include "irb_kernels.cuh"
 #include "irb_mac_p.cuh"
+#include "irb_mac_mx.cuh"
 #include "irb_tuning.hpp"
 
 namespace irbh {
@@ -207,6 +208,51 @@ int launch_mac_p(irb::MacArgs a, int num_sms, cudaStream_t st) {
     CK(cudaGetLastError());
     return 0;
 }
+// the IR-matrix block step (irb_mac_mx.cuh): a.n_rows output rows, units of whole groups, one launch
+template <int M, int INS, int OUTS, bool PG>
+int launch_mac_mx_t(irb::MacArgs a, int num_sms, cudaStream_t st) {
+    using C = irb::MxCfg<M, INS, OUTS, PG>;
+    if (a.n_rows <= 0) return 0;
+    if (!a.work) return fail(IRB_ERR_STATE, "matrix block step without a work counter");
+    const int ctas = persistent_ctas_per_sm() * num_sms;
+    const int n_groups = a.n_rows / OUTS;
+    a.unit_n[0] = (n_groups + C::GROUPS - 1) / C::GROUPS; a.unit_n[1] = a.unit_n[2] = a.unit_n[3] = 0;
+    const int grid = std::min(a.unit_n[0], ctas);
+    const size_t smem = sizeof(irb::MxSmem<M, INS, OUTS, PG>);
+    static thread_local int configured_dev = -1;
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    if (configured_dev != dev) {
+        CK(cudaFuncSetAttribute(irb::k_mac_mx<M, INS, OUTS, PG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+        CK(cudaFuncSetAttribute(irb::k_mac_mx<M, INS, OUTS, PG>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        int resident = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, irb::k_mac_mx<M, INS, OUTS, PG>, irb::kThreads + 32, smem));
+        if (resident < 2) return fail(IRB_ERR_CUDA, "k_mac_mx<%d, %d, %d>: only %d CTA per SM fits (registers / shared memory), 2 expected", M, INS, OUTS, resident);
+        configured_dev = dev;
+    }
+    irb::k_mac_mx<M, INS, OUTS, PG><<<grid, irb::kThreads + 32, smem, st>>>(a);
+    g_launches++;
+    CK(cudaGetLastError());
+    return 0;
+}
+template <int M, int INS, int OUTS>
+int launch_mac_mx_pg(const irb::MacArgs& a, bool pergroup, int num_sms, cudaStream_t st) {
+    return pergroup ? launch_mac_mx_t<M, INS, OUTS, true>(a, num_sms, st) : launch_mac_mx_t<M, INS, OUTS, false>(a, num_sms, st);
+}
+template <int M>
+int launch_mac_mx_m(const irb::MacArgs& a, int ins, int outs, bool pergroup, int num_sms, cudaStream_t st) {
+    if (ins == 1 && outs == 2) return launch_mac_mx_pg<M, 1, 2>(a, pergroup, num_sms, st);
+    if (ins == 2 && outs == 2) return launch_mac_mx_pg<M, 2, 2>(a, pergroup, num_sms, st);
+    return fail(IRB_ERR_ARG, "unsupported IR matrix %d x %d", ins, outs);
+}
+int launch_mac_mx(int M, int ins, int outs, bool pergroup, int num_sms, const irb::MacArgs& a, cudaStream_t st) {
+    switch (M) {
+        case 256: return launch_mac_mx_m<256>(a, ins, outs, pergroup, num_sms, st);
+        case 512: return launch_mac_mx_m<512>(a, ins, outs, pergroup, num_sms, st);
+        case 1024: return launch_mac_mx_m<1024>(a, ins, outs, pergroup, num_sms, st);
+        default: return fail(IRB_ERR_ARG, "the matrix engine takes FFT half sizes 256 .. 1024, not %d", M);
+    }
+}
 template <int M>
 int launch_mac_tma(const irb::MacArgs& a, cudaStream_t st) {
     const int grid = (a.n_rows + irb::Tile<M>::ROWS - 1) / irb::Tile<M>::ROWS;
@@ -329,6 +375,15 @@ int tile_rows(int M) { return irb::kTile / M; }
 struct irb_engine {
     int device = 0, B = 0, M = 0, ring = 0, n_chans = 0, n_irs = 0;
     int active = 0;                    // channels [0, active) take part in a block step (irb_engine_set_active_channels); I/O arrays are dense over them
+    // IR-matrix engine (irb_engine_create_matrix): groups of `ins` input channels producing `outs` output channels each.  The
+    // channels above (n_chans, active, FDL rows, heads) are the INPUTS; ov and the output staging hold n_chans / ins * outs
+    // rows; h_ir_of_chan / ir_of_chan hold the matrix table [group][ins * outs]; per_row_ir means "some unit mixes matrices".
+    // A plain engine is the 1 x 1 case.
+    int ins = 1, outs = 1;
+    bool matrix() const { return ins != 1 || outs != 1; }
+    int out_chans() const { return active / ins * outs; }
+    size_t in_blk() const { return (size_t) B * active; }
+    size_t out_blk() const { return (size_t) B * out_chans(); }
     // FDL layout [chan / fdl_group][slot][chan % fdl_group][M], fdl_group = channels per kernel tile (irb_kernels.cuh, MacArgs)
     int fdl_group = 1;
     long long fdl_group_stride() const { return (long long) ring * fdl_group * M; }
@@ -412,6 +467,22 @@ namespace {
 int floor_pow2(long long x) { int r = 1; while (2LL * r <= x) r *= 2; return r; }
 
 int engine_check_binding(irb_engine* e) {
+    if (e->matrix()) {
+        // one launch of k_mac_mx per step, no partition split; PERGROUP when some unit's groups are bound to different matrices
+        if (e->binding_dirty) {
+            const int terms = e->ins * e->outs, n_groups = e->n_chans / e->ins;
+            const int per_unit = tile_rows(e->M) / e->outs;
+            e->per_row_ir = false;
+            for (int g = 0; g < n_groups && !e->per_row_ir; ++g)
+                if (g % per_unit && !std::equal(e->h_ir_of_chan.begin() + (size_t) g * terms, e->h_ir_of_chan.begin() + (size_t) (g + 1) * terms,
+                                                e->h_ir_of_chan.begin() + (size_t) (g - g % per_unit) * terms)) e->per_row_ir = true;
+            CK(cudaMemcpyAsync(e->ir_of_chan.p, e->h_ir_of_chan.data(), sizeof(int) * e->h_ir_of_chan.size(), cudaMemcpyHostToDevice, e->stream));
+            CK(cudaStreamSynchronize(e->stream));
+            e->binding_dirty = false;
+        }
+        e->split_in = 1; e->cluster_dim = 1; e->plan_dirty = false;
+        return 0;
+    }
     if (e->binding_dirty) {
         const int rows = tile_rows(e->M);
         e->per_row_ir = false;
@@ -471,6 +542,7 @@ bool use_slots(const irb_engine* e) { return e->per_row_ir || e->split_in > 1 ||
 // Is the block step ONE launch (forward transform in the MAC kernel's prologue)?  Shared-IR tiles: always (unless switched off);
 // per-stream IRs: through the persistent kernel; few rows (partitions split over slots / a cluster): in the cluster kernel.
 bool step_is_fused(const irb_engine* e) {
+    if (e->matrix()) return true;                   // k_mac_mx always transforms the new blocks itself
     if (!e->fuse_fwd) return false;
     if (e->split_in > 1 || e->cluster_dim > 1) return irbh::g_tuning.fuse_split != 0;      // the cluster kernel's rank 0 transforms the new blocks itself
     if (e->per_row_ir) return irbh::g_tuning.mac_persistent && e->M >= kPersistMinM;
@@ -503,8 +575,22 @@ int engine_launch_fwd(irb_engine* e, const float* in_dev, bool audio, bool refre
     e->launches += 1;
     return 0;
 }
+// the IR-matrix block step over every group: inputs in_dev [n_chans][B], outputs out_dev [n_chans / ins * outs][B]
+int engine_launch_mx(irb_engine* e, float* out_dev, const float* in_dev) {
+    irb::MacArgs m{};
+    fill_mac_args(e, m, 0, e->n_chans);
+    m.n_rows = e->out_chans(); m.work = e->work.as<int>();
+    m.Y = nullptr; m.out = out_dev; m.out_chan_stride = e->B; m.Lout = e->B;
+    m.ov = e->ov.as<float>(); m.tail = nullptr; m.head_back = 0;
+    m.in = in_dev; m.in_chan_stride = e->B; m.head_rw = e->head.as<int>();
+    int rc = launch_mac_mx(e->M, e->ins, e->outs, e->per_row_ir, e->num_sms, m, e->stream);
+    if (rc) return rc;
+    e->launches += 1;
+    return 0;
+}
 // in_dev != nullptr: the forward transform of that block runs inside the MAC kernel (shared-IR kernel only)
 int engine_launch_mac(irb_engine* e, float* out_dev, int head_back, const float* in_dev, int c0, int cn) {
+    if (e->matrix()) return engine_launch_mx(e, out_dev, in_dev);
     irb::MacArgs m{};
     fill_mac_args(e, m, c0, cn);
     m.Y = nullptr; m.out = out_dev + (size_t) c0 * e->B; m.out_chan_stride = e->B; m.Lout = e->B;
@@ -574,20 +660,22 @@ long long irb_launch_count(void) { return g_launches.load(); }
 size_t irb_release_workspace(void) { return irbh::pool_release(); }
 double irb_last_compute_ms(void) { return irbh::g_last_compute_ms; }
 
-int irb_engine_create(irb_engine** out, int device, int block_size, int max_partitions, int n_channels, int n_irs) {
-    if (!out) return fail(IRB_ERR_ARG, "out is null");
-    *out = nullptr;
-    if (block_size < 1 || half_size_for_block(block_size) > kMaxM) return fail(IRB_ERR_ARG, "block_size %d outside [1, %d]", block_size, kMaxM);
-    if (max_partitions < 1 || n_channels < 1 || n_irs < 1) return fail(IRB_ERR_ARG, "max_partitions, n_channels and n_irs must be >= 1");
+}  // extern "C"
+namespace {
+// n_channels INPUT channels; a matrix engine (ins x outs != 1 x 1) has n_channels / ins groups and n_channels / ins * outs outputs
+int engine_create(irb_engine** out, int device, int block_size, int max_partitions, int n_channels, int n_irs, int ins, int outs) {
     CK(cudaSetDevice(device));
     irb_engine* e = new (std::nothrow) irb_engine;
     if (!e) return fail(IRB_ERR_ARG, "out of host memory");
     e->device = device; e->B = block_size; e->M = half_size_for_block(block_size);
     e->ring = max_partitions; e->n_chans = n_channels; e->active = n_channels; e->n_irs = n_irs;
+    e->ins = ins; e->outs = outs;
+    const int n_out = n_channels / ins * outs, n_table = n_channels / ins * ins * outs;     // output rows; ir_of_chan entries
     int rc = irbh::twiddles(device, e->M, &e->W);
     if (rc) { delete e; return rc; }
     const size_t spec = sizeof(float2) * (size_t) e->M;
-    e->fdl_group = irbh::g_tuning.fdl_plain ? 1 : tile_rows(e->M);     // A/B: [chan][slot][M] instead of the tile-interleaved layout
+    // A/B: [chan][slot][M] instead of the tile-interleaved layout.  A matrix engine interleaves the input rows of one unit of its kernel.
+    e->fdl_group = irbh::g_tuning.fdl_plain ? 1 : (e->matrix() ? tile_rows(e->M) / outs * ins : tile_rows(e->M));
     // shared IR spectra in several identical copies (MacArgs::h_reps): as many as fit 24 MB, at most 32; one when the IRs are many
     {
         const size_t one = spec * e->ring * n_irs;
@@ -595,10 +683,11 @@ int irb_engine_create(irb_engine** out, int device, int block_size, int max_part
         e->h_reps = pref > 0 ? std::min(pref, 64) : (int) std::max<size_t>(1, std::min<size_t>(32, (24u << 20) / one));
     }
     const size_t b_fdl = e->fdl_bytes(), b_H = spec * e->ring * n_irs * e->h_reps, b_io = sizeof(float) * (size_t) e->B * n_channels;
-    if ((rc = e->fdl.alloc(b_fdl, true)) || (rc = e->H.alloc(b_H, true)) || (rc = e->ov.alloc(b_io, true)) ||
-        (rc = e->head.alloc(sizeof(int) * n_channels, false)) || (rc = e->ir_of_chan.alloc(sizeof(int) * n_channels, true)) ||
-        (rc = e->nparts.alloc(sizeof(int) * n_irs, true)) || (rc = e->io_in[0].alloc(b_io, true)) || (rc = e->io_out[0].alloc(b_io, true)) ||
-        (rc = e->io_in[1].alloc(b_io, true)) || (rc = e->io_out[1].alloc(b_io, true)) ||
+    const size_t b_oo = sizeof(float) * (size_t) e->B * n_out;
+    if ((rc = e->fdl.alloc(b_fdl, true)) || (rc = e->H.alloc(b_H, true)) || (rc = e->ov.alloc(b_oo, true)) ||
+        (rc = e->head.alloc(sizeof(int) * n_channels, false)) || (rc = e->ir_of_chan.alloc(sizeof(int) * n_table, true)) ||
+        (rc = e->nparts.alloc(sizeof(int) * n_irs, true)) || (rc = e->io_in[0].alloc(b_io, true)) || (rc = e->io_out[0].alloc(b_oo, true)) ||
+        (rc = e->io_in[1].alloc(b_io, true)) || (rc = e->io_out[1].alloc(b_oo, true)) ||
         (rc = e->taps.alloc(sizeof(float) * 2 * (size_t) e->B * e->ring, true)) || (rc = e->rr_ptrs.alloc(sizeof(float*) * n_irs, true)) ||
         (rc = e->rr_pos.alloc(sizeof(int) * n_irs, true)) || (rc = e->rr_list.alloc(sizeof(int) * n_irs, true)) || (rc = e->work.alloc(sizeof(int) * 4, true))) {
         delete e;
@@ -606,8 +695,9 @@ int irb_engine_create(irb_engine** out, int device, int block_size, int max_part
     }
     e->rr_buf.resize(n_irs);
     if (cudaDeviceGetAttribute(&e->num_sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || e->num_sms < 1) { cudaGetLastError(); e->num_sms = 148; }
-    e->bytes = b_fdl + b_H + 5 * b_io + sizeof(int) * (2 * (size_t) n_channels + 3 * (size_t) n_irs) + sizeof(float*) * n_irs + sizeof(float) * 2 * (size_t) e->B * e->ring;
-    e->h_ir_of_chan.assign(n_channels, 0);
+    e->bytes = b_fdl + b_H + 2 * b_io + 3 * b_oo + sizeof(int) * ((size_t) n_channels + n_table + 3 * (size_t) n_irs) + sizeof(float*) * n_irs + sizeof(float) * 2 * (size_t) e->B * e->ring;
+    e->h_ir_of_chan.assign(n_table, 0);
+    for (int i = 0; i < n_table; ++i) e->h_ir_of_chan[i] = i % (ins * outs);        // matrix: every group starts on IRs 0 .. ins*outs-1
     e->h_nparts.assign(n_irs, 0);
     bool ok = cudaStreamCreateWithFlags(&e->own_stream, cudaStreamNonBlocking) == cudaSuccess &&
               cudaStreamCreateWithFlags(&e->s_in, cudaStreamNonBlocking) == cudaSuccess &&
@@ -620,6 +710,40 @@ int irb_engine_create(irb_engine** out, int device, int block_size, int max_part
     e->stream = e->own_stream;
     *out = e;
     return irb_engine_reset(e);
+}
+}  // namespace
+extern "C" {
+
+int irb_engine_create(irb_engine** out, int device, int block_size, int max_partitions, int n_channels, int n_irs) {
+    if (!out) return fail(IRB_ERR_ARG, "out is null");
+    *out = nullptr;
+    if (block_size < 1 || half_size_for_block(block_size) > kMaxM) return fail(IRB_ERR_ARG, "block_size %d outside [1, %d]", block_size, kMaxM);
+    if (max_partitions < 1 || n_channels < 1 || n_irs < 1) return fail(IRB_ERR_ARG, "max_partitions, n_channels and n_irs must be >= 1");
+    return engine_create(out, device, block_size, max_partitions, n_channels, n_irs, 1, 1);
+}
+
+int irb_engine_create_matrix(irb_engine** out, int device, int block_size, int max_partitions, int n_groups, int ins, int outs, int n_irs) {
+    if (!out) return fail(IRB_ERR_ARG, "out is null");
+    *out = nullptr;
+    if (!((ins == 1 && outs == 2) || (ins == 2 && outs == 2))) return fail(IRB_ERR_ARG, "IR matrix %d x %d: only 1 x 2 (mono -> stereo) and 2 x 2 (true stereo) exist", ins, outs);
+    if (block_size < 129 || block_size > 1024) return fail(IRB_ERR_ARG, "block_size %d outside [129, 1024] (FFT half sizes 256 .. 1024)", block_size);
+    if (max_partitions < 1 || n_groups < 1) return fail(IRB_ERR_ARG, "max_partitions and n_groups must be >= 1");
+    if (n_irs < ins * outs) return fail(IRB_ERR_ARG, "n_irs %d is fewer than the %d IRs of one matrix", n_irs, ins * outs);
+    if ((long long) n_groups * (ins > outs ? ins : outs) > 0x7fffffffLL / 2048) return fail(IRB_ERR_ARG, "n_groups %d too large", n_groups);
+    return engine_create(out, device, block_size, max_partitions, n_groups * ins, n_irs, ins, outs);
+}
+
+int irb_engine_bind_matrix(irb_engine* e, int group_begin, int group_end, const int* ir_ids) {
+    if (!e || !ir_ids) return fail(IRB_ERR_ARG, "engine or ir_ids null");
+    if (!e->matrix()) return fail(IRB_ERR_STATE, "a plain engine binds channels: use irb_engine_bind");
+    const int n_groups = e->n_chans / e->ins, terms = e->ins * e->outs;
+    if (group_begin < 0 || group_end > n_groups || group_begin > group_end) return fail(IRB_ERR_ARG, "group range [%d, %d) outside [0, %d)", group_begin, group_end, n_groups);
+    for (int t = 0; t < terms; ++t)
+        if (ir_ids[t] < 0 || ir_ids[t] >= e->n_irs) return fail(IRB_ERR_ARG, "ir_ids[%d] = %d outside [0, %d)", t, ir_ids[t], e->n_irs);
+    for (int g = group_begin; g < group_end; ++g)
+        for (int t = 0; t < terms; ++t) e->h_ir_of_chan[(size_t) g * terms + t] = ir_ids[t];
+    e->binding_dirty = true;
+    return 0;
 }
 
 int irb_engine_destroy(irb_engine* e) {
@@ -643,7 +767,7 @@ int irb_engine_reset(irb_engine* e) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
     CK(cudaSetDevice(e->device));
     CK(cudaMemsetAsync(e->fdl.p, 0, e->fdl_bytes(), e->stream));
-    CK(cudaMemsetAsync(e->ov.p, 0, sizeof(float) * (size_t) e->B * e->n_chans, e->stream));
+    CK(cudaMemsetAsync(e->ov.p, 0, sizeof(float) * (size_t) e->B * (e->n_chans / e->ins * e->outs), e->stream));
     std::vector<int> h(e->n_chans, e->ring - 1);     // first block lands in slot 0
     CK(cudaMemcpyAsync(e->head.p, h.data(), sizeof(int) * e->n_chans, cudaMemcpyHostToDevice, e->stream));
     // staged IRs start over like irFftBufferArray.clearAndResize in prepareToPlay (PluginProcessor.cpp:226): spectra
@@ -741,6 +865,7 @@ int irb_engine_stage_ir(irb_engine* e, int ir_id, const float* left, const float
 
 int irb_engine_bind(irb_engine* e, int chan_begin, int chan_end, int ir_id) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
+    if (e->matrix()) return fail(IRB_ERR_STATE, "an IR-matrix engine binds whole groups: use irb_engine_bind_matrix");
     if (chan_begin < 0 || chan_end > e->n_chans || chan_begin > chan_end) return fail(IRB_ERR_ARG, "channel range [%d, %d) outside [0, %d)", chan_begin, chan_end, e->n_chans);
     if (ir_id < 0 || ir_id >= e->n_irs) return fail(IRB_ERR_ARG, "ir_id %d outside [0, %d)", ir_id, e->n_irs);
     for (int c = chan_begin; c < chan_end; ++c) e->h_ir_of_chan[c] = ir_id;
@@ -750,6 +875,7 @@ int irb_engine_bind(irb_engine* e, int chan_begin, int chan_end, int ir_id) {
 int irb_engine_tile_channels(const irb_engine* e) { return e ? tile_rows(e->M) : fail(IRB_ERR_ARG, "engine is null"); }
 int irb_engine_set_mac_split(irb_engine* e, int split_in, int cluster) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
+    if (e->matrix()) return fail(IRB_ERR_STATE, "an IR-matrix engine has no partition split: its block step is one k_mac_mx launch");
     if (split_in < 0 || cluster < 0 || (split_in == 0) != (cluster == 0)) return fail(IRB_ERR_ARG, "split_in and cluster must both be 0 (automatic) or both >= 1");
     e->force_split_in = split_in; e->force_cluster = cluster;
     e->plan_dirty = true;
@@ -757,6 +883,7 @@ int irb_engine_set_mac_split(irb_engine* e, int split_in, int cluster) {
 }
 int irb_engine_set_fused_step(irb_engine* e, int enable) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
+    if (e->matrix() && !enable) return fail(IRB_ERR_STATE, "an IR-matrix engine has no two-launch form: its block step always transforms the new blocks itself");
     e->fuse_fwd = enable != 0;
     return 0;
 }
@@ -777,9 +904,9 @@ int irb_engine_process_device(irb_engine* e, const float* in_dev, float* out_dev
     CK(cudaSetDevice(e->device));
     int rc = engine_check_binding(e);
     if (rc) return rc;
-    const size_t blk = (size_t) e->B * e->active;
+    const size_t iblk = e->in_blk(), oblk = e->out_blk();
     for (int b = 0; b < n_blocks; ++b)
-        if ((rc = engine_step_device(e, in_dev + b * blk, out_dev + b * blk))) return rc;
+        if ((rc = engine_step_device(e, in_dev + b * iblk, out_dev + b * oblk))) return rc;
     return 0;
 }
 
@@ -787,11 +914,12 @@ namespace {
 constexpr size_t kGraphMaxBytes = 256 << 10;         // blocks up to this size take the captured-graph path
 constexpr int kMaxGroups = 16;                       // channel groups a large single block is pipelined over
 
-// one block, host to host, as a single graph launch; *done = false when the caller should take the plain path instead
+// one block, host to host, as a single graph launch; *done = false when the caller should take the plain path instead.
+// Matrix engines take this path too: input and output staging are sized by their own channel counts.
 int engine_process_one_graphed(irb_engine* e, const float* in_host, float* out_host, bool* done) {
     *done = false;
-    const size_t bytes = sizeof(float) * (size_t) e->B * e->active;
-    if (irbh::g_tuning.no_graph || !e->use_graph || e->timing || bytes > kGraphMaxBytes) return 0;
+    const size_t bytes = sizeof(float) * e->in_blk(), obytes = sizeof(float) * e->out_blk();      // (differ on a matrix engine)
+    if (irbh::g_tuning.no_graph || !e->use_graph || e->timing || std::max(bytes, obytes) > kGraphMaxBytes) return 0;
     const irb_engine::GraphSig sig{(int) e->h_rr_list.size(), e->split_in, e->cluster_dim, use_slots(e) ? 1 : 0, e->fuse_fwd ? 1 : 0, e->active, tuning_variant(), e->stream};
     if (!(sig == e->g_sig)) {
         if (e->g_exec) { cudaGraphExecDestroy(e->g_exec); e->g_exec = nullptr; }
@@ -806,7 +934,7 @@ int engine_process_one_graphed(irb_engine* e, const float* in_host, float* out_h
         CK(cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeRelaxed));
         int rc = cudaMemcpyAsync(e->io_in[0].p, e->g_hin, bytes, cudaMemcpyHostToDevice, e->stream) == cudaSuccess ? 0 : IRB_ERR_CUDA;
         if (!rc) rc = engine_step_device(e, e->io_in[0].as<float>(), e->io_out[0].as<float>());
-        if (!rc && cudaMemcpyAsync(e->g_hout, e->io_out[0].p, bytes, cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) rc = IRB_ERR_CUDA;
+        if (!rc && cudaMemcpyAsync(e->g_hout, e->io_out[0].p, obytes, cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) rc = IRB_ERR_CUDA;
         const cudaError_t ce = cudaStreamEndCapture(e->stream, &graph);
         e->g_kernels = (int) (e->launches - l0);
         e->launches = l0;                                    // nothing ran yet
@@ -826,7 +954,7 @@ int engine_process_one_graphed(irb_engine* e, const float* in_host, float* out_h
     e->launches += e->g_kernels;
     g_launches += e->g_kernels;
     CK(cudaStreamSynchronize(e->stream));
-    memcpy(out_host, e->g_hout, bytes);
+    memcpy(out_host, e->g_hout, obytes);
     *done = true;
     return 0;
 }
@@ -834,7 +962,8 @@ int engine_process_one_graphed(irb_engine* e, const float* in_host, float* out_h
 
 namespace {
 // Host-buffer block steps: block b of this engine's channels starts at in_host + b*stride (stride == n_channels*B for a
-// dense array; larger when the engine owns a channel range of a wider array).  wait == false returns once everything
+// dense array; larger when the engine owns a channel range of a wider array) and out_host + b*out_stride (the output count
+// of a matrix engine differs from its input count).  wait == false returns once everything
 // is enqueued (engine_process_wait completes it) so that one host thread can keep several devices busy.
 int engine_process_wait(irb_engine* e) {
     CK(cudaSetDevice(e->device));
@@ -844,11 +973,11 @@ int engine_process_wait(irb_engine* e) {
     return 0;
 }
 
-int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host, int n_blocks, size_t stride, bool allow_graph) {
+int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host, int n_blocks, size_t stride, size_t out_stride, bool allow_graph) {
     CK(cudaSetDevice(e->device));
     int rc = engine_check_binding(e);
     if (rc) return rc;
-    const size_t blk = (size_t) e->B * e->active;
+    const size_t blk = e->in_blk(), oblk = e->out_blk();
     if (n_blocks == 1) {
         if (e->pipe_pending && (rc = engine_process_wait(e))) return rc;               // submitted blocks still own the staging slots
         // a live callback: one block in, one block out.  Small blocks replay a captured graph (one launch); larger ones
@@ -859,11 +988,12 @@ int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host,
         }
         const int rows = tile_rows(e->M);
         const int tiles = (e->active + rows - 1) / rows;
-        const int groups = (e->timing || sizeof(float) * blk < (4u << 20)) ? 1 : (int) std::min<long long>(kMaxGroups, tiles / (4LL * e->num_sms) > 0 ? tiles / (4LL * e->num_sms) : 1);
+        // (a matrix engine always takes the one-range form: its launch covers every group)
+        const int groups = (e->timing || e->matrix() || sizeof(float) * blk < (4u << 20)) ? 1 : (int) std::min<long long>(kMaxGroups, tiles / (4LL * e->num_sms) > 0 ? tiles / (4LL * e->num_sms) : 1);
         if (groups <= 1) {
             CK(cudaMemcpyAsync(e->io_in[0].p, in_host, sizeof(float) * blk, cudaMemcpyHostToDevice, e->stream));
             if ((rc = engine_step_device(e, e->io_in[0].as<float>(), e->io_out[0].as<float>()))) return rc;
-            CK(cudaMemcpyAsync(out_host, e->io_out[0].p, sizeof(float) * blk, cudaMemcpyDeviceToHost, e->stream));
+            CK(cudaMemcpyAsync(out_host, e->io_out[0].p, sizeof(float) * oblk, cudaMemcpyDeviceToHost, e->stream));
             return 0;
         }
         // A large block: cut the channels into groups of whole tiles and pipeline upload | kernels | download across the
@@ -900,7 +1030,7 @@ int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host,
         if ((rc = engine_step_device(e, e->io_in[q].as<float>(), e->io_out[q].as<float>()))) return rc;
         CK(cudaEventRecord(e->ev_done[q], e->stream));
         CK(cudaStreamWaitEvent(e->s_out, e->ev_done[q], 0));
-        CK(cudaMemcpyAsync(out_host + b * stride, e->io_out[q].p, sizeof(float) * blk, cudaMemcpyDeviceToHost, e->s_out));
+        CK(cudaMemcpyAsync(out_host + b * out_stride, e->io_out[q].p, sizeof(float) * oblk, cudaMemcpyDeviceToHost, e->s_out));
         CK(cudaEventRecord(e->ev_out[q], e->s_out));
     }
     e->pipe_pending = true;
@@ -913,6 +1043,7 @@ int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host,
 // n_active must be a whole number of kernel tiles (irb_engine_tile_channels()) or n_channels.
 int irb_engine_set_active_channels(irb_engine* e, int n_active) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
+    if (e->matrix()) return fail(IRB_ERR_STATE, "an IR-matrix engine always runs all its groups");
     if (n_active < 1 || n_active > e->n_chans) return fail(IRB_ERR_ARG, "n_active %d outside [1, %d]", n_active, e->n_chans);
     if (n_active != e->n_chans && n_active % tile_rows(e->M)) return fail(IRB_ERR_ARG, "n_active %d is not a multiple of the %d channels of a kernel tile", n_active, tile_rows(e->M));
     if (e->pipe_pending) { int rc = engine_process_wait(e); if (rc) return rc; }
@@ -925,7 +1056,7 @@ int irb_engine_active_channels(const irb_engine* e) { return e ? e->active : fai
 int irb_engine_process(irb_engine* e, const float* in_host, float* out_host, int n_blocks) {
     if (!e || !in_host || !out_host) return fail(IRB_ERR_ARG, "null argument");
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
-    int rc = engine_process_enqueue(e, in_host, out_host, n_blocks, (size_t) e->B * e->active, true);
+    int rc = engine_process_enqueue(e, in_host, out_host, n_blocks, e->in_blk(), e->out_blk(), true);
     if (rc) return rc;
     return engine_process_wait(e);
 }
@@ -938,7 +1069,7 @@ int irb_engine_submit(irb_engine* e, const float* in_host, float* out_host, int 
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
     if (n_blocks == 0) return 0;
     if (n_blocks == 1) return fail(IRB_ERR_ARG, "irb_engine_submit takes at least two blocks per call (one block at a time is irb_engine_process)");
-    return engine_process_enqueue(e, in_host, out_host, n_blocks, (size_t) e->B * e->active, false);
+    return engine_process_enqueue(e, in_host, out_host, n_blocks, e->in_blk(), e->out_blk(), false);
 }
 int irb_engine_wait(irb_engine* e) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
@@ -954,6 +1085,7 @@ int irb_engine_wait(irb_engine* e) {
 int irb_engine_process_callback(irb_engine* e, const float* in_host, float* out_host, int n_blocks) {
     if (!e || !in_host || !out_host) return fail(IRB_ERR_ARG, "null argument");
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
+    if (e->matrix()) return fail(IRB_ERR_STATE, "an IR-matrix engine has no callback-order path: use irb_engine_process");
     if (n_blocks > e->ring) return fail(IRB_ERR_ARG, "%d blocks in one callback exceed the FDL ring of %d slots", n_blocks, e->ring);
     if (n_blocks == 0) return 0;
     CK(cudaSetDevice(e->device));
@@ -1242,7 +1374,7 @@ int irb_group_process(irb_group* g, const float* in_host, float* out_host, int n
     size_t started = 0;
     for (; started < g->eng.size() && !rc; ++started) {
         const size_t off = (size_t) g->begin[started] * g->B;
-        rc = engine_process_enqueue(g->eng[started], in_host + off, out_host + off, n_blocks, stride, false);
+        rc = engine_process_enqueue(g->eng[started], in_host + off, out_host + off, n_blocks, stride, stride, false);
     }
     for (size_t i = 0; i < started; ++i) { const int w = engine_process_wait(g->eng[i]); if (!rc) rc = w; }
     return rc;

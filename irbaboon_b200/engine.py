@@ -67,6 +67,8 @@ _SIGS = {
     "irb_launch_count": (ctypes.c_longlong, []),
     "irb_release_workspace": (ctypes.c_size_t, []),
     "irb_last_compute_ms": (ctypes.c_double, []),
+    "irb_engine_create_matrix": (ctypes.c_int, [ctypes.POINTER(_vp)] + [ctypes.c_int] * 7),
+    "irb_engine_bind_matrix": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]),
     "irb_group_create": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(ctypes.c_int)] + [ctypes.c_int] * 5),
     "irb_group_destroy": (ctypes.c_int, [_vp]),
     "irb_group_device_count": (ctypes.c_int, [_vp]),
@@ -509,6 +511,64 @@ class Engine:
         out = np.zeros(self.fft_size, np.float32)
         _ck(lib().irb_engine_read_fdl_spectrum(self._h, int(chan), int(age), _ptr(out)))
         return out
+
+
+class MatrixEngine(Engine):
+    """IR-matrix streaming engine (irb_engine_create_matrix): n_groups groups of `ins` input channels, each producing `outs`
+    output channels, out[g*outs + o] = sum_i conv(in[g*ins + i], IR ir_ids[i*outs + o]).  (ins, outs) = (1, 2) is mono -> stereo,
+    (2, 2) true stereo with the IRs in the order LL, LR, RL, RR.  Every input keeps one delay line, read once per block step for
+    all the IRs it feeds.  I/O arrays: in [n_blocks][n_groups*ins][B], out [n_blocks][n_groups*outs][B]."""
+
+    def __init__(self, block_size, max_partitions, n_groups, ins, outs, n_irs=None, device=0):
+        self._h = _vp()
+        n_irs = ins * outs if n_irs is None else n_irs
+        _ck(lib().irb_engine_create_matrix(ctypes.byref(self._h), int(device), int(block_size), int(max_partitions), int(n_groups), int(ins), int(outs), int(n_irs)))
+        self.block_size, self.max_partitions, self.n_irs, self.device = block_size, max_partitions, n_irs, device
+        self.n_groups, self.ins, self.outs = n_groups, ins, outs
+        self.n_channels = self.active_channels = n_groups * ins         # input channels (FDL rows)
+        self.n_outputs = n_groups * outs
+        self.fft_size = lib().irb_engine_fft_size(self._h)
+
+    def bind_matrix(self, group_begin, group_end, ir_ids):
+        """groups [group_begin, group_end) convolve with the IRs ir_ids[i*outs + o] (input i -> output o)."""
+        ids = [int(v) for v in ir_ids]
+        if len(ids) != self.ins * self.outs:
+            raise ValueError("ir_ids needs %d entries (ins*outs)" % (self.ins * self.outs))
+        arr = (ctypes.c_int * len(ids))(*ids)
+        _ck(lib().irb_engine_bind_matrix(self._h, int(group_begin), int(group_end), arr))
+
+    def _out_shape(self, x):
+        return x.shape[:-2] + (self.n_outputs, self.block_size)
+
+    def process(self, x, out=None):
+        """x: host [n_blocks][n_groups*ins][B] (or [n_groups*ins][B]) -> [n_blocks][n_groups*outs][B]."""
+        x = np.ascontiguousarray(x, np.float32)
+        if x.ndim not in (2, 3) or x.shape[-2:] != (self.n_channels, self.block_size):
+            raise ValueError("input shape %r, expected [n_blocks][%d][%d]" % (x.shape, self.n_channels, self.block_size))
+        nb = 1 if x.ndim == 2 else x.shape[0]
+        shp = self._out_shape(x)
+        if out is None:
+            out = np.empty(shp, np.float32)
+        elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.shape == shp and out.flags.c_contiguous and out.flags.writeable):
+            raise ValueError("out must be a writable C-contiguous float32 array of shape %r" % (shp,))
+        _ck(lib().irb_engine_process(self._h, _ptr(x), _ptr(out), nb))
+        return out
+
+    def submit(self, x, out):
+        """Asynchronous multi-block call on pinned host arrays (in [n_blocks >= 2][n_groups*ins][B], out [..][n_groups*outs][B])."""
+        assert x.dtype == np.float32 and out.dtype == np.float32 and x.flags.c_contiguous and out.flags.c_contiguous
+        assert x.ndim == 3 and x.shape[1:] == (self.n_channels, self.block_size) and out.shape == self._out_shape(x), (x.shape, out.shape)
+        _ck(lib().irb_engine_submit(self._h, _ptr(x), _ptr(out), x.shape[0]))
+
+    def process_stream(self, x):
+        """Planar inputs x[n_groups*ins][n] -> outputs y[n_groups*outs][n], block by block (zero-padded to whole blocks)."""
+        x = _planar(x)
+        B, n = self.block_size, x.shape[1]
+        nb = (n + B - 1) // B
+        xp = np.zeros((self.n_channels, nb * B), np.float32)
+        xp[:, :n] = x
+        y = self.process(np.ascontiguousarray(xp.reshape(self.n_channels, nb, B).transpose(1, 0, 2)))
+        return np.ascontiguousarray(y.transpose(1, 0, 2)).reshape(self.n_outputs, nb * B)[:, :n]
 
 
 class Group:

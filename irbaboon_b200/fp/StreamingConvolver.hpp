@@ -44,6 +44,40 @@ private:
     std::vector<float> stageIn, stageOut;
 };
 
+// IR-matrix streaming convolution (irb_engine_create_matrix): `groups` groups of `ins` input channels, each producing `outs`
+// output channels, out[g*outs + o] = sum_i conv(in[g*ins + i], IR ids[i*outs + o]).  (1, 2) is mono -> stereo (a binaural or
+// spatial source), (2, 2) true stereo with the IRs LL, LR, RL, RR.  Every input keeps one delay line, read once per block for
+// all the IRs it feeds.
+class MatrixConvolver {
+public:
+    // numIRs = 0: one matrix, ins*outs IRs; until bindMatrix every group uses IRs 0 .. ins*outs-1
+    MatrixConvolver(int blockSize, int maxPartitions, int groups, int ins, int outs, int numIRs = 0, int device = 0);
+    ~MatrixConvolver();
+    MatrixConvolver(const MatrixConvolver&) = delete;
+    MatrixConvolver& operator=(const MatrixConvolver&) = delete;
+
+    // An IR file: a mono one sets IR irId; one with ins*outs channels sets IRs irId .. irId + ins*outs - 1 from its channels
+    // (a stereo file is the {L, R} pair of a (1, 2) matrix, a four-channel file the LL, LR, RL, RR of a (2, 2) matrix)
+    void setIR(int irId, const AudioBuffer<float>& ir);
+    void bindMatrix(int groupBegin, int groupEnd, const std::vector<int>& irIds);    // irIds[i*outs + o]
+    void reset();
+    // one block per call: `in` holds groups*ins channels, `out` groups*outs channels, of exactly blockSize samples
+    void processBlock(const AudioBuffer<float>& in, AudioBuffer<float>& out);
+    // dense host arrays: in [nBlocks][groups*ins][blockSize], out [nBlocks][groups*outs][blockSize]
+    void process(const float* in, float* out, int nBlocks);
+
+    int getBlockSize() const { return blockSize; }
+    int getNumInputs() const { return groups * ins; }
+    int getNumOutputs() const { return groups * outs; }
+    int getLatencySamples() const { return blockSize; }
+    irb_engine* handle() const { return engine; }
+
+private:
+    irb_engine* engine = nullptr;
+    int blockSize, groups, ins, outs;
+    std::vector<float> stageIn, stageOut;
+};
+
 // The same over several GPUs driven from this process (irb_group_*): channels are sharded by contiguous ranges, shared IRs are
 // replicated on every device (numIRs > 0) or every channel owns the IR with its own number (numIRs == 0).
 class MultiGpuConvolver {

@@ -161,6 +161,40 @@ void StreamingConvolver::process(const float* in, float* out, int nBlocks) {
     if (irb_engine_process(engine, in, out, nBlocks) != IRB_OK) raise("irb_engine_process");
 }
 
+// ---- MatrixConvolver ------------------------------------------------------------------------------------
+MatrixConvolver::MatrixConvolver(int blockSize_, int maxPartitions, int groups_, int ins_, int outs_, int numIRs, int device)
+    : blockSize(blockSize_), groups(groups_), ins(ins_), outs(outs_) {
+    if (irb_engine_create_matrix(&engine, device, blockSize, maxPartitions, groups, ins, outs, numIRs > 0 ? numIRs : ins * outs) != IRB_OK)
+        raise("irb_engine_create_matrix");
+    stageIn.resize((size_t) blockSize * groups * ins);
+    stageOut.resize((size_t) blockSize * groups * outs);
+}
+MatrixConvolver::~MatrixConvolver() { irb_engine_destroy(engine); }
+void MatrixConvolver::setIR(int irId, const AudioBuffer<float>& ir) {
+    const int ch = ir.getNumChannels();
+    if (ch != 1 && ch != ins * outs)
+        throw std::invalid_argument("MatrixConvolver::setIR: an IR file has 1 channel or one per IR of the matrix (" + std::to_string(ins * outs) + ")");
+    for (int c = 0; c < ch; ++c)
+        if (irb_engine_set_ir(engine, irId + c, ir.getReadPointer(c), nullptr, ir.getNumSamples()) != IRB_OK) raise("irb_engine_set_ir");
+}
+void MatrixConvolver::bindMatrix(int groupBegin, int groupEnd, const std::vector<int>& irIds) {
+    if ((int) irIds.size() != ins * outs) throw std::invalid_argument("MatrixConvolver::bindMatrix: one IR id per input and output (ins*outs)");
+    if (irb_engine_bind_matrix(engine, groupBegin, groupEnd, irIds.data()) != IRB_OK) raise("irb_engine_bind_matrix");
+}
+void MatrixConvolver::reset() {
+    if (irb_engine_reset(engine) != IRB_OK) raise("irb_engine_reset");
+}
+void MatrixConvolver::processBlock(const AudioBuffer<float>& in, AudioBuffer<float>& out) {
+    if (in.getNumChannels() != groups * ins || in.getNumSamples() != blockSize || out.getNumChannels() != groups * outs || out.getNumSamples() != blockSize)
+        throw std::invalid_argument("MatrixConvolver::processBlock: in must be groups*ins x blockSize, out groups*outs x blockSize");
+    for (int c = 0; c < groups * ins; ++c) std::copy_n(in.getReadPointer(c), blockSize, stageIn.begin() + (size_t) c * blockSize);
+    if (irb_engine_process(engine, stageIn.data(), stageOut.data(), 1) != IRB_OK) raise("irb_engine_process");
+    for (int c = 0; c < groups * outs; ++c) out.copyFrom(c, 0, stageOut.data() + (size_t) c * blockSize, blockSize);
+}
+void MatrixConvolver::process(const float* in, float* out, int nBlocks) {
+    if (irb_engine_process(engine, in, out, nBlocks) != IRB_OK) raise("irb_engine_process");
+}
+
 // ---- MultiGpuConvolver ----------------------------------------------------------------------------------
 MultiGpuConvolver::MultiGpuConvolver(const std::vector<int>& devices, int blockSize, int maxPartitions, int channels, int numIRs) {
     if (irb_group_create(&group, devices.data(), (int) devices.size(), blockSize, maxPartitions, channels, numIRs) != IRB_OK) raise("irb_group_create");
