@@ -195,7 +195,9 @@ int irb_deconvolve(const float* num, int len_num, const float* den, int len_den,
 int irb_deconvolve_batch(const float* nums, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
                          int include_amplitude, float* out);
 /* _batch with DEVICE-resident captures nums_dev[batch][len_num] and results out_dev[batch][N] (den: host or device memory):
- * the batched capture when the recordings already live in HBM.  No staging copies for large plain divisions. */
+ * the batched capture when the recordings already live in HBM.  No staging copies for large plain divisions (no smoothing,
+ * phase kept, even len_num) when nums_dev and out_dev are both 8-byte aligned; any other alignment of a float pointer is
+ * accepted too, and goes through staged device-to-device copies. */
 int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing,
                                 int include_phase, int include_amplitude, float* out_dev);
 /* fp::ir::invertFilter (fp/ir.hpp:20, fp/ir.cpp:13-18); out[nextPowerOfTwo(len)] */

@@ -4,6 +4,7 @@
 // irb_spectral.cuh; the host only sizes buffers, copies and launches.
 #include <algorithm>
 #include <cmath>
+#include <cstdint>
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -536,8 +537,10 @@ int irb_deconvolve_batch(const float* nums, int batch, int len_num, const float*
 // The same with DEVICE-resident captures and results (den: host or device).  Large plain divisions (no smoothing, phase kept, an
 // even capture length) run with no staging at all: every sub-batch's column pass reads the captures where they lie, the
 // inverse column pass writes the impulse responses where they belong, and consecutive sub-batches alternate between compute
-// streams so that one sub-batch's row kernels fill the SMs another one's column pass leaves idle.  Everything else goes
-// through the staged pipeline above with device-to-device copies.  irb_last_compute_ms() is the device time of the whole call.
+// streams so that one sub-batch's row kernels fill the SMs another one's column pass leaves idle.  The column passes read the
+// captures and write the results as float2, so that path also needs both pointers 8-byte aligned (a float view at an odd
+// offset is only 4-byte aligned).  Everything else goes through the staged pipeline above with device-to-device copies, which
+// take any alignment.  irb_last_compute_ms() is the device time of the whole call.
 int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
                                 int include_amplitude, float* out_dev) {
     if (!nums_dev || !den || !out_dev) return fail(IRB_ERR_ARG, "null argument");
@@ -548,7 +551,8 @@ int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, c
     CK(cudaSetDevice(dev));
     Plan plan;
     if ((rc = plan.init(dev, M))) return rc;
-    if (!(plan.big() && !smoothing && include_phase && len_num % 2 == 0))
+    const bool aligned = (((uintptr_t) nums_dev | (uintptr_t) out_dev) % alignof(float2)) == 0;
+    if (!(plan.big() && !smoothing && include_phase && len_num % 2 == 0 && aligned))
         return deconvolve_batch_staged(nums_dev, batch, len_num, den, len_den, sample_rate, smoothing, include_phase, include_amplitude, out_dev, true);
     constexpr int kStreams = 3;
     const int sub_pref = irbh::g_tuning.deconv_sub;
