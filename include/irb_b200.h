@@ -8,7 +8,8 @@
  * reference tree).  The C++ facade in irbaboon_b200/fp/ (same namespaces, names, defaults as the
  * reference's fp/ headers) is a thin wrapper over these calls -- see INTEGRATION.md.
  *
- * Conventions: plain pointers and sizes, no C++/torch types.  All audio is float32.  Every function
+ * Conventions: plain pointers and sizes, no C++/torch types.  All audio is float32, except that the streaming engine's
+ * _pcm entry points also take and return 16- and 24-bit integer PCM (irb_sample_format).  Every function
  * returns 0 on success or a negative irb_status; irb_last_error() gives the message of the calling
  * thread's most recent failure.  No exception crosses this boundary.  There is NO CPU fallback: if no
  * sm_100 device is usable every compute entry point fails with IRB_ERR_CUDA.
@@ -34,6 +35,18 @@ typedef enum irb_status {
 } irb_status;
 
 typedef struct irb_engine irb_engine;
+
+/* Sample format of the block arrays of the streaming engine's _pcm entry points.  The layout does not change with the format:
+ * [n_blocks][channels][block_size] elements.  S16 is an int16_t; S24 is 3 bytes, little-endian and packed as in a WAV file
+ * (element k at bytes 3k .. 3k+2).  Any pointer aligned to its element works (2 bytes for S16, any byte for S24).
+ *   integer in  -> float: value / 2^(bits-1), exact (so a PCM input gives the same delay line as the float engine fed the
+ *                  dequantised block);
+ *   float out -> integer: the integer-WAV writer's rule (JUCE 6's AudioFormatWriter, as fp::formats::writeWav), in double:
+ *                  y <= -1 gives INT32_MIN, y >= 1 gives INT32_MAX, NaN gives 0, otherwise lrint(2147483647.0 * y) rounding
+ *                  half to even; then an arithmetic shift right by 32 - bits, which rounds toward minus infinity.  No dither.
+ * An integer output block is therefore exactly what writeWav writes for the float output block.  The engine applies no gain and
+ * no limiting: outputs at or beyond full scale clip to the extreme codes; to avoid clipping, scale the IR. */
+typedef enum irb_sample_format { IRB_SAMPLE_F32 = 0, IRB_SAMPLE_S16 = 1, IRB_SAMPLE_S24 = 2 } irb_sample_format;
 
 /* ---- library ------------------------------------------------------------------------------------ */
 const char* irb_last_error(void);
@@ -115,6 +128,14 @@ int irb_engine_synchronize(irb_engine* e);
  * submitted so far is back in host memory. */
 int irb_engine_submit(irb_engine* e, const float* in_host, float* out_host, int n_blocks);
 int irb_engine_wait(irb_engine* e);
+/* The same block steps with the input and the output in any irb_sample_format each (all nine pairs; in and out sized over the
+ * input and output channels, as above, on a matrix engine too).  The formats are arguments of each call, not engine state;
+ * _process, _submit and _process_device are the (F32, F32) case.  A format outside the enum gives IRB_ERR_ARG without touching
+ * a device; _submit_pcm takes n_blocks >= 2 like _submit and is completed by irb_engine_wait.  Blocks of different formats may
+ * follow each other on one engine.  _process_callback stays float only. */
+int irb_engine_process_pcm(irb_engine* e, const void* in_host, int in_format, void* out_host, int out_format, int n_blocks);
+int irb_engine_submit_pcm(irb_engine* e, const void* in_host, int in_format, void* out_host, int out_format, int n_blocks);
+int irb_engine_process_device_pcm(irb_engine* e, const void* in_dev, int in_format, void* out_dev, int out_format, int n_blocks);
 
 /* Per-step device timing with CUDA events on the engine's stream: whole block step (k_fwd + k_mac) and the
  * FDL-MAC kernel alone (on a one-launch block step the two are the same pair of events: no event is recorded in between).
@@ -171,6 +192,8 @@ int irb_group_stage_ir(irb_group* g, int ir_id, const float* left, const float* 
 int irb_group_bind(irb_group* g, int chan_begin, int chan_end, int ir_id);
 int irb_group_reset(irb_group* g);
 int irb_group_process(irb_group* g, const float* in_host, float* out_host, int n_blocks);
+/* irb_group_process with the input and output in any irb_sample_format (see irb_engine_process_pcm) */
+int irb_group_process_pcm(irb_group* g, const void* in_host, int in_format, void* out_host, int out_format, int n_blocks);
 size_t irb_group_state_bytes(const irb_group* g);
 
 /* ---- offline functions ------------------------------------------------------------------------------

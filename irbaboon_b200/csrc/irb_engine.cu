@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <memory>
 #include <mutex>
+#include <type_traits>
 #include <new>
 #include <vector>
 #include <atomic>
@@ -424,12 +425,12 @@ struct irb_engine {
     // The latency path (one small block per call): copy-in, the step's kernels and copy-out are captured ONCE into a CUDA
     // graph over pinned staging owned by the engine and replayed with a single launch per block.  The signature records
     // everything the captured launches baked in; a change re-captures.
-    struct GraphSig { int n_rr, split_in, cluster, slots, fuse, active, variant; cudaStream_t stream; bool operator==(const GraphSig& o) const {
+    struct GraphSig { int n_rr, split_in, cluster, slots, fuse, active, variant; cudaStream_t stream; int in_fmt, out_fmt; bool operator==(const GraphSig& o) const {
         return n_rr == o.n_rr && split_in == o.split_in && cluster == o.cluster && slots == o.slots && fuse == o.fuse && active == o.active &&
-               variant == o.variant && stream == o.stream; } };
+               variant == o.variant && stream == o.stream && in_fmt == o.in_fmt && out_fmt == o.out_fmt; } };
     cudaGraphExec_t g_exec = nullptr;
-    GraphSig g_sig{-1, 0, 0, 0, 0, 0, 0, nullptr};
-    float *g_hin = nullptr, *g_hout = nullptr;
+    GraphSig g_sig{-1, 0, 0, 0, 0, 0, 0, nullptr, 0, 0};
+    void *g_hin = nullptr, *g_hout = nullptr;
     int g_kernels = 0;
     bool g_warm = false;                             // a plain step with this signature has run (kernel attributes are set)
     bool use_graph = true;
@@ -556,11 +557,19 @@ int tuning_variant() {
 
 constexpr int kTimingCap = 16384;
 
+// the sample format of a block array (irb_sample_format): element size, and the address of element i
+bool fmt_valid(int fmt) { return fmt == IRB_SAMPLE_F32 || fmt == IRB_SAMPLE_S16 || fmt == IRB_SAMPLE_S24; }
+size_t fmt_size(int fmt) { return (size_t) irb::fmt_bytes(fmt); }
+template <class T> T* fmt_at(T* p, int fmt, size_t i) {
+    using Byte = typename std::conditional<std::is_const<T>::value, const unsigned char, unsigned char>::type;
+    return p ? (T*) ((Byte*) p + i * fmt_size(fmt)) : nullptr;
+}
+
 // forward FFT of one block of the channels of the range into the FDL (advances their heads) and/or the round-robin IR
-// refresh rows; in_dev / out_dev below are the block's arrays for ALL channels
-int engine_launch_fwd(irb_engine* e, const float* in_dev, bool audio, bool refresh, int c0, int cn) {
+// refresh rows; in_dev / out_dev below are the block's arrays for ALL channels, in the formats in_fmt / out_fmt
+int engine_launch_fwd(irb_engine* e, const void* in_dev, int in_fmt, bool audio, bool refresh, int c0, int cn) {
     irb::FwdArgs f{};
-    f.src = in_dev ? in_dev + (size_t) c0 * e->B : nullptr; f.src2 = nullptr; f.src_chan_stride = e->B; f.L = e->B; f.B = e->B;
+    f.src = fmt_at(in_dev, in_fmt, (size_t) c0 * e->B); f.src_fmt = in_fmt; f.src2 = nullptr; f.src_chan_stride = e->B; f.L = e->B; f.B = e->B;
     f.blocks_per_chan = 1; f.n_rows = audio ? cn : 0;
     f.dst = e->fdl.as<float2>() + (size_t) (c0 / e->fdl_group) * e->fdl_group_stride(); f.dst_chan_stride = e->fdl_group_stride();
     f.dst_group = e->fdl_group; f.dst_slot_stride = (long long) e->fdl_group * e->M;
@@ -576,26 +585,26 @@ int engine_launch_fwd(irb_engine* e, const float* in_dev, bool audio, bool refre
     return 0;
 }
 // the IR-matrix block step over every group: inputs in_dev [n_chans][B], outputs out_dev [n_chans / ins * outs][B]
-int engine_launch_mx(irb_engine* e, float* out_dev, const float* in_dev) {
+int engine_launch_mx(irb_engine* e, void* out_dev, int out_fmt, const void* in_dev, int in_fmt) {
     irb::MacArgs m{};
     fill_mac_args(e, m, 0, e->n_chans);
     m.n_rows = e->out_chans(); m.work = e->work.as<int>();
-    m.Y = nullptr; m.out = out_dev; m.out_chan_stride = e->B; m.Lout = e->B;
+    m.Y = nullptr; m.out = out_dev; m.out_fmt = out_fmt; m.out_chan_stride = e->B; m.Lout = e->B;
     m.ov = e->ov.as<float>(); m.tail = nullptr; m.head_back = 0;
-    m.in = in_dev; m.in_chan_stride = e->B; m.head_rw = e->head.as<int>();
+    m.in = in_dev; m.in_fmt = in_fmt; m.in_chan_stride = e->B; m.head_rw = e->head.as<int>();
     int rc = launch_mac_mx(e->M, e->ins, e->outs, e->per_row_ir, e->num_sms, m, e->stream);
     if (rc) return rc;
     e->launches += 1;
     return 0;
 }
 // in_dev != nullptr: the forward transform of that block runs inside the MAC kernel (shared-IR kernel only)
-int engine_launch_mac(irb_engine* e, float* out_dev, int head_back, const float* in_dev, int c0, int cn) {
-    if (e->matrix()) return engine_launch_mx(e, out_dev, in_dev);
+int engine_launch_mac(irb_engine* e, void* out_dev, int out_fmt, int head_back, const void* in_dev, int in_fmt, int c0, int cn) {
+    if (e->matrix()) return engine_launch_mx(e, out_dev, out_fmt, in_dev, in_fmt);
     irb::MacArgs m{};
     fill_mac_args(e, m, c0, cn);
-    m.Y = nullptr; m.out = out_dev + (size_t) c0 * e->B; m.out_chan_stride = e->B; m.Lout = e->B;
+    m.Y = nullptr; m.out = fmt_at(out_dev, out_fmt, (size_t) c0 * e->B); m.out_fmt = out_fmt; m.out_chan_stride = e->B; m.Lout = e->B;
     m.ov = e->ov.as<float>() + (size_t) c0 * e->B; m.tail = nullptr; m.head_back = head_back;
-    m.in = in_dev ? in_dev + (size_t) c0 * e->B : nullptr; m.in_chan_stride = e->B; m.head_rw = e->head.as<int>() + c0;
+    m.in = fmt_at(in_dev, in_fmt, (size_t) c0 * e->B); m.in_fmt = in_fmt; m.in_chan_stride = e->B; m.head_rw = e->head.as<int>() + c0;
     int rc = launch_mac(e->M, true, use_slots(e), e->cluster_dim, e->num_sms, m, e->stream);
     if (rc) return rc;
     e->launches += 1;
@@ -603,27 +612,27 @@ int engine_launch_mac(irb_engine* e, float* out_dev, int head_back, const float*
 }
 
 // one block step for the channels [c0, c0+cn); refresh: also run the staged IRs' refresh rows (once per block)
-int engine_step_range(irb_engine* e, const float* in_dev, float* out_dev, int c0, int cn, bool refresh) {
+int engine_step_range(irb_engine* e, const void* in_dev, int in_fmt, void* out_dev, int out_fmt, int c0, int cn, bool refresh) {
     // ONE launch per block step, the forward transform is the MAC kernel's prologue (staged IRs still get their refresh
     // rows through a k_fwd launch of their own).  The few-row cluster kernel transforms the new blocks on its rank 0.
     const bool fused = step_is_fused(e);
-    int rc = engine_launch_fwd(e, in_dev, !fused, refresh, c0, cn);
+    int rc = engine_launch_fwd(e, in_dev, in_fmt, !fused, refresh, c0, cn);
     if (rc) return rc;
-    return engine_launch_mac(e, out_dev, 0, fused ? in_dev : nullptr, c0, cn);
+    return engine_launch_mac(e, out_dev, out_fmt, 0, fused ? in_dev : nullptr, in_fmt, c0, cn);
 }
 
-int engine_step_device(irb_engine* e, const float* in_dev, float* out_dev) {
+int engine_step_device(irb_engine* e, const void* in_dev, int in_fmt, void* out_dev, int out_fmt) {
     const bool rec = e->timing && e->t_rec < kTimingCap;
     if (rec) CK(cudaEventRecord(e->tev[3 * e->t_rec], e->stream));
     const bool fused = step_is_fused(e);
     const long long launched = g_launches.load();
-    int rc = engine_launch_fwd(e, in_dev, !fused, true, 0, e->active);
+    int rc = engine_launch_fwd(e, in_dev, in_fmt, !fused, true, 0, e->active);
     if (rc) return rc;
     // the middle event only where a kernel ran before the MAC launch: on a one-launch step it would add its own 2-3 us to the step
     const bool mid = rec && g_launches.load() != launched;
     if (rec) e->tev_mid[e->t_rec] = mid;
     if (mid) CK(cudaEventRecord(e->tev[3 * e->t_rec + 1], e->stream));
-    if ((rc = engine_launch_mac(e, out_dev, 0, fused ? in_dev : nullptr, 0, e->active))) return rc;
+    if ((rc = engine_launch_mac(e, out_dev, out_fmt, 0, fused ? in_dev : nullptr, in_fmt, 0, e->active))) return rc;
     if (rec) { CK(cudaEventRecord(e->tev[3 * e->t_rec + 2], e->stream)); e->t_rec++; }
     return 0;
 }
@@ -899,6 +908,10 @@ int irb_engine_mac_plan(irb_engine* e, int* slots_kernel, int* split_in, int* cl
 }
 
 int irb_engine_process_device(irb_engine* e, const float* in_dev, float* out_dev, int n_blocks) {
+    return irb_engine_process_device_pcm(e, in_dev, IRB_SAMPLE_F32, out_dev, IRB_SAMPLE_F32, n_blocks);
+}
+int irb_engine_process_device_pcm(irb_engine* e, const void* in_dev, int in_format, void* out_dev, int out_format, int n_blocks) {
+    if (!fmt_valid(in_format) || !fmt_valid(out_format)) return fail(IRB_ERR_ARG, "sample format %d / %d is not an irb_sample_format", in_format, out_format);
     if (!e || !in_dev || !out_dev) return fail(IRB_ERR_ARG, "null argument");
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
     CK(cudaSetDevice(e->device));
@@ -906,7 +919,7 @@ int irb_engine_process_device(irb_engine* e, const float* in_dev, float* out_dev
     if (rc) return rc;
     const size_t iblk = e->in_blk(), oblk = e->out_blk();
     for (int b = 0; b < n_blocks; ++b)
-        if ((rc = engine_step_device(e, in_dev + b * iblk, out_dev + b * oblk))) return rc;
+        if ((rc = engine_step_device(e, fmt_at(in_dev, in_format, b * iblk), in_format, fmt_at(out_dev, out_format, b * oblk), out_format))) return rc;
     return 0;
 }
 
@@ -916,11 +929,14 @@ constexpr int kMaxGroups = 16;                       // channel groups a large s
 
 // one block, host to host, as a single graph launch; *done = false when the caller should take the plain path instead.
 // Matrix engines take this path too: input and output staging are sized by their own channel counts.
-int engine_process_one_graphed(irb_engine* e, const float* in_host, float* out_host, bool* done) {
+// The pinned staging holds kGraphMaxBytes whatever the formats; the eligibility test is made at float size, so a change of
+// format never changes which path a block takes, only the captured byte counts (the signature holds both formats).
+int engine_process_one_graphed(irb_engine* e, const void* in_host, int in_fmt, void* out_host, int out_fmt, bool* done) {
     *done = false;
-    const size_t bytes = sizeof(float) * e->in_blk(), obytes = sizeof(float) * e->out_blk();      // (differ on a matrix engine)
-    if (irbh::g_tuning.no_graph || !e->use_graph || e->timing || std::max(bytes, obytes) > kGraphMaxBytes) return 0;
-    const irb_engine::GraphSig sig{(int) e->h_rr_list.size(), e->split_in, e->cluster_dim, use_slots(e) ? 1 : 0, e->fuse_fwd ? 1 : 0, e->active, tuning_variant(), e->stream};
+    if (irbh::g_tuning.no_graph || !e->use_graph || e->timing || sizeof(float) * std::max(e->in_blk(), e->out_blk()) > kGraphMaxBytes) return 0;
+    const size_t bytes = fmt_size(in_fmt) * e->in_blk(), obytes = fmt_size(out_fmt) * e->out_blk();      // (differ on a matrix engine)
+    const irb_engine::GraphSig sig{(int) e->h_rr_list.size(), e->split_in, e->cluster_dim, use_slots(e) ? 1 : 0, e->fuse_fwd ? 1 : 0, e->active, tuning_variant(), e->stream,
+                                   in_fmt, out_fmt};
     if (!(sig == e->g_sig)) {
         if (e->g_exec) { cudaGraphExecDestroy(e->g_exec); e->g_exec = nullptr; }
         e->g_sig = sig;
@@ -933,7 +949,7 @@ int engine_process_one_graphed(irb_engine* e, const float* in_host, float* out_h
         cudaGraph_t graph = nullptr;
         CK(cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeRelaxed));
         int rc = cudaMemcpyAsync(e->io_in[0].p, e->g_hin, bytes, cudaMemcpyHostToDevice, e->stream) == cudaSuccess ? 0 : IRB_ERR_CUDA;
-        if (!rc) rc = engine_step_device(e, e->io_in[0].as<float>(), e->io_out[0].as<float>());
+        if (!rc) rc = engine_step_device(e, e->io_in[0].p, in_fmt, e->io_out[0].p, out_fmt);
         if (!rc && cudaMemcpyAsync(e->g_hout, e->io_out[0].p, obytes, cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) rc = IRB_ERR_CUDA;
         const cudaError_t ce = cudaStreamEndCapture(e->stream, &graph);
         e->g_kernels = (int) (e->launches - l0);
@@ -973,27 +989,28 @@ int engine_process_wait(irb_engine* e) {
     return 0;
 }
 
-int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host, int n_blocks, size_t stride, size_t out_stride, bool allow_graph) {
+int engine_process_enqueue(irb_engine* e, const void* in_host, int in_fmt, void* out_host, int out_fmt, int n_blocks, size_t stride, size_t out_stride, bool allow_graph) {
     CK(cudaSetDevice(e->device));
     int rc = engine_check_binding(e);
     if (rc) return rc;
-    const size_t blk = e->in_blk(), oblk = e->out_blk();
+    const size_t blk = e->in_blk(), oblk = e->out_blk();              // elements; strides too
+    const size_t isz = fmt_size(in_fmt), osz = fmt_size(out_fmt);
     if (n_blocks == 1) {
         if (e->pipe_pending && (rc = engine_process_wait(e))) return rc;               // submitted blocks still own the staging slots
         // a live callback: one block in, one block out.  Small blocks replay a captured graph (one launch); larger ones
         // run copy, kernels, copy back to back on the engine's stream -- no cross-stream events to wait on.
         if (allow_graph) {
             bool done = false;
-            if ((rc = engine_process_one_graphed(e, in_host, out_host, &done)) || done) return rc;
+            if ((rc = engine_process_one_graphed(e, in_host, in_fmt, out_host, out_fmt, &done)) || done) return rc;
         }
         const int rows = tile_rows(e->M);
         const int tiles = (e->active + rows - 1) / rows;
         // (a matrix engine always takes the one-range form: its launch covers every group)
-        const int groups = (e->timing || e->matrix() || sizeof(float) * blk < (4u << 20)) ? 1 : (int) std::min<long long>(kMaxGroups, tiles / (4LL * e->num_sms) > 0 ? tiles / (4LL * e->num_sms) : 1);
+        const int groups = (e->timing || e->matrix() || isz * blk < (4u << 20)) ? 1 : (int) std::min<long long>(kMaxGroups, tiles / (4LL * e->num_sms) > 0 ? tiles / (4LL * e->num_sms) : 1);
         if (groups <= 1) {
-            CK(cudaMemcpyAsync(e->io_in[0].p, in_host, sizeof(float) * blk, cudaMemcpyHostToDevice, e->stream));
-            if ((rc = engine_step_device(e, e->io_in[0].as<float>(), e->io_out[0].as<float>()))) return rc;
-            CK(cudaMemcpyAsync(out_host, e->io_out[0].p, sizeof(float) * oblk, cudaMemcpyDeviceToHost, e->stream));
+            CK(cudaMemcpyAsync(e->io_in[0].p, in_host, isz * blk, cudaMemcpyHostToDevice, e->stream));
+            if ((rc = engine_step_device(e, e->io_in[0].p, in_fmt, e->io_out[0].p, out_fmt))) return rc;
+            CK(cudaMemcpyAsync(out_host, e->io_out[0].p, osz * oblk, cudaMemcpyDeviceToHost, e->stream));
             return 0;
         }
         // A large block: cut the channels into groups of whole tiles and pipeline upload | kernels | download across the
@@ -1006,13 +1023,13 @@ int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host,
         for (int g = 0; g < groups; ++g) {
             const int c0 = (int) ((long long) tiles * g / groups) * rows, c1 = std::min(e->active, (int) ((long long) tiles * (g + 1) / groups) * rows);
             const size_t off = (size_t) c0 * e->B, cnt = (size_t) (c1 - c0) * e->B;
-            CK(cudaMemcpyAsync(e->io_in[0].as<float>() + off, in_host + off, sizeof(float) * cnt, cudaMemcpyHostToDevice, e->s_in));
+            CK(cudaMemcpyAsync(fmt_at(e->io_in[0].p, in_fmt, off), fmt_at(in_host, in_fmt, off), isz * cnt, cudaMemcpyHostToDevice, e->s_in));
             CK(cudaEventRecord(e->ev_grp[2 * g], e->s_in));
             CK(cudaStreamWaitEvent(e->stream, e->ev_grp[2 * g], 0));
-            if ((rc = engine_step_range(e, e->io_in[0].as<float>(), e->io_out[0].as<float>(), c0, c1 - c0, g == 0))) return rc;
+            if ((rc = engine_step_range(e, e->io_in[0].p, in_fmt, e->io_out[0].p, out_fmt, c0, c1 - c0, g == 0))) return rc;
             CK(cudaEventRecord(e->ev_grp[2 * g + 1], e->stream));
             CK(cudaStreamWaitEvent(e->s_out, e->ev_grp[2 * g + 1], 0));
-            CK(cudaMemcpyAsync(out_host + off, e->io_out[0].as<float>() + off, sizeof(float) * cnt, cudaMemcpyDeviceToHost, e->s_out));
+            CK(cudaMemcpyAsync(fmt_at(out_host, out_fmt, off), fmt_at(e->io_out[0].p, out_fmt, off), osz * cnt, cudaMemcpyDeviceToHost, e->s_out));
         }
         return 0;
     }
@@ -1023,14 +1040,14 @@ int engine_process_enqueue(irb_engine* e, const float* in_host, float* out_host,
         const bool reused = e->pipe_seq >= 2;
         ++e->pipe_seq;
         if (reused) CK(cudaStreamWaitEvent(e->s_in, e->ev_done[q], 0));            // the step two blocks back has consumed io_in[q]
-        CK(cudaMemcpyAsync(e->io_in[q].p, in_host + b * stride, sizeof(float) * blk, cudaMemcpyHostToDevice, e->s_in));
+        CK(cudaMemcpyAsync(e->io_in[q].p, fmt_at(in_host, in_fmt, b * stride), isz * blk, cudaMemcpyHostToDevice, e->s_in));
         CK(cudaEventRecord(e->ev_in[q], e->s_in));
         CK(cudaStreamWaitEvent(e->stream, e->ev_in[q], 0));
         if (reused) CK(cudaStreamWaitEvent(e->stream, e->ev_out[q], 0));           // its download has drained io_out[q]
-        if ((rc = engine_step_device(e, e->io_in[q].as<float>(), e->io_out[q].as<float>()))) return rc;
+        if ((rc = engine_step_device(e, e->io_in[q].p, in_fmt, e->io_out[q].p, out_fmt))) return rc;
         CK(cudaEventRecord(e->ev_done[q], e->stream));
         CK(cudaStreamWaitEvent(e->s_out, e->ev_done[q], 0));
-        CK(cudaMemcpyAsync(out_host + b * out_stride, e->io_out[q].p, sizeof(float) * oblk, cudaMemcpyDeviceToHost, e->s_out));
+        CK(cudaMemcpyAsync(fmt_at(out_host, out_fmt, b * out_stride), e->io_out[q].p, osz * oblk, cudaMemcpyDeviceToHost, e->s_out));
         CK(cudaEventRecord(e->ev_out[q], e->s_out));
     }
     e->pipe_pending = true;
@@ -1054,9 +1071,13 @@ int irb_engine_set_active_channels(irb_engine* e, int n_active) {
 int irb_engine_active_channels(const irb_engine* e) { return e ? e->active : fail(IRB_ERR_ARG, "engine is null"); }
 
 int irb_engine_process(irb_engine* e, const float* in_host, float* out_host, int n_blocks) {
+    return irb_engine_process_pcm(e, in_host, IRB_SAMPLE_F32, out_host, IRB_SAMPLE_F32, n_blocks);
+}
+int irb_engine_process_pcm(irb_engine* e, const void* in_host, int in_format, void* out_host, int out_format, int n_blocks) {
+    if (!fmt_valid(in_format) || !fmt_valid(out_format)) return fail(IRB_ERR_ARG, "sample format %d / %d is not an irb_sample_format", in_format, out_format);
     if (!e || !in_host || !out_host) return fail(IRB_ERR_ARG, "null argument");
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
-    int rc = engine_process_enqueue(e, in_host, out_host, n_blocks, e->in_blk(), e->out_blk(), true);
+    int rc = engine_process_enqueue(e, in_host, in_format, out_host, out_format, n_blocks, e->in_blk(), e->out_blk(), true);
     if (rc) return rc;
     return engine_process_wait(e);
 }
@@ -1065,11 +1086,15 @@ int irb_engine_process(irb_engine* e, const float* in_host, float* out_host, int
 // (the host arrays must stay valid and pinned until the wait); consecutive submits keep the three-stage pipeline full
 // instead of draining it at every call.  irb_engine_wait returns when everything submitted so far is back in host memory.
 int irb_engine_submit(irb_engine* e, const float* in_host, float* out_host, int n_blocks) {
+    return irb_engine_submit_pcm(e, in_host, IRB_SAMPLE_F32, out_host, IRB_SAMPLE_F32, n_blocks);
+}
+int irb_engine_submit_pcm(irb_engine* e, const void* in_host, int in_format, void* out_host, int out_format, int n_blocks) {
+    if (!fmt_valid(in_format) || !fmt_valid(out_format)) return fail(IRB_ERR_ARG, "sample format %d / %d is not an irb_sample_format", in_format, out_format);
+    if (n_blocks == 1) return fail(IRB_ERR_ARG, "irb_engine_submit takes at least two blocks per call (one block at a time is irb_engine_process)");
     if (!e || !in_host || !out_host) return fail(IRB_ERR_ARG, "null argument");
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
     if (n_blocks == 0) return 0;
-    if (n_blocks == 1) return fail(IRB_ERR_ARG, "irb_engine_submit takes at least two blocks per call (one block at a time is irb_engine_process)");
-    return engine_process_enqueue(e, in_host, out_host, n_blocks, e->in_blk(), e->out_blk(), false);
+    return engine_process_enqueue(e, in_host, in_format, out_host, out_format, n_blocks, e->in_blk(), e->out_blk(), false);
 }
 int irb_engine_wait(irb_engine* e) {
     if (!e) return fail(IRB_ERR_ARG, "engine is null");
@@ -1104,10 +1129,10 @@ int irb_engine_process_callback(irb_engine* e, const float* in_host, float* out_
     float* dout = e->cb_out->as<float>();
     CK(cudaMemcpyAsync(din, in_host, sizeof(float) * blk * n_blocks, cudaMemcpyHostToDevice, e->stream));
     for (int b = 0; b < n_blocks; ++b)
-        if ((rc = engine_launch_fwd(e, din + b * blk, true, false, 0, e->active))) return rc;
+        if ((rc = engine_launch_fwd(e, din + b * blk, IRB_SAMPLE_F32, true, false, 0, e->active))) return rc;
     for (int b = 0; b < n_blocks; ++b) {
-        if ((rc = engine_launch_fwd(e, nullptr, false, true, 0, e->active))) return rc;
-        if ((rc = engine_launch_mac(e, dout + b * blk, n_blocks - 1 - b, nullptr, 0, e->active))) return rc;
+        if ((rc = engine_launch_fwd(e, nullptr, IRB_SAMPLE_F32, false, true, 0, e->active))) return rc;
+        if ((rc = engine_launch_mac(e, dout + b * blk, IRB_SAMPLE_F32, n_blocks - 1 - b, nullptr, IRB_SAMPLE_F32, 0, e->active))) return rc;
     }
     CK(cudaMemcpyAsync(out_host, dout, sizeof(float) * blk * n_blocks, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
@@ -1367,14 +1392,18 @@ int irb_group_reset(irb_group* g) {
 }
 // in/out: HOST [n_blocks][n_channels][block_size] for ALL channels; every device is fed from one thread (enqueue all, then wait all)
 int irb_group_process(irb_group* g, const float* in_host, float* out_host, int n_blocks) {
+    return irb_group_process_pcm(g, in_host, IRB_SAMPLE_F32, out_host, IRB_SAMPLE_F32, n_blocks);
+}
+int irb_group_process_pcm(irb_group* g, const void* in_host, int in_format, void* out_host, int out_format, int n_blocks) {
+    if (!fmt_valid(in_format) || !fmt_valid(out_format)) return fail(IRB_ERR_ARG, "sample format %d / %d is not an irb_sample_format", in_format, out_format);
     if (!g || !in_host || !out_host) return fail(IRB_ERR_ARG, "null argument");
     if (n_blocks < 0) return fail(IRB_ERR_ARG, "n_blocks < 0");
-    const size_t stride = (size_t) g->B * g->n_chans;
+    const size_t stride = (size_t) g->B * g->n_chans;            // elements
     int rc = 0;
     size_t started = 0;
     for (; started < g->eng.size() && !rc; ++started) {
         const size_t off = (size_t) g->begin[started] * g->B;
-        rc = engine_process_enqueue(g->eng[started], in_host + off, out_host + off, n_blocks, stride, stride, false);
+        rc = engine_process_enqueue(g->eng[started], fmt_at(in_host, in_format, off), in_format, fmt_at(out_host, out_format, off), out_format, n_blocks, stride, stride, false);
     }
     for (size_t i = 0; i < started; ++i) { const int w = engine_process_wait(g->eng[i]); if (!rc) rc = w; }
     return rc;

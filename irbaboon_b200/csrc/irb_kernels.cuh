@@ -101,6 +101,42 @@ __device__ __forceinline__ void ldg_stream256(const float4* p, float4& a, float4
     asm volatile("ld.global.nc.L1::no_allocate.L2::evict_first.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                  : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w) : "l"(p));
 }
+// ---- sample formats of the streaming block step's audio rows (irb_sample_format in include/irb_b200.h) ----------------
+// The new block a step reads (load_in) and the output block it writes (store_out) are float32, int16 or packed little-endian
+// 24-bit integers; element i of a row sits at byte i * fmt_bytes(fmt).  Every access is one element wide (three single bytes
+// for 24-bit), so any element-aligned pointer works.  The format is a launch argument, uniform over the launch.
+constexpr int kFmtF32 = 0, kFmtS16 = 1, kFmtS24 = 2;
+__host__ __device__ __forceinline__ int fmt_bytes(int fmt) { return fmt == kFmtS16 ? 2 : fmt == kFmtS24 ? 3 : 4; }
+// integer -> float: value / 2^(bits-1), exact in float (formats::readWav)
+__device__ __forceinline__ float load_in(const void* p, int fmt, long long i) {
+    if (fmt == kFmtS16) return __fmul_rn((float) reinterpret_cast<const int16_t*>(p)[i], 1.0f / 32768.0f);
+    if (fmt == kFmtS24) {
+        const unsigned char* b = reinterpret_cast<const unsigned char*>(p) + 3 * i;
+        const int v = (int) ((unsigned) b[0] << 8 | (unsigned) b[1] << 16 | (unsigned) b[2] << 24) >> 8;      // sign-extended
+        return __fmul_rn((float) v, 1.0f / 8388608.0f);
+    }
+    return reinterpret_cast<const float*>(p)[i];
+}
+// float -> integer: the integer-WAV writer's rule (formats::writeWav), in double: y <= -1 -> INT32_MIN, y >= 1 -> INT32_MAX,
+// NaN -> 0, otherwise round-half-even(2147483647 * y); then an arithmetic shift right by 32 - bits (toward -infinity, no dither)
+__device__ __forceinline__ int quantise_s32(float y) {
+    const double d = (double) y;
+    if (d <= -1.0) return (int) 0x80000000u;
+    if (d >= 1.0) return 0x7fffffff;
+    if (d != d) return 0;
+    return __double2int_rn(__dmul_rn(2147483647.0, d));
+}
+__device__ __forceinline__ void store_out(void* p, int fmt, long long i, float y) {
+    if (fmt == kFmtS16) { reinterpret_cast<int16_t*>(p)[i] = (int16_t) (quantise_s32(y) >> 16); return; }
+    if (fmt == kFmtS24) {
+        const int q = quantise_s32(y) >> 8;
+        unsigned char* b = reinterpret_cast<unsigned char*>(p) + 3 * i;
+        b[0] = (unsigned char) q; b[1] = (unsigned char) (q >> 8); b[2] = (unsigned char) (q >> 16);
+        return;
+    }
+    reinterpret_cast<float*>(p)[i] = y;
+}
+
 // MAC layout of the shared-IR kernel: a thread owns V float4 of each of K rows (K*V = 4).  Narrow: the float4 are TPR apart
 // (a warp instruction reads 512 contiguous bytes).  WIDE: they come in adjacent pairs, one 32-byte load each (1 KB per warp
 // instruction, half the load instructions for the same bytes in flight).
@@ -134,9 +170,10 @@ __device__ __forceinline__ void fft_run(float2 (&v)[kPts], int t, float2* srow, 
 // Destination slot: blk (offline / IR preparation) or, when head != nullptr, the next ring slot of chan
 // (streaming: the kernel also advances head[chan]).
 struct FwdArgs {
-    const float* src;          // device samples
+    const void* src;           // device samples, format src_fmt (load_in)
+    int src_fmt;
     const float* src2;         // optional second channel folded in as (a + b) / 2  (tools::sumToMono, fp/tools.cpp:25-29)
-    long long src_chan_stride; // floats
+    long long src_chan_stride; // elements
     int L;                     // samples per channel
     int B;                     // block size (<= M)
     int blocks_per_chan;
@@ -162,12 +199,12 @@ struct FwdArgs {
     long long h_rep_stride;
 };
 
-struct FwdRow {                // what one row of k_fwd reads and writes
-    const float* p; const float* q; int len; float2* d; bool live; int reps;
+struct FwdRow {                // what one row of k_fwd reads (p in format fmt) and writes
+    const void* p; const float* q; int len; float2* d; bool live; int reps; int fmt;
 };
 template <int ROWS, int M>
 __device__ __forceinline__ FwdRow fwd_row(const FwdArgs& a, int main_tiles, int tile, int r) {
-    FwdRow w{nullptr, nullptr, 0, nullptr, false, 1};
+    FwdRow w{nullptr, nullptr, 0, nullptr, false, 1, kFmtF32};
     if (tile < main_tiles) {
         const int row = tile * ROWS + r;
         if (row >= a.n_rows) return w;
@@ -175,7 +212,8 @@ __device__ __forceinline__ FwdRow fwd_row(const FwdArgs& a, int main_tiles, int 
         int len = a.L - blk * a.B;
         w.len = len < 0 ? 0 : (len > a.B ? a.B : len);
         const long long off = chan * a.src_chan_stride + (long long) blk * a.B;
-        w.p = a.src + off;
+        w.p = reinterpret_cast<const unsigned char*>(a.src) + off * fmt_bytes(a.src_fmt);
+        w.fmt = a.src_fmt;
         w.q = a.src2 ? a.src2 + off : nullptr;
         int slot = blk;
         if (a.head) { slot = a.head[chan] + 1; if (slot >= a.ring) slot = 0; }
@@ -211,8 +249,8 @@ __global__ void __launch_bounds__(kThreads) k_fwd(const FwdArgs a) {
             for (int j = 0; j < kPts; ++j) {
                 const int m = 2 * (t + j * T::TPF);
                 float x0 = 0.f, x1 = 0.f;
-                if (m < w.len) x0 = w.p[m];
-                if (m + 1 < w.len) x1 = w.p[m + 1];
+                if (m < w.len) x0 = load_in(w.p, w.fmt, m);
+                if (m + 1 < w.len) x1 = load_in(w.p, w.fmt, m + 1);
                 if (w.q) {
                     if (m < w.len) { x0 += w.q[m]; x0 /= 2.0f; }
                     if (m + 1 < w.len) { x1 += w.q[m + 1]; x1 /= 2.0f; }
@@ -287,7 +325,8 @@ struct MacArgs {
     float2* Y;                 // [row][M]
     // INV: time-domain epilogue
     int B;
-    float* out;                // out + chan*out_chan_stride + blk*B + m, m < clamp(Lout - blk*B, 0, B)
+    void* out;                 // element chan*out_chan_stride + blk*B + m, m < clamp(Lout - blk*B, 0, B), format out_fmt (store_out)
+    int out_fmt;
     long long out_chan_stride;
     int Lout;
     float* ov;                 // streaming: overlap state [chan][B] (read, then replaced); offline: nullptr
@@ -296,9 +335,10 @@ struct MacArgs {
     int head_back;             // streaming: the newest spectrum of this step sits head_back slots behind head (callback order)
     // k_mac<FUSE>: the step's forward transform runs in the MAC kernel's prologue (no k_fwd launch): in[chan*in_chan_stride + i],
     // i < B, is the new block of every row; its spectrum goes to slot head+1, is used from registers as partition 0, and
-    // head[chan] is advanced by this kernel.  `head` must not be const for that.
-    const float* in;
-    long long in_chan_stride;
+    // head[chan] is advanced by this kernel.  `head` must not be const for that.  The new blocks are in format in_fmt (load_in).
+    const void* in;
+    int in_fmt;
+    long long in_chan_stride;  // elements
     int* head_rw;
     int producer_sleep_ns;     // the TMA producer sleeps this long between polls of a busy stage (0: spin)
     unsigned zero;             // always 0; unknown to the compiler (mbar_arrive_after)
@@ -342,7 +382,7 @@ __device__ __forceinline__ void inv_epilogue(const MacArgs& a, float2* tile, int
     const int chan = live ? row / a.blocks_per_chan : 0, blk = live ? row % a.blocks_per_chan : 0;
     int olen = a.Lout - blk * a.B;
     olen = olen < 0 ? 0 : (olen > a.B ? a.B : olen);
-    float* outp = a.out + chan * a.out_chan_stride + (long long) blk * a.B;
+    const long long out0 = chan * a.out_chan_stride + (long long) blk * a.B;      // element index of the output row
     float* ovp = a.ov ? a.ov + (long long) chan * a.B : nullptr;
     float* tailp = a.tail ? a.tail + (long long) row * a.B : nullptr;
     // The overlap of the previous block, all 2 x kPts values of a thread requested back to back (predicated loads, no branches:
@@ -381,6 +421,12 @@ __device__ __forceinline__ void inv_epilogue(const MacArgs& a, float2* tile, int
     if (a.ov) bar_compute();                           // all overlap reads precede the overlap writes
     if constexpr (LAT) stamp(a, 13);
     if (live) {
+        // Integer output (streaming only, so the barrier above has ended every read of the row): the output half is parked in the
+        // thread's own places of the row and converted by a rolled loop, so that the double-precision rule (store_out) does not
+        // run in 2 x kPts unrolled copies next to the live transform values.
+        const bool pcm = a.out_fmt != kFmtF32;
+        float* park = reinterpret_cast<float*>(srow);
+        float* outp = reinterpret_cast<float*>(a.out) + out0;
 #pragma unroll
         for (int j = 0; j < kPts; ++j) {
             const int m = 2 * (t + j * T::TPF);
@@ -389,8 +435,15 @@ __device__ __forceinline__ void inv_epilogue(const MacArgs& a, float2* tile, int
             for (int e = 0; e < 2; ++e) {                   // one predicated store per sample: output block, or the next overlap / the tail
                 const int mm = m + e;
                 const bool first = mm < a.B;
-                float* dst = first ? outp + mm : (ovp ? ovp : tailp) + (mm - a.B);
+                float* dst = first ? (pcm ? park : outp) + mm : (ovp ? ovp : tailp) + (mm - a.B);
                 if (first ? mm < olen : mm < 2 * a.B) *dst = val[e];
+            }
+        }
+        if (pcm) {
+#pragma unroll 1
+            for (int i = 0; i < 2 * kPts; ++i) {
+                const int m = 2 * (t + (i >> 1) * T::TPF) + (i & 1);
+                if (m < olen) store_out(a.out, a.out_fmt, out0 + m, park[m]);
             }
         }
     }
@@ -470,12 +523,12 @@ __global__ void __launch_bounds__(kThreads + 32, U == 1 ? 3 : 2) k_mac(const Mac
 #pragma unroll
         for (int j = 0; j < kPts; ++j) v[j] = make_float2(0.f, 0.f);
         if (row < a.n_rows) {
-            const float* p = a.in + row * a.in_chan_stride;
+            const long long i0 = (long long) row * a.in_chan_stride;
 #pragma unroll
             for (int j = 0; j < kPts; ++j) {
                 const int m = 2 * (t + j * T::TPF);                  // scalar loads: a row starts at an odd float offset when B is odd
-                if (m < a.B) v[j].x = p[m];
-                if (m + 1 < a.B) v[j].y = p[m + 1];
+                if (m < a.B) v[j].x = load_in(a.in, a.in_fmt, i0 + m);
+                if (m + 1 < a.B) v[j].y = load_in(a.in, a.in_fmt, i0 + m + 1);
             }
         }
         float2* srow = sm.spec + rf * M;
@@ -742,12 +795,12 @@ __global__ void __launch_bounds__(kThreads + 32, M <= 1024 ? 3 : 2) k_mac_tma(co
 #pragma unroll
         for (int j = 0; j < kPts; ++j) v[j] = make_float2(0.f, 0.f);
         if (row < a.n_rows) {
-            const float* p = a.in + row * a.in_chan_stride;
+            const long long i0 = (long long) row * a.in_chan_stride;
 #pragma unroll
             for (int j = 0; j < kPts; ++j) {
                 const int m = 2 * (t + j * T::TPF);
-                if (m < a.B) v[j].x = p[m];
-                if (m + 1 < a.B) v[j].y = p[m + 1];
+                if (m < a.B) v[j].x = load_in(a.in, a.in_fmt, i0 + m);
+                if (m + 1 < a.B) v[j].y = load_in(a.in, a.in_fmt, i0 + m + 1);
             }
         }
         float2* srow = spec + rf * M;
@@ -966,12 +1019,12 @@ __global__ void __launch_bounds__(kThreads + 32, 1) k_mac_slots(const MacArgs a)
 #pragma unroll
             for (int j = 0; j < kPts; ++j) v[j] = make_float2(0.f, 0.f);
             if (rf < rpt && row < a.n_rows) {
-                const float* p = a.in + row * a.in_chan_stride;
+                const long long i0 = (long long) row * a.in_chan_stride;
 #pragma unroll
                 for (int j = 0; j < kPts; ++j) {
                     const int m = 2 * (t + j * T::TPF);
-                    if (m < a.B) v[j].x = p[m];
-                    if (m + 1 < a.B) v[j].y = p[m + 1];
+                    if (m < a.B) v[j].x = load_in(a.in, a.in_fmt, i0 + m);
+                    if (m + 1 < a.B) v[j].y = load_in(a.in, a.in_fmt, i0 + m + 1);
                 }
             }
             float2* srow = sm.spec + rf * M;

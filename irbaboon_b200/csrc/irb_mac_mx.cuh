@@ -180,12 +180,12 @@ __global__ void __launch_bounds__(kThreads + 32, 2) k_mac_mx(const MacArgs a) {
 #pragma unroll
                 for (int j = 0; j < kPts; ++j) v[j] = make_float2(0.f, 0.f);
                 if (rf < nin) {
-                    const float* p = a.in + (r0 + rf) * a.in_chan_stride;
+                    const long long i0 = (long long) (r0 + rf) * a.in_chan_stride;
 #pragma unroll
                     for (int j = 0; j < kPts; ++j) {
                         const int m = 2 * (t + j * T::TPF);
-                        if (m < a.B) v[j].x = p[m];
-                        if (m + 1 < a.B) v[j].y = p[m + 1];
+                        if (m < a.B) v[j].x = load_in(a.in, a.in_fmt, i0 + m);
+                        if (m + 1 < a.B) v[j].y = load_in(a.in, a.in_fmt, i0 + m + 1);
                     }
                 }
                 float2* srow = tile + rf * M;

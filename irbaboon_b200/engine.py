@@ -56,6 +56,9 @@ _SIGS = {
     "irb_engine_synchronize": (ctypes.c_int, [_vp]),
     "irb_engine_submit": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int]),
     "irb_engine_wait": (ctypes.c_int, [_vp]),
+    "irb_engine_process_pcm": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int]),
+    "irb_engine_submit_pcm": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int]),
+    "irb_engine_process_device_pcm": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int]),
     "irb_engine_set_timing": (ctypes.c_int, [_vp, ctypes.c_int]),
     "irb_engine_get_timings": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int]),
     "irb_engine_state_bytes": (ctypes.c_size_t, [_vp]),
@@ -78,6 +81,7 @@ _SIGS = {
     "irb_group_bind": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "irb_group_reset": (ctypes.c_int, [_vp]),
     "irb_group_process": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int]),
+    "irb_group_process_pcm": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int]),
     "irb_group_state_bytes": (ctypes.c_size_t, [_vp]),
     "irb_convolve_periodic": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_convolve_nonperiodic": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int, _vp]),
@@ -128,6 +132,59 @@ def _ck(rc):
 
 def _ptr(a):
     return a.ctypes.data_as(_vp)
+
+
+# irb_sample_format (include/irb_b200.h): the streaming engine's block arrays in float32, int16 or packed little-endian 24-bit PCM
+IRB_SAMPLE_F32, IRB_SAMPLE_S16, IRB_SAMPLE_S24 = 0, 1, 2
+SAMPLE_FORMATS = {"f32": IRB_SAMPLE_F32, "s16": IRB_SAMPLE_S16, "s24": IRB_SAMPLE_S24}
+_FORMAT_DTYPE = {IRB_SAMPLE_F32: np.float32, IRB_SAMPLE_S16: np.int16, IRB_SAMPLE_S24: np.uint8}
+
+
+def sample_format(name):
+    """"f32" | "s16" | "s24" -> irb_sample_format code."""
+    f = SAMPLE_FORMATS.get(name)
+    if f is None:
+        raise ValueError("sample format %r: expected one of %s" % (name, ", ".join(SAMPLE_FORMATS)))
+    return f
+
+
+def _process_call(h, x, fin, out, fout, nb, group=False):
+    """irb_engine_process_pcm / irb_group_process_pcm.  On the one-block latency path the binding's own microseconds show:
+    float in and out take the float entry point (two ctypes arguments fewer), and the addresses go over as plain integers
+    (a.ctypes.data costs half of a.ctypes.data_as)."""
+    L = lib()
+    if fin == IRB_SAMPLE_F32 and fout == IRB_SAMPLE_F32:
+        return _ck((L.irb_group_process if group else L.irb_engine_process)(h, x.ctypes.data, out.ctypes.data, nb))
+    return _ck((L.irb_group_process_pcm if group else L.irb_engine_process_pcm)(h, x.ctypes.data, fin, out.ctypes.data, fout, nb))
+
+
+def _pcm_input(x, block_size):
+    """A block array and its sample format, taken from its dtype: int16 is 16-bit PCM, uint8 with a last axis of 3*block_size
+    bytes is packed 24-bit PCM, anything else is converted to float32.  -> (C-contiguous array, format, shape in samples)"""
+    x = np.asarray(x)
+    c = x.dtype.char
+    if c == "h":
+        x = np.ascontiguousarray(x)
+        return x, IRB_SAMPLE_S16, x.shape
+    if c == "B":
+        if x.ndim < 1 or x.shape[-1] != 3 * block_size:
+            raise ValueError("a uint8 (packed 24-bit) block array needs a last axis of 3*B = %d bytes, got shape %r" % (3 * block_size, x.shape))
+        x = np.ascontiguousarray(x)
+        return x, IRB_SAMPLE_S24, x.shape[:-1] + (block_size,)
+    x = np.ascontiguousarray(x, np.float32)
+    return x, IRB_SAMPLE_F32, x.shape
+
+
+def _pcm_output(shape, fmt, out):
+    """The output array for `shape` samples ([..][B]) in format fmt: a new one, or `out` once it is checked (its raw pointer goes
+    to the library).  Packed 24-bit arrays are uint8 with a last axis of 3*B."""
+    dt = _FORMAT_DTYPE[fmt]
+    shp = tuple(shape[:-1]) + (3 * shape[-1],) if fmt == IRB_SAMPLE_S24 else shape
+    if out is None:
+        return np.empty(shp, dt)
+    if not (isinstance(out, np.ndarray) and out.dtype == dt and out.shape == shp and out.flags.c_contiguous and out.flags.writeable):
+        raise ValueError("out must be a writable C-contiguous %s array of shape %r" % (np.dtype(dt).name, shp))
+    return out
 
 
 def _planar(a):
@@ -418,18 +475,17 @@ class Engine:
     def reset(self):
         _ck(lib().irb_engine_reset(self._h))
 
-    def process(self, x, out=None):
-        """x: host [n_blocks][n_channels][B] (or [n_channels][B]); returns the same shape."""
-        x = np.ascontiguousarray(x, np.float32)
-        shp = x.shape
-        nb = 1 if x.ndim == 2 else shp[0]
-        if x.ndim not in (2, 3) or shp[-2:] != (self.active_channels, self.block_size):
-            raise ValueError("input shape %r, expected [n_blocks][%d][%d]" % (shp, self.active_channels, self.block_size))
-        if out is None:
-            out = np.empty(shp, np.float32)
-        elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.shape == shp and out.flags.c_contiguous and out.flags.writeable):
-            raise ValueError("out must be a writable C-contiguous float32 array of shape %r" % (shp,))      # its raw pointer goes to the library
-        _ck(lib().irb_engine_process(self._h, _ptr(x), _ptr(out), nb))
+    def process(self, x, out=None, out_format="f32"):
+        """x: host [n_blocks][n_channels][B] (or [n_channels][B]); returns the same shape.  The input format follows x's dtype
+        (float32; int16 = 16-bit PCM; uint8 with a last axis of 3*B = packed 24-bit PCM), the output's is out_format
+        ("f32", "s16" or "s24"); integer PCM is converted on the device (include/irb_b200.h, irb_sample_format)."""
+        x, fin, shp = _pcm_input(x, self.block_size)
+        nb = 1 if len(shp) == 2 else shp[0]
+        if len(shp) not in (2, 3) or shp[-2:] != (self.active_channels, self.block_size):
+            raise ValueError("input shape %r, expected [n_blocks][%d][%d]" % (x.shape, self.active_channels, self.block_size))
+        fout = sample_format(out_format)
+        out = _pcm_output(shp, fout, out)
+        _process_call(self._h, x, fin, out, fout, nb)
         return out
 
     def process_callback(self, x):
@@ -440,17 +496,23 @@ class Engine:
         _ck(lib().irb_engine_process_callback(self._h, _ptr(x), _ptr(out), x.shape[0]))
         return out
 
-    def submit(self, x, out):
-        """Asynchronous multi-block call on pinned host arrays [n_blocks >= 2][n_channels][B]; pair with wait()."""
-        assert x.dtype == np.float32 and out.dtype == np.float32 and x.flags.c_contiguous and out.flags.c_contiguous and x.shape == out.shape
-        assert x.ndim == 3 and x.shape[1:] == (self.active_channels, self.block_size), x.shape
-        _ck(lib().irb_engine_submit(self._h, _ptr(x), _ptr(out), x.shape[0]))
+    def submit(self, x, out, out_format="f32"):
+        """Asynchronous multi-block call on pinned host arrays [n_blocks >= 2][n_channels][B]; pair with wait().  Formats as in
+        process(); both arrays are used in place."""
+        assert isinstance(x, np.ndarray) and x.flags.c_contiguous, "x must be a C-contiguous (pinned) array"
+        x2, fin, shp = _pcm_input(x, self.block_size)
+        assert x2 is x, "x must be float32, int16 or uint8: it is used in place"
+        assert len(shp) == 3 and shp[1:] == (self.active_channels, self.block_size), x.shape
+        fout = sample_format(out_format)
+        _pcm_output(shp, fout, out)
+        _ck(lib().irb_engine_submit_pcm(self._h, _ptr(x), fin, _ptr(out), fout, shp[0]))
 
     def wait(self):
         _ck(lib().irb_engine_wait(self._h))
 
-    def process_device(self, in_ptr, out_ptr, n_blocks=1):
-        _ck(lib().irb_engine_process_device(self._h, _vp(int(in_ptr)), _vp(int(out_ptr)), int(n_blocks)))
+    def process_device(self, in_ptr, out_ptr, n_blocks=1, in_format="f32", out_format="f32"):
+        """Raw DEVICE pointers to [n_blocks][channels][B] elements of the given formats ("f32", "s16", "s24"); asynchronous."""
+        _ck(lib().irb_engine_process_device_pcm(self._h, _vp(int(in_ptr)), sample_format(in_format), _vp(int(out_ptr)), sample_format(out_format), int(n_blocks)))
 
     def mac_only_device(self, acc_ptr):
         """bench-only (irb_b200_bench.h): the bare FDL multiply-accumulate into a device buffer"""
@@ -537,28 +599,31 @@ class MatrixEngine(Engine):
         arr = (ctypes.c_int * len(ids))(*ids)
         _ck(lib().irb_engine_bind_matrix(self._h, int(group_begin), int(group_end), arr))
 
-    def _out_shape(self, x):
-        return x.shape[:-2] + (self.n_outputs, self.block_size)
+    def _out_shape(self, shape):
+        return tuple(shape[:-2]) + (self.n_outputs, self.block_size)
 
-    def process(self, x, out=None):
-        """x: host [n_blocks][n_groups*ins][B] (or [n_groups*ins][B]) -> [n_blocks][n_groups*outs][B]."""
-        x = np.ascontiguousarray(x, np.float32)
-        if x.ndim not in (2, 3) or x.shape[-2:] != (self.n_channels, self.block_size):
+    def process(self, x, out=None, out_format="f32"):
+        """x: host [n_blocks][n_groups*ins][B] (or [n_groups*ins][B]) -> [n_blocks][n_groups*outs][B].  Formats as in
+        Engine.process."""
+        x, fin, ishp = _pcm_input(x, self.block_size)
+        if len(ishp) not in (2, 3) or ishp[-2:] != (self.n_channels, self.block_size):
             raise ValueError("input shape %r, expected [n_blocks][%d][%d]" % (x.shape, self.n_channels, self.block_size))
-        nb = 1 if x.ndim == 2 else x.shape[0]
-        shp = self._out_shape(x)
-        if out is None:
-            out = np.empty(shp, np.float32)
-        elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.shape == shp and out.flags.c_contiguous and out.flags.writeable):
-            raise ValueError("out must be a writable C-contiguous float32 array of shape %r" % (shp,))
-        _ck(lib().irb_engine_process(self._h, _ptr(x), _ptr(out), nb))
+        nb = 1 if len(ishp) == 2 else ishp[0]
+        fout = sample_format(out_format)
+        out = _pcm_output(self._out_shape(ishp), fout, out)
+        _process_call(self._h, x, fin, out, fout, nb)
         return out
 
-    def submit(self, x, out):
-        """Asynchronous multi-block call on pinned host arrays (in [n_blocks >= 2][n_groups*ins][B], out [..][n_groups*outs][B])."""
-        assert x.dtype == np.float32 and out.dtype == np.float32 and x.flags.c_contiguous and out.flags.c_contiguous
-        assert x.ndim == 3 and x.shape[1:] == (self.n_channels, self.block_size) and out.shape == self._out_shape(x), (x.shape, out.shape)
-        _ck(lib().irb_engine_submit(self._h, _ptr(x), _ptr(out), x.shape[0]))
+    def submit(self, x, out, out_format="f32"):
+        """Asynchronous multi-block call on pinned host arrays (in [n_blocks >= 2][n_groups*ins][B], out [..][n_groups*outs][B]).
+        Formats as in Engine.process."""
+        assert isinstance(x, np.ndarray) and x.flags.c_contiguous, "x must be a C-contiguous (pinned) array"
+        x2, fin, ishp = _pcm_input(x, self.block_size)
+        assert x2 is x, "x must be float32, int16 or uint8: it is used in place"
+        assert len(ishp) == 3 and ishp[1:] == (self.n_channels, self.block_size), x.shape
+        fout = sample_format(out_format)
+        _pcm_output(self._out_shape(ishp), fout, out)
+        _ck(lib().irb_engine_submit_pcm(self._h, _ptr(x), fin, _ptr(out), fout, ishp[0]))
 
     def process_stream(self, x):
         """Planar inputs x[n_groups*ins][n] -> outputs y[n_groups*outs][n], block by block (zero-padded to whole blocks)."""
@@ -621,15 +686,14 @@ class Group:
     def reset(self):
         _ck(lib().irb_group_reset(self._h))
 
-    def process(self, x, out=None):
-        x = np.ascontiguousarray(x, np.float32)
-        nb = 1 if x.ndim == 2 else x.shape[0]
-        assert x.shape[-2:] == (self.n_channels, self.block_size), x.shape
-        if out is None:
-            out = np.empty(x.shape, np.float32)
-        elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.shape == x.shape and out.flags.c_contiguous and out.flags.writeable):
-            raise ValueError("out must be a writable C-contiguous float32 array of shape %r" % (x.shape,))
-        _ck(lib().irb_group_process(self._h, _ptr(x), _ptr(out), nb))
+    def process(self, x, out=None, out_format="f32"):
+        """Host [n_blocks][n_channels][B] for all channels; formats as in Engine.process."""
+        x, fin, shp = _pcm_input(x, self.block_size)
+        nb = 1 if len(shp) == 2 else shp[0]
+        assert shp[-2:] == (self.n_channels, self.block_size), x.shape
+        fout = sample_format(out_format)
+        out = _pcm_output(shp, fout, out)
+        _process_call(self._h, x, fin, out, fout, nb, group=True)
         return out
 
     @property

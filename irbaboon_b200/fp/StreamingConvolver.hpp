@@ -10,8 +10,7 @@
 #endif
 #include <vector>
 
-struct irb_engine;
-struct irb_group;
+#include "../../include/irb_b200.h"
 
 namespace fp {
 namespace b200 {
@@ -32,6 +31,8 @@ public:
     void processBlock(AudioBuffer<float>& buffer);
     // dense [nBlocks][channels][blockSize] host arrays (pinned memory from irb_host_alloc is fastest)
     void process(const float* in, float* out, int nBlocks);
+    // the same with 16- or 24-bit integer PCM (or float) in and out, converted on the device (irb_engine_process_pcm)
+    void process(const void* in, irb_sample_format inFormat, void* out, irb_sample_format outFormat, int nBlocks);
 
     int getBlockSize() const { return blockSize; }
     int getNumChannels() const { return channels; }
@@ -65,6 +66,8 @@ public:
     void processBlock(const AudioBuffer<float>& in, AudioBuffer<float>& out);
     // dense host arrays: in [nBlocks][groups*ins][blockSize], out [nBlocks][groups*outs][blockSize]
     void process(const float* in, float* out, int nBlocks);
+    // the same in any irb_sample_format each (irb_engine_process_pcm)
+    void process(const void* in, irb_sample_format inFormat, void* out, irb_sample_format outFormat, int nBlocks);
 
     int getBlockSize() const { return blockSize; }
     int getNumInputs() const { return groups * ins; }
@@ -90,6 +93,8 @@ public:
     void bind(int channelBegin, int channelEnd, int irId);
     void reset();
     void process(const float* in, float* out, int nBlocks);   // dense [nBlocks][channels][blockSize] host arrays
+    // the same in any irb_sample_format each (irb_group_process_pcm)
+    void process(const void* in, irb_sample_format inFormat, void* out, irb_sample_format outFormat, int nBlocks);
     irb_group* handle() const { return group; }
 
 private:

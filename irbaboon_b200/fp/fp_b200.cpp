@@ -160,6 +160,9 @@ void StreamingConvolver::processBlock(AudioBuffer<float>& buffer) {
 void StreamingConvolver::process(const float* in, float* out, int nBlocks) {
     if (irb_engine_process(engine, in, out, nBlocks) != IRB_OK) raise("irb_engine_process");
 }
+void StreamingConvolver::process(const void* in, irb_sample_format inFormat, void* out, irb_sample_format outFormat, int nBlocks) {
+    if (irb_engine_process_pcm(engine, in, inFormat, out, outFormat, nBlocks) != IRB_OK) raise("irb_engine_process_pcm");
+}
 
 // ---- MatrixConvolver ------------------------------------------------------------------------------------
 MatrixConvolver::MatrixConvolver(int blockSize_, int maxPartitions, int groups_, int ins_, int outs_, int numIRs, int device)
@@ -194,6 +197,9 @@ void MatrixConvolver::processBlock(const AudioBuffer<float>& in, AudioBuffer<flo
 void MatrixConvolver::process(const float* in, float* out, int nBlocks) {
     if (irb_engine_process(engine, in, out, nBlocks) != IRB_OK) raise("irb_engine_process");
 }
+void MatrixConvolver::process(const void* in, irb_sample_format inFormat, void* out, irb_sample_format outFormat, int nBlocks) {
+    if (irb_engine_process_pcm(engine, in, inFormat, out, outFormat, nBlocks) != IRB_OK) raise("irb_engine_process_pcm");
+}
 
 // ---- MultiGpuConvolver ----------------------------------------------------------------------------------
 MultiGpuConvolver::MultiGpuConvolver(const std::vector<int>& devices, int blockSize, int maxPartitions, int channels, int numIRs) {
@@ -212,6 +218,9 @@ void MultiGpuConvolver::reset() {
 }
 void MultiGpuConvolver::process(const float* in, float* out, int nBlocks) {
     if (irb_group_process(group, in, out, nBlocks) != IRB_OK) raise("irb_group_process");
+}
+void MultiGpuConvolver::process(const void* in, irb_sample_format inFormat, void* out, irb_sample_format outFormat, int nBlocks) {
+    if (irb_group_process_pcm(group, in, inFormat, out, outFormat, nBlocks) != IRB_OK) raise("irb_group_process_pcm");
 }
 
 // ---- PluginConvolver ------------------------------------------------------------------------------------
