@@ -231,8 +231,9 @@ def c5(eng, synth, args):
                     "captures_per_s_device": nb / dev, "min_bytes_per_capture": 2 * n * 4, "four_step_bytes_per_capture": four_step,
                     "device_gbs_at_four_step_bytes": nb * four_step / dev / 1e9, "frac_of_measured_peak": nb * four_step / dev / 1e9 / peak(),
                     "peak_abs": float(np.abs(y).max())}
-    # secondary (SURVEY 8d): the Farina form of the same capture, convolveNonPeriodic(capture, inverse sweep) at N = 2^21,
-    # one irb_convolve_nonperiodic call per capture (no batched entry point: the plug-in itself deconvolves by division)
+    # secondary (SURVEY 8d): the Farina form of the same capture, convolveNonPeriodic(capture, inverse sweep) at N = 2^21, as the
+    # reference runs it (one irb_convolve_nonperiodic call per capture, the full result) and batched (irb_convolve_batch, every
+    # capture at once, only the window from 4 800 samples before lag len_sweep - 1 to 48 000 after it)
     sweep_inv = eng.ess(n / SR, SR, 20.0, 24000.0, 0.0, True).astype(np.float32)
     eng.convolve_nonperiodic(caps[0], sweep_inv)
     kf, ts, dev = min(nb, 8), [], []
@@ -244,6 +245,19 @@ def c5(eng, synth, args):
     out["farina_variant"] = {"what": "convolveNonPeriodic(capture, ExpSineSweep inverse filter), N = 2^21, one call per capture, pageable result",
                              "captures": kf, "wall_seconds_per_capture_median": float(np.median(ts)), "device_seconds_per_capture_median": float(np.median(dev)),
                              "output_samples": int(yf.shape[1])}
+    off, win = len(sweep_inv) - 1 - 4800, 4800 + 48000
+    wres = eng.pinned_empty((nb, win))
+    eng.convolve_batch(caps[:2], sweep_inv, off, win, out=wres[:2])
+    ts = []
+    for _ in range(3):
+        t0 = time.perf_counter()
+        eng.convolve_batch(caps, sweep_inv, off, win, out=wres)
+        ts.append((time.perf_counter() - t0, eng.last_compute_ms() * 1e-3))
+    wall, dev_b = min(ts)
+    out["farina_variant_batched"] = {"what": "irb_convolve_batch of all captures with the inverse filter, N = 2^21, pinned host buffers, window [%d, %d)" % (off, off + win),
+                                     "captures": nb, "wall_seconds": wall, "wall_seconds_per_capture": wall / nb, "device_seconds": dev_b,
+                                     "device_seconds_per_capture": dev_b / nb, "output_samples": win}
+    eng.pinned_free(wres)
     try:
         import oracle
         if oracle.have_reference():

@@ -209,6 +209,20 @@ int irb_convolve_periodic(const float* x, int ch_x, int len_x, const float* h, i
  * layouts the reference rejects (it returns a cleared copy of the input there, :271-275). */
 int irb_convolve_nonperiodic(const float* x, int ch_x, int len_x, const float* h, int ch_h, int len_h, float* out);
 
+/* `batch` signals x[batch][len_x], each linearly convolved with an IR h[h_batch][len_h], h_batch = 1 (one IR shared by every
+ * signal) or batch (signal b with IR b).  N = nextPowerOfTwo(len_x + len_h - 1), at least 16, at most 2^22, as irb_convolve_nonperiodic.
+ * Only the window [out_offset, out_offset + out_len) of each full result is written: out[batch][out_len].
+ * Requires 0 <= out_offset and out_offset + out_len <= len_x + len_h - 1.
+ * With out_offset = 0 and out_len = len_x + len_h - 1, row b is bit-identical to irb_convolve_nonperiodic(x[b], 1, len_x, h[b or 0], 1, len_h).
+ * Every argument error (null pointer, batch < 1, h_batch not 1 or batch, an empty signal, out_len < 1, a window outside the
+ * result, a result above 2^22 points) is IRB_ERR_ARG, returned before any CUDA call.  The batch runs in sub-batches with uploads,
+ * kernels and downloads overlapped; only the window's samples are written to device memory and copied back. */
+int irb_convolve_batch(const float* x, int batch, int len_x, const float* h, int h_batch, int len_h, int out_offset, int out_len, float* out);
+/* The same on DEVICE-resident x_dev and out_dev.  h may be in host or device memory, as `den` of irb_deconvolve_batch_device.
+ * No staging copies when N > 4096, x_dev is 8-byte aligned and len_x even, and a per-signal h (h_batch = batch) is device memory,
+ * 8-byte aligned, with len_h even; any other float alignment is accepted and goes through staged device-to-device copies. */
+int irb_convolve_batch_device(const float* x_dev, int batch, int len_x, const float* h, int h_batch, int len_h, int out_offset, int out_len, float* out_dev);
+
 /* fp::convolution::deconvolve (fp/convolution.hpp:38, fp/convolution.cpp:351-403): spectral division
  * FFT(num)/FFT(den) at N = nextPowerOfTwo(max(len_num, len_den)) (circular), optional 3x 1/13-octave
  * averagingFilter, inverse FFT, ir::shifteroo when the phase is dropped.  out[N] (or [batch][N]).

@@ -1,5 +1,5 @@
 // irb_spectral.cu -- host side of the single-large-FFT entry points of include/irb_b200.h:
-// irb_convolve_nonperiodic, irb_deconvolve(_batch), irb_averaging_filter, irb_fft_transform,
+// irb_convolve_nonperiodic, irb_convolve_batch(_device), irb_deconvolve(_batch), irb_averaging_filter, irb_fft_transform,
 // irb_fft_inv_transform, irb_invert_filter, irb_ess_generate.  Every arithmetic step is a kernel of
 // irb_spectral.cuh; the host only sizes buffers, copies and launches.
 #include <algorithm>
@@ -21,25 +21,36 @@ using irbh::g_launches;
 
 constexpr int kMinM = 8;                 // smallest half size the Stockham passes take (N = 16)
 constexpr int kMaxBigM = 1 << 21;        // N up to 2^22 (87 s at 48 kHz)
+constexpr int kMaxGridY = 65535;         // largest grid.y of a launch: batch items per launch
 
-template <int L, bool INV>
-int launch_line_t(const irb::LineArgs& a, int batch, cudaStream_t st) {
+// Real-output window of an inverse transform's last pass (irb::LineWindow): floats [off, off + len) of each batch item's real
+// result go to out + b * stride - off; len < 0: the whole complex result is stored as float2 (irb::k_line_fft)
+struct OutWindow {
+    long long off = 0, stride = 0;
+    int len = -1;
+};
+
+template <int L, bool INV, bool WIN = false>
+int launch_line_t(const irb::LineArgs& a, const OutWindow& w, int batch, cudaStream_t st) {
     using T = irb::LineTile<L>;
     static thread_local int configured_dev = -1;
     int dev = 0;
     CK(cudaGetDevice(&dev));
     if (configured_dev != dev) {
-        CK(cudaFuncSetAttribute(irb::k_line_fft<L, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) T::SMEM));
+        if constexpr (WIN) CK(cudaFuncSetAttribute(irb::k_line_fft_win<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) T::SMEM));
+        else CK(cudaFuncSetAttribute(irb::k_line_fft<L, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) T::SMEM));
         configured_dev = dev;
     }
     dim3 grid((a.n_lines + T::C - 1) / T::C, batch);
-    irb::k_line_fft<L, INV><<<grid, irb::kThreads, T::SMEM, st>>>(a);
+    if constexpr (WIN) irb::k_line_fft_win<L><<<grid, irb::kThreads, T::SMEM, st>>>(a, irb::LineWindow{w.off, w.stride, w.len});
+    else irb::k_line_fft<L, INV><<<grid, irb::kThreads, T::SMEM, st>>>(a);
     g_launches++;
     CK(cudaGetLastError());
     return 0;
 }
-int launch_line(int L, bool inv, const irb::LineArgs& a, int batch, cudaStream_t st) {
-#define IRB_LINE_CASE(LL) case LL: return inv ? launch_line_t<LL, true>(a, batch, st) : launch_line_t<LL, false>(a, batch, st);
+int launch_line(int L, bool inv, const irb::LineArgs& a, int batch, cudaStream_t st, const OutWindow& w = {}) {
+    if (w.len >= 0 && !inv) return fail(IRB_ERR_ARG, "an output window needs an inverse transform");
+#define IRB_LINE_CASE(LL) case LL: return w.len >= 0 ? launch_line_t<LL, true, true>(a, w, batch, st) : inv ? launch_line_t<LL, true>(a, w, batch, st) : launch_line_t<LL, false>(a, w, batch, st);
     switch (L) {
         IRB_LINE_CASE(8) IRB_LINE_CASE(16) IRB_LINE_CASE(32) IRB_LINE_CASE(64) IRB_LINE_CASE(128) IRB_LINE_CASE(256)
         IRB_LINE_CASE(512) IRB_LINE_CASE(1024) IRB_LINE_CASE(2048)
@@ -101,20 +112,20 @@ struct Plan {
         return 0;
     }
     // batch items at in + b*in_stride -> out + b*out_stride (float2 units); real_len >= 0: `in` is real data.
-    // tmp: M complex per batch item (two-pass only; may alias neither in nor out)
+    // tmp: M complex per batch item (two-pass only; may alias neither in nor out).  win: real-output window of the result.
     int run(const void* in, long long in_stride, int real_len, float2* out, long long out_stride, float2* tmp, int batch, bool inv, float scale,
-            cudaStream_t st) const {
+            cudaStream_t st, const OutWindow& win = {}) const {
         irb::LineArgs a{};
         if (M1 == 1) {                                           // batch items are the lines
             a.in = in; a.out = out; a.in_elem_stride = 1; a.in_line_stride = in_stride; a.in_batch_stride = 0;
             a.out_elem_stride = 1; a.out_line_stride = out_stride; a.out_batch_stride = 0;
             a.n_lines = batch; a.in_real_len = real_len; a.tw_M = 0; a.scale = scale; a.W = W2;
-            if (real_len >= 0 && batch > 1) {
-                // the real-input bounds check is per batch item: run items one grid.y slice each
+            if ((real_len >= 0 || win.len >= 0) && batch > 1) {
+                // the real-input bounds check and the output window are per batch item: run items one grid.y slice each
                 a.in_line_stride = 0; a.in_batch_stride = in_stride; a.out_line_stride = 0; a.out_batch_stride = out_stride; a.n_lines = 1;
-                return launch_line(M2, inv, a, batch, st);
+                return launch_line(M2, inv, a, batch, st, win);
             }
-            return launch_line(M2, inv, a, 1, st);
+            return launch_line(M2, inv, a, 1, st, win);
         }
         // pass 1: M2 column transforms of length M1 (element n1 of line n2 at n1*M2 + n2), twiddle exp(-+2 pi i n2 k1 / M)
         a.in = in; a.out = tmp; a.in_elem_stride = M2; a.in_line_stride = 1; a.in_batch_stride = in_stride;
@@ -126,7 +137,7 @@ struct Plan {
         a.in = tmp; a.out = out; a.in_elem_stride = 1; a.in_line_stride = M2; a.in_batch_stride = M;
         a.out_elem_stride = M1; a.out_line_stride = 1; a.out_batch_stride = out_stride;
         a.n_lines = M1; a.in_real_len = -1; a.tw_M = 0; a.scale = scale; a.W = W2;
-        return launch_line(M2, inv, a, batch, st);
+        return launch_line(M2, inv, a, batch, st, win);
     }
     // ---- the fused pipeline of the big transforms (M1 > 1); rows = [batch][M1][M2] ------------------------------
     // column pass of the forward transform: signal (real when real_len >= 0) -> rows, inter-pass twiddle applied
@@ -158,13 +169,13 @@ struct Plan {
         a.Nhi = Nhi; a.Nlo = Nlo; a.Mhi = Thi; a.Mlo = Tlo;
         return launch_pair(M2, a, batch, st);
     }
-    // column pass of the inverse transform: rows -> out (natural order), scaled
-    int cols_inv(const float2* rows, float2* out, long long out_stride, int batch, float scale, cudaStream_t st) const {
+    // column pass of the inverse transform: rows -> out (natural order), scaled; win: real-output window
+    int cols_inv(const float2* rows, float2* out, long long out_stride, int batch, float scale, cudaStream_t st, const OutWindow& win = {}) const {
         irb::LineArgs a{};
         a.in = rows; a.out = out; a.in_elem_stride = M2; a.in_line_stride = 1; a.in_batch_stride = M;
         a.out_elem_stride = M2; a.out_line_stride = 1; a.out_batch_stride = out_stride;
         a.n_lines = M2; a.in_real_len = -1; a.tw_M = 0; a.scale = scale; a.W = W1;
-        return launch_line(M1, true, a, batch, st);
+        return launch_line(M1, true, a, batch, st, win);
     }
 };
 
@@ -246,84 +257,37 @@ int fft_size_for(int len, int* N) {
 
 }  // namespace
 
-extern "C" {
+// One batched spectral product, the core of the batched division and of the (batched) linear convolution:
+//   y_b = IFFT_N(FFT_N(x_b) op FFT_N(h_b)),  h_b = h[0] (h_batch == 1, one operand shared by every item) or h[b] (h_batch == batch),
+// both signals zero-padded to N; op is the per-bin product, or the division tools::complexDivCartesian carried out as a product with
+// the reciprocal spectrum.  win.len < 0: each row of out is the whole N-point result; else the rows hold win.len floats, the
+// window [win.off, win.off + win.len) of each result (win.stride == win.len).
+struct BatchJob {
+    const float* x; int batch, len_x;
+    const float* h; int h_batch, len_h;          // host or device memory
+    int N;
+    bool divide;
+    OutWindow win;
+    float* out;
+    long long out_row() const { return win.len >= 0 ? win.len : N; }
+};
 
-// fp::convolution::convolveNonPeriodic (fp/convolution.cpp:246-347)
-int irb_convolve_nonperiodic(const float* x, int ch_x, int len_x, const float* h, int ch_h, int len_h, float* out) {
-    if (!x || !h || !out) return fail(IRB_ERR_ARG, "null argument");
-    if (len_x < 1 || len_h < 1 || ch_x < 1 || ch_h < 1) return fail(IRB_ERR_ARG, "empty input");
-    if (!((ch_x == 1 || ch_x == 2) && (ch_h == 1 || ch_h == 2)))
-        return fail(IRB_ERR_LAYOUT, "audio has %d channels and the IR %d: only mono/stereo layouts exist (fp/convolution.cpp:259-275)", ch_x, ch_h);
-    const long long Lout = (long long) len_x + len_h - 1;
-    int N = 1;
-    while (N < Lout) { N *= 2; if (N > 2 * kMaxBigM) return fail(IRB_ERR_ARG, "result of %lld samples needs an FFT above 2^22 points", Lout); }
-    if (N < 2 * kMinM) N = 2 * kMinM;                    // a longer zero-padded transform yields the same linear convolution
-    const int M = N / 2, dev = irbh::current_device();
-    CK(cudaSetDevice(dev));
-    Plan plan;
-    int rc = plan.init(dev, M);
-    if (rc) return rc;
-    DevBuf dx, dh, dhf, Zx, Zh, tmp, dy;
-    irbh::StreamGuard sg;                                // after the buffers: drains the stream before they return to the pool
-    if ((rc = sg.create())) return rc;
-    cudaStream_t st = sg.s;
-    const bool fold = ch_h == 2 && ch_x == 1;            // IRStereoAudioMono -> sumToMono (:302)
-    const int n_ir = (ch_h == 2 && ch_x == 2) ? 2 : 1;   // IRStereoAudioStereo is channel-wise (:320-323)
-    const long long lxe = (len_x + 1) & ~1LL, lhe = (len_h + 1) & ~1LL;     // even strides keep float2 loads aligned
-    if ((rc = dx.alloc(sizeof(float) * lxe * ch_x, true)) || (rc = dh.alloc(sizeof(float) * lhe * ch_h, true)) || (rc = dhf.alloc(sizeof(float) * lhe, true)) ||
-        (rc = Zx.alloc(sizeof(float2) * (size_t) M * ch_x, false)) || (rc = Zh.alloc(sizeof(float2) * (size_t) M * n_ir, false)) ||
-        (rc = tmp.alloc(sizeof(float2) * (size_t) M * 2, false)) || (rc = dy.alloc(sizeof(float2) * (size_t) M * ch_x, false)))
-        return rc;
-    for (int c = 0; c < ch_x; ++c) CK(cudaMemcpyAsync(dx.as<float>() + c * lxe, x + (size_t) c * len_x, sizeof(float) * len_x, cudaMemcpyHostToDevice, st));
-    for (int c = 0; c < ch_h; ++c) CK(cudaMemcpyAsync(dh.as<float>() + c * lhe, h + (size_t) c * len_h, sizeof(float) * len_h, cudaMemcpyHostToDevice, st));
-    irbh::ComputeTimer tm;
-    if ((rc = tm.init(st)) || (rc = tm.begin())) return rc;
-    const float* hsrc = dh.as<float>();
-    if (fold) {
-        irb::k_fold_mono<<<grid1(len_h, 1), 256, 0, st>>>(dh.as<float>(), dh.as<float>() + lhe, dhf.as<float>(), len_h);
-        LAUNCHED();
-        hsrc = dhf.as<float>();
-    }
-    if (plan.big()) {
-        // column passes, then one fused kernel per row pair: row FFT, bins of the audio times bins of its IR, inverse row FFT
-        if ((rc = plan.cols_fwd(dx.p, lxe / 2, len_x, Zx.as<float2>(), ch_x, st)) || (rc = plan.cols_fwd(hsrc, lhe / 2, len_h, Zh.as<float2>(), n_ir, st)) ||
-            (rc = plan.rows_to_split_spectrum(Zh.as<float2>(), tmp.as<float2>(), n_ir, false, st)) ||
-            (rc = plan.rows_binop(Zx.as<float2>(), tmp.as<float2>(), n_ir == 2 ? M : 0, ch_x, st)) ||
-            (rc = plan.cols_inv(Zx.as<float2>(), dy.as<float2>(), M, ch_x, 1.0f / (float) N, st)))
-            return rc;
-    } else {
-        if ((rc = plan.run(dx.p, lxe / 2, len_x, Zx.as<float2>(), M, tmp.as<float2>(), ch_x, false, 1.0f, st))) return rc;
-        if ((rc = plan.run(hsrc, lhe / 2, len_h, Zh.as<float2>(), M, tmp.as<float2>(), n_ir, false, 1.0f, st))) return rc;
-        // per channel: bins of the audio times bins of its IR (fp/convolution.cpp:326-335), in place on Zx
-        irb::k_spec_fused<false><<<grid1(M / 2 + 1, ch_x), 256, 0, st>>>(Zx.as<float2>(), M, Zh.as<float2>(), n_ir == 2 ? M : 0, Zx.as<float2>(), M, M, plan.WN);
-        LAUNCHED();
-        if ((rc = plan.run(Zx.p, M, -1, dy.as<float2>(), M, tmp.as<float2>(), ch_x, true, 1.0f / (float) N, st))) return rc;
-    }
-    if ((rc = tm.end())) return rc;
-    for (int c = 0; c < ch_x; ++c)
-        CK(cudaMemcpyAsync(out + (size_t) c * Lout, dy.as<float>() + (size_t) c * N, sizeof(float) * Lout, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return tm.collect();
-}
-
-// fp::convolution::deconvolve (fp/convolution.cpp:351-403) for `batch` numerators against one denominator.
-// nums: [batch][len_num] (channel 0 of each capture, as tools::fftTransform reads only channel 0, fp/tools.cpp:328)
-// out: [batch][N], N = nextPowerOfTwo(max(len_num, len_den))
 // The batch runs in sub-batches through a three-stage pipeline (upload i+1 | kernels i | download i-1) over
 // double-buffered device memory; a sub-batch is small enough for its intermediate spectra to stay in the L2.
-// device_io: captures and results lie in device memory, so the smoothed path reports irb_last_compute_ms() as the device span from its
+// Per-item operands are uploaded and transformed with their sub-batch.  The smoothing path (division only: a shared
+// denominator, no window) is fp::convolution::deconvolve's averagingFilter between the division and the inverse transform.
+// device_io: inputs and results lie in device memory, so the smoothed path reports irb_last_compute_ms() as the device span from its
 // first to its last kernel (groups overlap); from host buffers it is the sum of the kernel sections' spans, copies excluded.
-static int deconvolve_batch_staged(const float* nums, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
-                                   int include_amplitude, float* out, bool device_io = false) {
-    if (!nums || !den || !out) return fail(IRB_ERR_ARG, "null argument");
-    if (batch < 1 || len_num < 1 || len_den < 1) return fail(IRB_ERR_ARG, "empty input");
-    int N = 0, rc;
-    if ((rc = fft_size_for(len_num > len_den ? len_num : len_den, &N))) return rc;
-    const int M = N / 2, dev = irbh::current_device();
+static int batch_staged(const BatchJob& J, double sample_rate, int smoothing, int include_phase, int include_amplitude, bool device_io) {
+    const float* nums = J.x;
+    const int batch = J.batch, len_num = J.len_x, len_den = J.len_h, N = J.N, M = N / 2, dev = irbh::current_device();
+    const bool per_item = J.h_batch > 1;
+    const long long out_row = J.out_row();
+    int rc;
     CK(cudaSetDevice(dev));
     Plan plan;
     if ((rc = plan.init(dev, M))) return rc;
-    struct Slot { DevBuf dn, Zn, dy, dy2, tmp; cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr, t0 = nullptr, t1 = nullptr;
+    struct Slot { DevBuf dn, Zn, dy, dy2, tmp, dh, Zh, Bh; cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr, t0 = nullptr, t1 = nullptr;
                   bool dn_busy = false, dy_busy = false, timed = false;
                   ~Slot() { for (cudaEvent_t e : {ev_in, ev_done, ev_out, t0, t1}) if (e) cudaEventDestroy(e); } } slot[4];   // [2], [3]: the smoothing path's last phase
     // smoothing runs in up to kLanes groups of captures at once, each on its own compute stream with its own spectrum array and
@@ -342,10 +306,14 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
     if ((rc = sg.create()) || (rc = sg_in.create()) || (rc = sg_out.create())) return rc;
     cudaStream_t st = sg.s;
     const long long lne = (len_num + 1) & ~1LL, lde = (len_den + 1) & ~1LL;
-    // captures per sub-batch: about 48 MB of spectra (IRB_DECONV_SUB overrides), never more than the batch
+    const bool fused = plan.big() && !smoothing;
+    // items per sub-batch: about 48 MB of spectra (IRB_DECONV_SUB overrides), never more than the batch; per-item operands add
+    // their spectrum (and, on the fused path, its split copy).  The per-item kernels run one item per grid.y slice, so a sub-batch
+    // also stays within the 65 535 slices a launch can have (many short signals).
+    const int spectra = per_item ? (fused ? 3 : 2) : 1;
     const int sub_pref = irbh::g_tuning.deconv_sub;
-    int sub = sub_pref > 0 ? sub_pref : (int) std::max<long long>(1, (48LL << 20) / ((long long) sizeof(float2) * M));
-    sub = std::min(sub, batch);
+    int sub = sub_pref > 0 ? sub_pref : (int) std::max<long long>(1, (48LL << 20) / ((long long) sizeof(float2) * M * spectra));
+    sub = std::min(std::min(sub, batch), kMaxGridY);
     // smoothing: the running sum is one sequential chain per capture and costs the same few milliseconds for 1 or 500 captures,
     // so a whole GROUP of captures is smoothed at once, between a first phase (upload | forward transform, split, divide) and a
     // last phase (merge, inverse transform | download) that both run in sub-batches with their copies overlapped; the batch is
@@ -354,22 +322,26 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
     const long long grp_cap = irbh::g_tuning.deconv_group_cap > 0 ? irbh::g_tuning.deconv_group_cap : (3LL << 29) / (20LL * (M + 1));
     const int grp = smoothing ? (int) std::min<long long>(batch, std::max<long long>(sub, std::min<long long>((batch + lanes_pref - 1) / lanes_pref, grp_cap))) : batch;
     const int ngroups = (batch + grp - 1) / grp, nlanes = std::min(ngroups, lanes_pref);
-    const bool fused = plan.big() && !smoothing;
     const float smooth_per_avg = 1.0 / 13.0;                                          // fp/convolution.cpp:390 (a float there)
     const int nslots = batch > sub ? 2 : 1;
     for (int i = 0; i < (smoothing ? 2 * nslots : nslots); ++i) {
         Slot& q = slot[i < nslots ? i : 2 + (i - nslots)];
         const bool first = i < nslots, last = !smoothing || !first;                // which phase(s) of the pipeline the slot serves
         if ((first && (rc = q.dn.alloc(sizeof(float) * lne * sub, true))) || (rc = q.Zn.alloc(sizeof(float2) * (size_t) M * sub, false)) ||
-            (last && (rc = q.dy.alloc(sizeof(float2) * (size_t) M * sub, false))))
+            (last && (rc = q.dy.alloc(sizeof(float) * (size_t) out_row * sub, false))))
             return rc;
         if (!fused && (rc = q.tmp.alloc(sizeof(float2) * (size_t) M * sub, false))) return rc;
         if (last && !include_phase && (rc = q.dy2.alloc(sizeof(float) * (size_t) N * sub, false))) return rc;
+        if (per_item && ((rc = q.dh.alloc(sizeof(float) * lde * sub, true)) || (rc = q.Zh.alloc(sizeof(float2) * (size_t) M * sub, false)) ||
+                         (fused && (rc = q.Bh.alloc(sizeof(float2) * (size_t) M * sub, false)))))
+            return rc;
         CK(cudaEventCreateWithFlags(&q.ev_in, cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&q.ev_done, cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&q.ev_out, cudaEventDisableTiming)); CK(cudaEventCreate(&q.t0)); CK(cudaEventCreate(&q.t1));
     }
-    if ((rc = dd.alloc(sizeof(float) * lde, true)) || (rc = Zd.alloc(sizeof(float2) * (size_t) M, false)) || (rc = dtmp.alloc(sizeof(float2) * (size_t) M, false))) return rc;
-    if (fused && (rc = Bd.alloc(sizeof(float2) * (size_t) M, false))) return rc;
+    if (!per_item) {
+        if ((rc = dd.alloc(sizeof(float) * lde, true)) || (rc = Zd.alloc(sizeof(float2) * (size_t) M, false)) || (rc = dtmp.alloc(sizeof(float2) * (size_t) M, false))) return rc;
+        if (fused && (rc = Bd.alloc(sizeof(float2) * (size_t) M, false))) return rc;
+    }
     cudaStream_t lst[kLanes];
     for (int l = 0; l < kLanes; ++l) lst[l] = st;
     cudaEvent_t ev_den = nullptr, ev_join[kLanes] = {};
@@ -385,15 +357,17 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
         }
     }
     irbh::set_last_compute_ms(0.0);
-    // the denominator's spectrum, once
-    CK(cudaMemcpyAsync(dd.p, den, sizeof(float) * len_den, cudaMemcpyDefault, st));
-    if (fused) {
-        if ((rc = plan.cols_fwd(dd.p, lde / 2, len_den, Zd.as<float2>(), 1, st)) || (rc = plan.rows_to_split_spectrum(Zd.as<float2>(), Bd.as<float2>(), 1, true, st))) return rc;
-    } else {
-        if ((rc = plan.run(dd.p, lde / 2, len_den, Zd.as<float2>(), M, dtmp.as<float2>(), 1, false, 1.0f, st))) return rc;
-        if (smoothing) {
-            irb::k_spec_split<<<grid1(M + 1, 1), 256, 0, st>>>(Zd.as<float2>(), M, Sd.as<float2>(), M + 1, M, 0, plan.WN);
-            LAUNCHED();
+    // a shared operand's spectrum, once (the reciprocal for a division)
+    if (!per_item) {
+        CK(cudaMemcpyAsync(dd.p, J.h, sizeof(float) * len_den, cudaMemcpyDefault, st));
+        if (fused) {
+            if ((rc = plan.cols_fwd(dd.p, lde / 2, len_den, Zd.as<float2>(), 1, st)) || (rc = plan.rows_to_split_spectrum(Zd.as<float2>(), Bd.as<float2>(), 1, J.divide, st))) return rc;
+        } else {
+            if ((rc = plan.run(dd.p, lde / 2, len_den, Zd.as<float2>(), M, dtmp.as<float2>(), 1, false, 1.0f, st))) return rc;
+            if (smoothing) {
+                irb::k_spec_split<<<grid1(M + 1, 1), 256, 0, st>>>(Zd.as<float2>(), M, Sd.as<float2>(), M + 1, M, 0, plan.WN);
+                LAUNCHED();
+            }
         }
     }
     double total_ms = 0.0;
@@ -406,10 +380,13 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
         q.timed = false;
         return 0;
     };
-    // upload of a sub-batch into q.dn (after the kernels that last used the slot), and the compute stream cs waiting for it
+    // upload of a sub-batch into q.dn (and its per-item operands into q.dh) after the kernels that last used the slot, and the
+    // compute stream cs waiting for it
     auto upload = [&](Slot& q, int b0, int nb, cudaStream_t cs) -> int {
         if (q.dn_busy) CK(cudaStreamWaitEvent(sg_in.s, q.ev_done, 0));
         CK(cudaMemcpy2DAsync(q.dn.p, sizeof(float) * lne, nums + (size_t) b0 * len_num, sizeof(float) * len_num, sizeof(float) * len_num, nb, cudaMemcpyDefault, sg_in.s));
+        if (per_item)
+            CK(cudaMemcpy2DAsync(q.dh.p, sizeof(float) * lde, J.h + (size_t) b0 * len_den, sizeof(float) * len_den, sizeof(float) * len_den, nb, cudaMemcpyDefault, sg_in.s));
         CK(cudaEventRecord(q.ev_in, sg_in.s));
         CK(cudaStreamWaitEvent(cs, q.ev_in, 0));
         return 0;
@@ -426,13 +403,15 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
         else CK(cudaEventRecord(q.t1, cs));
         CK(cudaEventRecord(q.ev_done, cs));
         CK(cudaStreamWaitEvent(sg_out.s, q.ev_done, 0));
-        CK(cudaMemcpyAsync(out + (size_t) b0 * N, res, sizeof(float) * (size_t) N * nb, cudaMemcpyDefault, sg_out.s));
+        CK(cudaMemcpyAsync(J.out + (size_t) b0 * out_row, res, sizeof(float) * (size_t) out_row * nb, cudaMemcpyDefault, sg_out.s));
         CK(cudaEventRecord(q.ev_out, sg_out.s));
         q.dy_busy = true;
         return 0;
     };
     int it = 0;
     if (!smoothing) {
+        const float inv_n = 1.0f / (float) N;
+        const OutWindow win{J.win.off, out_row, J.win.len};
         for (int b0 = 0; b0 < batch; b0 += sub, ++it) {
             Slot& q = slot[it % nslots];
             const int nb = std::min(sub, batch - b0);
@@ -441,14 +420,28 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
             CK(cudaEventRecord(q.t0, st));
             q.timed = true;
             if (fused) {
-                if ((rc = plan.cols_fwd(q.dn.p, lne / 2, len_num, q.Zn.as<float2>(), nb, st)) || (rc = plan.rows_binop(q.Zn.as<float2>(), Bd.as<float2>(), 0, nb, st)) ||
-                    (rc = plan.cols_inv(q.Zn.as<float2>(), q.dy.as<float2>(), M, nb, 1.0f / (float) N, st)))
+                const float2* B = Bd.as<float2>();
+                if (per_item) {
+                    if ((rc = plan.cols_fwd(q.dh.p, lde / 2, len_den, q.Zh.as<float2>(), nb, st)) ||
+                        (rc = plan.rows_to_split_spectrum(q.Zh.as<float2>(), q.Bh.as<float2>(), nb, J.divide, st)))
+                        return rc;
+                    B = q.Bh.as<float2>();
+                }
+                if ((rc = plan.cols_fwd(q.dn.p, lne / 2, len_num, q.Zn.as<float2>(), nb, st)) || (rc = plan.rows_binop(q.Zn.as<float2>(), B, per_item ? M : 0, nb, st)) ||
+                    (rc = plan.cols_inv(q.Zn.as<float2>(), q.dy.as<float2>(), M, nb, inv_n, st, win)))
                     return rc;
             } else {
+                const float2* B = Zd.as<float2>();
+                if (per_item) {
+                    if ((rc = plan.run(q.dh.p, lde / 2, len_den, q.Zh.as<float2>(), M, q.tmp.as<float2>(), nb, false, 1.0f, st))) return rc;
+                    B = q.Zh.as<float2>();
+                }
                 if ((rc = plan.run(q.dn.p, lne / 2, len_num, q.Zn.as<float2>(), M, q.tmp.as<float2>(), nb, false, 1.0f, st))) return rc;
-                irb::k_spec_fused<true><<<grid1(M / 2 + 1, nb), 256, 0, st>>>(q.Zn.as<float2>(), M, Zd.as<float2>(), 0, q.Zn.as<float2>(), M, M, plan.WN);
+                const long long bs = per_item ? M : 0;
+                if (J.divide) irb::k_spec_fused<true><<<grid1(M / 2 + 1, nb), 256, 0, st>>>(q.Zn.as<float2>(), M, B, bs, q.Zn.as<float2>(), M, M, plan.WN);
+                else irb::k_spec_fused<false><<<grid1(M / 2 + 1, nb), 256, 0, st>>>(q.Zn.as<float2>(), M, B, bs, q.Zn.as<float2>(), M, M, plan.WN);
                 LAUNCHED();
-                if ((rc = plan.run(q.Zn.p, M, -1, q.dy.as<float2>(), M, q.tmp.as<float2>(), nb, true, 1.0f / (float) N, st))) return rc;
+                if ((rc = plan.run(q.Zn.p, M, -1, q.dy.as<float2>(), M, q.tmp.as<float2>(), nb, true, inv_n, st, win))) return rc;
             }
             if ((rc = download(q, b0, nb, st))) return rc;
             q.dn_busy = true;
@@ -529,61 +522,60 @@ static int deconvolve_batch_staged(const float* nums, int batch, int len_num, co
     return 0;
 }
 
-int irb_deconvolve_batch(const float* nums, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
-                         int include_amplitude, float* out) {
-    return deconvolve_batch_staged(nums, batch, len_num, den, len_den, sample_rate, smoothing, include_phase, include_amplitude, out);
-}
-
-// The same with DEVICE-resident captures and results (den: host or device).  Large plain divisions (no smoothing, phase kept, an
-// even capture length) run with no staging at all: every sub-batch's column pass reads the captures where they lie, the
-// inverse column pass writes the impulse responses where they belong, and consecutive sub-batches alternate between compute
-// streams so that one sub-batch's row kernels fill the SMs another one's column pass leaves idle.  The column passes read the
-// captures and write the results as float2, so that path also needs both pointers 8-byte aligned (a float view at an odd
-// offset is only 4-byte aligned).  Everything else goes through the staged pipeline above with device-to-device copies, which
-// take any alignment.  irb_last_compute_ms() is the device time of the whole call.
-int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
-                                int include_amplitude, float* out_dev) {
-    if (!nums_dev || !den || !out_dev) return fail(IRB_ERR_ARG, "null argument");
-    if (batch < 1 || len_num < 1 || len_den < 1) return fail(IRB_ERR_ARG, "empty input");
-    int N = 0, rc;
-    if ((rc = fft_size_for(len_num > len_den ? len_num : len_den, &N))) return rc;
-    const int M = N / 2, dev = irbh::current_device();
-    CK(cudaSetDevice(dev));
-    Plan plan;
-    if ((rc = plan.init(dev, M))) return rc;
-    const bool aligned = (((uintptr_t) nums_dev | (uintptr_t) out_dev) % alignof(float2)) == 0;
-    if (!(plan.big() && !smoothing && include_phase && len_num % 2 == 0 && aligned))
-        return deconvolve_batch_staged(nums_dev, batch, len_num, den, len_den, sample_rate, smoothing, include_phase, include_amplitude, out_dev, true);
+// The same on DEVICE-resident inputs and results with no staging at all: every sub-batch's column pass reads the signals (and
+// per-item operands) where they lie, the inverse column pass writes the results (or their windows) where they belong, and
+// consecutive sub-batches alternate between compute streams so that one sub-batch's row kernels fill the SMs another one's column
+// pass leaves idle.  Needs the fused four-step plan, float2-aligned rows of x (and of a per-item h, which must be in device memory)
+// and, without a window, of out.  irb_last_compute_ms() is the device time of the whole call.
+static int batch_direct(const BatchJob& J, const Plan& plan) {
+    const int batch = J.batch, len_num = J.len_x, len_den = J.len_h, N = J.N, M = N / 2;
+    const bool per_item = J.h_batch > 1;
+    const long long out_row = J.out_row();
     constexpr int kStreams = 3;
+    const int spectra = per_item ? 3 : 1;
     const int sub_pref = irbh::g_tuning.deconv_sub;
-    int sub = sub_pref > 0 ? sub_pref : (int) std::max<long long>(1, (32LL << 20) / ((long long) sizeof(float2) * M));      // about 32 MB of spectra per sub-batch
+    int sub = sub_pref > 0 ? sub_pref : (int) std::max<long long>(1, (32LL << 20) / ((long long) sizeof(float2) * M * spectra));      // about 32 MB of spectra per sub-batch
     sub = std::min(sub, batch);
     const int ncs = std::max(1, std::min(std::min(kStreams, irbh::g_tuning.deconv_streams > 0 ? irbh::g_tuning.deconv_streams : 2), (batch + sub - 1) / sub));
     const long long lde = (len_den + 1) & ~1LL;
-    DevBuf Zn[kStreams], dd, Zd, Bd;
+    int rc;
+    DevBuf Zn[kStreams], Zh[kStreams], Bh[kStreams], dd, Zd, Bd;
     cudaEvent_t e0 = nullptr, e1 = nullptr, ev_den = nullptr, ev_end[kStreams] = {nullptr, nullptr, nullptr};
     struct EvGuard { cudaEvent_t *a, *b, *c, *d; ~EvGuard() { for (cudaEvent_t* e : {a, b, c}) if (*e) cudaEventDestroy(*e); for (int i = 0; i < kStreams; ++i) if (d[i]) cudaEventDestroy(d[i]); } } evg{&e0, &e1, &ev_den, ev_end};
     irbh::StreamGuard cs[kStreams];                      // after the buffers and events: drained first on an early return
     for (int i = 0; i < ncs; ++i) {
         if ((rc = cs[i].create()) || (rc = Zn[i].alloc(sizeof(float2) * (size_t) M * sub, false))) return rc;
+        if (per_item && ((rc = Zh[i].alloc(sizeof(float2) * (size_t) M * sub, false)) || (rc = Bh[i].alloc(sizeof(float2) * (size_t) M * sub, false)))) return rc;
         CK(cudaEventCreateWithFlags(&ev_end[i], cudaEventDisableTiming));
     }
-    if ((rc = dd.alloc(sizeof(float) * lde, true)) || (rc = Zd.alloc(sizeof(float2) * (size_t) M, false)) || (rc = Bd.alloc(sizeof(float2) * (size_t) M, false))) return rc;
+    if (!per_item && ((rc = dd.alloc(sizeof(float) * lde, true)) || (rc = Zd.alloc(sizeof(float2) * (size_t) M, false)) || (rc = Bd.alloc(sizeof(float2) * (size_t) M, false)))) return rc;
     CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1)); CK(cudaEventCreateWithFlags(&ev_den, cudaEventDisableTiming));
     cudaStream_t st = cs[0].s;
-    CK(cudaMemcpyAsync(dd.p, den, sizeof(float) * len_den, cudaMemcpyDefault, st));
-    CK(cudaEventRecord(e0, st));
-    // the denominator's reciprocal spectrum in row layout, once
-    if ((rc = plan.cols_fwd(dd.p, lde / 2, len_den, Zd.as<float2>(), 1, st)) || (rc = plan.rows_to_split_spectrum(Zd.as<float2>(), Bd.as<float2>(), 1, true, st))) return rc;
+    if (!per_item) {
+        CK(cudaMemcpyAsync(dd.p, J.h, sizeof(float) * len_den, cudaMemcpyDefault, st));
+        CK(cudaEventRecord(e0, st));
+        // the shared operand's spectrum (the reciprocal for a division) in row layout, once
+        if ((rc = plan.cols_fwd(dd.p, lde / 2, len_den, Zd.as<float2>(), 1, st)) || (rc = plan.rows_to_split_spectrum(Zd.as<float2>(), Bd.as<float2>(), 1, J.divide, st))) return rc;
+    } else {
+        CK(cudaEventRecord(e0, st));
+    }
     CK(cudaEventRecord(ev_den, st));
     for (int i = 1; i < ncs; ++i) CK(cudaStreamWaitEvent(cs[i].s, ev_den, 0));
+    const OutWindow win{J.win.off, out_row, J.win.len};
     int it = 0;
     for (int b0 = 0; b0 < batch; b0 += sub, ++it) {
         const int k = it % ncs, nb = std::min(sub, batch - b0);
         cudaStream_t s = cs[k].s;
-        if ((rc = plan.cols_fwd(nums_dev + (size_t) b0 * len_num, len_num / 2, len_num, Zn[k].as<float2>(), nb, s)) ||
-            (rc = plan.rows_binop(Zn[k].as<float2>(), Bd.as<float2>(), 0, nb, s)) ||
-            (rc = plan.cols_inv(Zn[k].as<float2>(), reinterpret_cast<float2*>(out_dev + (size_t) b0 * N), M, nb, 1.0f / (float) N, s)))
+        const float2* B = Bd.as<float2>();
+        if (per_item) {
+            if ((rc = plan.cols_fwd(J.h + (size_t) b0 * len_den, len_den / 2, len_den, Zh[k].as<float2>(), nb, s)) ||
+                (rc = plan.rows_to_split_spectrum(Zh[k].as<float2>(), Bh[k].as<float2>(), nb, J.divide, s)))
+                return rc;
+            B = Bh[k].as<float2>();
+        }
+        if ((rc = plan.cols_fwd(J.x + (size_t) b0 * len_num, len_num / 2, len_num, Zn[k].as<float2>(), nb, s)) ||
+            (rc = plan.rows_binop(Zn[k].as<float2>(), B, per_item ? M : 0, nb, s)) ||
+            (rc = plan.cols_inv(Zn[k].as<float2>(), reinterpret_cast<float2*>(J.out + (size_t) b0 * out_row), M, nb, 1.0f / (float) N, s, win)))
             return rc;
     }
     for (int i = 1; i < ncs; ++i) { CK(cudaEventRecord(ev_end[i], cs[i].s)); CK(cudaStreamWaitEvent(st, ev_end[i], 0)); }
@@ -593,6 +585,125 @@ int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, c
     CK(cudaEventElapsedTime(&ms, e0, e1));
     irbh::set_last_compute_ms((double) ms);
     return 0;
+}
+
+// the division's job: nums[batch][len_num] / den[len_den] -> out[batch][N], N = nextPowerOfTwo(max(len_num, len_den))
+static int deconvolve_job(const float* nums, int batch, int len_num, const float* den, int len_den, float* out, BatchJob* J) {
+    if (!nums || !den || !out) return fail(IRB_ERR_ARG, "null argument");
+    if (batch < 1 || len_num < 1 || len_den < 1) return fail(IRB_ERR_ARG, "empty input");
+    int N = 0, rc;
+    if ((rc = fft_size_for(len_num > len_den ? len_num : len_den, &N))) return rc;
+    *J = BatchJob{nums, batch, len_num, den, 1, len_den, N, true, OutWindow{}, out};
+    return 0;
+}
+
+// the convolution's job (include/irb_b200.h, irb_convolve_batch); every argument error is found here, before any CUDA call
+static int convolve_job(const float* x, int batch, int len_x, const float* h, int h_batch, int len_h, int out_offset, int out_len, float* out, BatchJob* J) {
+    if (!x || !h || !out) return fail(IRB_ERR_ARG, "null argument");
+    if (batch < 1 || len_x < 1 || len_h < 1) return fail(IRB_ERR_ARG, "empty input");
+    if (h_batch != 1 && h_batch != batch) return fail(IRB_ERR_ARG, "h_batch %d: one IR for every signal (1) or one per signal (%d)", h_batch, batch);
+    const long long Lout = (long long) len_x + len_h - 1;
+    if (out_offset < 0 || out_len < 1 || (long long) out_offset + out_len > Lout)
+        return fail(IRB_ERR_ARG, "window [%d, %lld) is empty or outside the %lld samples of the result", out_offset, (long long) out_offset + out_len, Lout);
+    if (Lout > 2LL * kMaxBigM) return fail(IRB_ERR_ARG, "result of %lld samples needs an FFT above 2^22 points", Lout);
+    int N = 2 * kMinM;                                   // a longer zero-padded transform yields the same linear convolution
+    while (N < Lout) N *= 2;
+    *J = BatchJob{x, batch, len_x, h, h_batch, len_h, N, false, OutWindow{out_offset, out_len, out_len}, out};
+    return 0;
+}
+
+// memory a pointer lies in: device (or managed) memory can be read in place by the kernels
+static bool on_device(const void* p) {
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    return at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
+}
+
+extern "C" {
+
+// fp::convolution::convolveNonPeriodic (fp/convolution.cpp:246-347): each channel of the audio is one item of the batched
+// convolution, with the IR channel of its own (stereo / stereo, :320-323) or the one IR (stereo audio, mono IR); a stereo IR
+// for mono audio is folded to mono first (IRStereoAudioMono -> sumToMono, :302)
+int irb_convolve_nonperiodic(const float* x, int ch_x, int len_x, const float* h, int ch_h, int len_h, float* out) {
+    if (!x || !h || !out) return fail(IRB_ERR_ARG, "null argument");
+    if (len_x < 1 || len_h < 1 || ch_x < 1 || ch_h < 1) return fail(IRB_ERR_ARG, "empty input");
+    if (!((ch_x == 1 || ch_x == 2) && (ch_h == 1 || ch_h == 2)))
+        return fail(IRB_ERR_LAYOUT, "audio has %d channels and the IR %d: only mono/stereo layouts exist (fp/convolution.cpp:259-275)", ch_x, ch_h);
+    const long long Lout = (long long) len_x + len_h - 1;
+    if (Lout > 2LL * kMaxBigM) return fail(IRB_ERR_ARG, "result of %lld samples needs an FFT above 2^22 points", Lout);
+    if (!(ch_h == 2 && ch_x == 1)) return irb_convolve_batch(x, ch_x, len_x, h, ch_h, len_h, 0, (int) Lout, out);
+    DevBuf dh, dhf;
+    irbh::StreamGuard sg;
+    int rc;
+    CK(cudaSetDevice(irbh::current_device()));
+    if ((rc = sg.create())) return rc;
+    const long long lhe = (len_h + 1) & ~1LL;
+    if ((rc = dh.alloc(sizeof(float) * lhe * 2, false)) || (rc = dhf.alloc(sizeof(float) * lhe, false))) return rc;
+    for (int c = 0; c < 2; ++c) CK(cudaMemcpyAsync(dh.as<float>() + c * lhe, h + (size_t) c * len_h, sizeof(float) * len_h, cudaMemcpyHostToDevice, sg.s));
+    cudaEvent_t f0 = nullptr, f1 = nullptr;
+    struct EvGuard { cudaEvent_t &a, &b; ~EvGuard() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); } } evg{f0, f1};
+    CK(cudaEventCreate(&f0)); CK(cudaEventCreate(&f1));
+    CK(cudaEventRecord(f0, sg.s));
+    irb::k_fold_mono<<<grid1(len_h, 1), 256, 0, sg.s>>>(dh.as<float>(), dh.as<float>() + lhe, dhf.as<float>(), len_h);
+    LAUNCHED();
+    CK(cudaEventRecord(f1, sg.s));
+    // the batch core runs on streams of its own and reads the folded IR as device memory: it has to be complete first
+    CK(cudaEventSynchronize(f1));
+    if ((rc = irb_convolve_batch(x, 1, len_x, dhf.as<float>(), 1, len_h, 0, (int) Lout, out))) return rc;
+    float fold_ms = 0.f;                                 // irb_last_compute_ms() covers the fold too
+    CK(cudaEventElapsedTime(&fold_ms, f0, f1));
+    irbh::set_last_compute_ms(irb_last_compute_ms() + fold_ms);
+    return 0;
+}
+
+int irb_convolve_batch(const float* x, int batch, int len_x, const float* h, int h_batch, int len_h, int out_offset, int out_len, float* out) {
+    BatchJob J;
+    const int rc = convolve_job(x, batch, len_x, h, h_batch, len_h, out_offset, out_len, out, &J);
+    return rc ? rc : batch_staged(J, 0.0, 0, 1, 1, false);
+}
+
+// Staging-free when the transform is a four-step one, x_dev is float2-aligned with an even len_x, and a per-item h lies in device
+// memory, float2-aligned with an even len_h (a shared h is copied once from wherever it is); any other case goes through the staged
+// pipeline with device-to-device copies.  The windowed store is scalar, so out_dev needs no more than float alignment either way.
+int irb_convolve_batch_device(const float* x_dev, int batch, int len_x, const float* h, int h_batch, int len_h, int out_offset, int out_len, float* out_dev) {
+    BatchJob J;
+    int rc;
+    if ((rc = convolve_job(x_dev, batch, len_x, h, h_batch, len_h, out_offset, out_len, out_dev, &J))) return rc;
+    const int dev = irbh::current_device();
+    CK(cudaSetDevice(dev));
+    Plan plan;
+    if ((rc = plan.init(dev, J.N / 2))) return rc;
+    const bool x_direct = (uintptr_t) x_dev % alignof(float2) == 0 && len_x % 2 == 0;
+    const bool h_direct = h_batch == 1 || ((uintptr_t) h % alignof(float2) == 0 && len_h % 2 == 0 && on_device(h));
+    if (!(plan.big() && x_direct && h_direct)) return batch_staged(J, 0.0, 0, 1, 1, true);
+    return batch_direct(J, plan);
+}
+
+int irb_deconvolve_batch(const float* nums, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
+                         int include_amplitude, float* out) {
+    BatchJob J;
+    const int rc = deconvolve_job(nums, batch, len_num, den, len_den, out, &J);
+    return rc ? rc : batch_staged(J, sample_rate, smoothing, include_phase, include_amplitude, false);
+}
+
+// The same with DEVICE-resident captures and results (den: host or device).  Large plain divisions (no smoothing, phase kept, an
+// even capture length) run with no staging at all (batch_direct).  The column passes read the captures and write the results as
+// float2, so that path also needs both pointers 8-byte aligned (a float view at an odd offset is only 4-byte aligned).  Everything
+// else goes through the staged pipeline with device-to-device copies, which take any alignment.  irb_last_compute_ms() is the
+// device time of the whole call.
+int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
+                                int include_amplitude, float* out_dev) {
+    BatchJob J;
+    int rc;
+    if ((rc = deconvolve_job(nums_dev, batch, len_num, den, len_den, out_dev, &J))) return rc;
+    const int dev = irbh::current_device();
+    CK(cudaSetDevice(dev));
+    Plan plan;
+    if ((rc = plan.init(dev, J.N / 2))) return rc;
+    const bool aligned = (((uintptr_t) nums_dev | (uintptr_t) out_dev) % alignof(float2)) == 0;
+    if (!(plan.big() && !smoothing && include_phase && len_num % 2 == 0 && aligned))
+        return batch_staged(J, sample_rate, smoothing, include_phase, include_amplitude, true);
+    return batch_direct(J, plan);
 }
 
 int irb_deconvolve(const float* num, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase, int include_amplitude,

@@ -33,6 +33,14 @@ struct LineArgs {
     float scale;                  // applied on store
     const float2* W;              // the 2L roots of unity of the line length
 };
+// Real-output window of an inverse transform's last pass (k_line_fft_win): the output element n = line * out_line_stride +
+// j * out_elem_stride of batch item b is the pair of floats 2n, 2n+1 of that item's real result; only floats f in [off, off + len)
+// are written, one scalar store each, to ((float*) out)[b * stride + f - off], so `out` needs 4-byte alignment only
+// (out_batch_stride is unused)
+struct LineWindow {
+    long long off, stride;
+    int len;
+};
 
 constexpr int kTwLoBits = 10;
 // exp(-2 pi i idx / M) from the two-level table: one complex product of two correctly rounded factors
@@ -125,6 +133,99 @@ static __global__ void __launch_bounds__(kThreads, L >= 1024 ? 2 : IRB_LINE_CTAS
             float2 v = s_lines[c * T::PITCH + j];
             v.x *= a.scale; v.y *= a.scale;
             a.out[ob + (long long) line * a.out_line_stride + (long long) j * a.out_elem_stride] = v;
+        }
+    }
+}
+
+// k_line_fft<L, true> whose last pass stores only the window w of each batch item's real result (LineWindow).  A copy rather than
+// a branch or a template argument of k_line_fft: any change to that kernel's source or arguments changes the code ptxas makes of
+// it (a run-time branch cost the division's device path 2 %), and the plain transforms are the hot path of the batched division.
+template <int L>
+static __global__ void __launch_bounds__(kThreads, L >= 1024 ? 2 : IRB_LINE_CTAS) k_line_fft_win(const LineArgs a, const LineWindow w) {
+    constexpr bool INV = true;
+    using T = LineTile<L>;
+    extern __shared__ __align__(16) float2 s_lines[];
+    __shared__ float2 s_step[T::C][kPts];                 // inter-pass twiddle: root(line * TPF * j), the same for every thread of a line
+    const int tid = threadIdx.x;
+    const int line0 = blockIdx.x * T::C;
+    const long long ib = (long long) blockIdx.y * a.in_batch_stride;
+    const bool in_contig = a.in_elem_stride == 1, out_contig = a.out_elem_stride == 1;
+    if (a.tw_M > 0) {
+        for (int i = tid; i < T::C * kPts; i += kThreads) {
+            const int c = i / kPts, j = i % kPts;
+            s_step[c][j] = root_big(a.tw_hi, a.tw_lo, ((long long) (line0 + c) * T::TPF * j) & (a.tw_M - 1));
+        }
+    }
+
+    // all of a thread's loads are issued before the first shared-memory store: PER x 8 bytes in flight per thread
+    constexpr int PER = T::C * L / kThreads;
+    {
+        float2 r[PER];
+#pragma unroll
+        for (int i = 0; i < PER; ++i) {
+            const int idx = tid + i * kThreads;
+            const int c = in_contig ? idx / L : idx % T::C;
+            const int j = in_contig ? idx % L : idx / T::C;
+            const int line = line0 + c;
+            float2 v = make_float2(0.f, 0.f);
+            if (line < a.n_lines) {
+                const long long off = (long long) line * a.in_line_stride + (long long) j * a.in_elem_stride;
+                if (a.in_real_len < 0) v = reinterpret_cast<const float2*>(a.in)[ib + off];
+                else {
+                    const float* rp = reinterpret_cast<const float*>(a.in) + 2 * ib;
+                    const long long e = 2 * off;
+                    if (e + 1 < a.in_real_len) v = *reinterpret_cast<const float2*>(rp + e);
+                    else if (e < a.in_real_len) v.x = rp[e];
+                }
+            }
+            r[i] = v;
+        }
+#pragma unroll
+        for (int i = 0; i < PER; ++i) {
+            const int idx = tid + i * kThreads;
+            const int c = in_contig ? idx / L : idx % T::C;
+            const int j = in_contig ? idx % L : idx / T::C;
+            s_lines[c * T::PITCH + j] = r[i];
+        }
+    }
+    bar_compute();
+    {
+        const int t = tid % T::TPF;
+        for (int c = tid / T::TPF; c < T::C; c += T::G) {
+            float2* srow = s_lines + c * T::PITCH;
+            float2 v[kPts];
+            fft_gather<L>(v, t, srow);
+            fft_run<L, INV>(v, t, srow, a.W);
+            const int line = line0 + c;
+            float2 tw_base = make_float2(1.f, 0.f);
+            if (a.tw_M > 0) tw_base = root_big(a.tw_hi, a.tw_lo, ((long long) line * t) & (a.tw_M - 1));
+#pragma unroll
+            for (int j = 0; j < kPts; ++j) {
+                const int k = t + j * T::TPF;
+                if (a.tw_M > 0) {
+                    // root(line*k), k = t + j*TPF, as root(line*t) * root(line*TPF*j): the second factor is the same for
+                    // the whole line and was looked up once per CTA (a broadcast read of shared memory here)
+                    const float2 w = cmul(tw_base, s_step[c][j]);
+                    v[j] = cmul(v[j], INV ? cconj(w) : w);
+                }
+                srow[k] = v[j];              // each thread rewrites exactly the elements it gathered last
+            }
+        }
+    }
+    bar_compute();
+#pragma unroll
+    for (int i = 0; i < PER; ++i) {
+        const int idx = tid + i * kThreads;
+        const int c = out_contig ? idx / L : idx % T::C;
+        const int j = out_contig ? idx % L : idx / T::C;
+        const int line = line0 + c;
+        if (line < a.n_lines) {
+            float2 v = s_lines[c * T::PITCH + j];
+            v.x *= a.scale; v.y *= a.scale;
+            const long long f = 2 * ((long long) line * a.out_line_stride + (long long) j * a.out_elem_stride) - w.off;
+            float* o = reinterpret_cast<float*>(a.out) + blockIdx.y * w.stride + f;
+            if (f >= 0 && f < w.len) o[0] = v.x;
+            if (f + 1 >= 0 && f + 1 < w.len) o[1] = v.y;
         }
     }
 }

@@ -85,6 +85,8 @@ _SIGS = {
     "irb_group_state_bytes": (ctypes.c_size_t, [_vp]),
     "irb_convolve_periodic": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_convolve_nonperiodic": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int, _vp]),
+    "irb_convolve_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
+    "irb_convolve_batch_device": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_deconvolve": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_deconvolve_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_deconvolve_batch_device": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
@@ -322,6 +324,52 @@ def convolve_nonperiodic(x, h):
         return np.zeros_like(x)         # the reference returns a cleared copy of the input (fp/convolution.cpp:271-275)
     _ck(rc)
     return out
+
+
+def _window(len_x, len_h, out_offset, out_len):
+    """(out_offset, out_len) of a batched convolution's window; out_len None: the rest of the len_x + len_h - 1 samples"""
+    full = int(len_x) + int(len_h) - 1
+    return int(out_offset), full - int(out_offset) if out_len is None else int(out_len)
+
+
+def convolve_batch(x, h, out_offset=0, out_len=None, out=None):
+    """irb_convolve_batch: signals x[batch][len_x], each convolved with h[len_h] (shared) or h[1 | batch][len_h] (h[b] for signal
+    b) -> out[batch][out_len], the window [out_offset, out_offset + out_len) of every len_x + len_h - 1 sample result (default: all
+    of it).  `out` may be a C-contiguous float32 array of that shape (pinned memory: eng.pinned_empty)."""
+    x = np.ascontiguousarray(x, np.float32)
+    x = x[None, :] if x.ndim == 1 else x
+    h = np.ascontiguousarray(h, np.float32)
+    h = h[None, :] if h.ndim == 1 else h
+    if x.ndim != 2 or h.ndim != 2:
+        raise ValueError("x must be [batch][len_x] and h [len_h] or [1 | batch][len_h], got %r and %r" % (x.shape, h.shape))
+    off, n = _window(x.shape[1], h.shape[1], out_offset, out_len)
+    if out is None:
+        out = np.empty((x.shape[0], max(n, 0)), np.float32)
+    elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.shape == (x.shape[0], n) and out.flags.c_contiguous and out.flags.writeable):
+        raise ValueError("out must be a writable C-contiguous float32 array of shape %r" % ((x.shape[0], n),))
+    _ck(lib().irb_convolve_batch(_ptr(x), x.shape[0], x.shape[1], _ptr(h), h.shape[0], h.shape[1], off, n, _ptr(out)))
+    return out
+
+
+def convolve_batch_device(x_ptr, batch, len_x, h, out_ptr, len_h=None, h_batch=None, out_offset=0, out_len=None):
+    """irb_convolve_batch_device: x and the result are raw DEVICE pointers ([batch][len_x] / [batch][out_len] float32).  h is either
+    a raw pointer (an int, e.g. tensor.data_ptr(), to device or host memory) with len_h given and h_batch 1 (the default) or batch,
+    or a host array-like ([len_h] or [h_batch][len_h]) whose shape gives both; len_h / h_batch that contradict it are an error."""
+    if isinstance(h, (int, np.integer)):
+        if len_h is None:
+            raise ValueError("len_h is needed with a pointer h")
+        hp = _vp(int(h))
+        h_batch = 1 if h_batch is None else h_batch
+    else:
+        ha = np.asarray(h)
+        if ha.ndim not in (1, 2):
+            raise ValueError("h must be [len_h] or [h_batch][len_h], got shape %r" % (ha.shape,))
+        ha = np.ascontiguousarray(ha[None, :] if ha.ndim == 1 else ha, np.float32)
+        if (len_h is not None and int(len_h) != ha.shape[1]) or (h_batch is not None and int(h_batch) != ha.shape[0]):
+            raise ValueError("len_h=%r, h_batch=%r contradict h of shape %r" % (len_h, h_batch, ha.shape))
+        h_batch, len_h, hp = ha.shape[0], ha.shape[1], _ptr(ha)
+    off, n = _window(len_x, len_h, out_offset, out_len)
+    _ck(lib().irb_convolve_batch_device(_vp(int(x_ptr)), int(batch), int(len_x), hp, int(h_batch), int(len_h), off, n, _vp(int(out_ptr))))
 
 
 def deconvolve(num, den, sample_rate=48000.0, smoothing=True, include_phase=True, include_amplitude=True):
