@@ -7,8 +7,10 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <map>
 #include <memory>
 #include <mutex>
+#include <tuple>
 #include <type_traits>
 #include <new>
 #include <vector>
@@ -183,62 +185,63 @@ void plan_units(int n_rows, int rows_per_tile, int ctas, bool narrowing, int out
         rem -= std::min(rem, cnt * s);
     }
 }
-template <int M, bool PERROW>
-int launch_mac_p(irb::MacArgs a, int num_sms, cudaStream_t st) {
+// ---- per-device kernel set-up ------------------------------------------------------------------------------------------
+// Cached per (kernel, device, key), not per thread: one thread drives every GPU of an irb_group, and a cache of its last device
+// would redo the set-up on every switch.  Key 0: the attributes (kernel_setup); key n >= 1: the usable size of a requested
+// cluster size n (launch_slots_t).
+std::mutex g_setup_mu;
+std::map<std::tuple<const void*, int, int>, int> g_setup;
+
+// Once per (kernel, device): the dynamic shared memory `smem`, the largest shared-memory carveout if `max_carveout`, clusters
+// above the portable size if `clusters`, and a check that `min_resident` CTAs fit on an SM (registers / shared memory): a
+// kernel built for two CTAs per SM (ring depth, register budget) refuses to run silently at half of it.
+int kernel_setup(const void* k, const char* name, int M, size_t smem, bool max_carveout, int min_resident, bool clusters = false) {
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lk(g_setup_mu);
+    if (g_setup.count({k, dev, 0})) return 0;
+    CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+    if (max_carveout) CK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    if (clusters) CK(cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    if (min_resident > 1) {
+        int resident = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, k, irb::kThreads + 32, smem));
+        if (resident < min_resident)
+            return fail(IRB_ERR_CUDA, "%s<%d>: only %d CTA per SM fits (registers / shared memory), %d expected", name, M, resident, min_resident);
+    }
+    g_setup[{k, dev, 0}] = 1;
+    return 0;
+}
+
+// The persistent block steps: k_mac_p (INS == 0; irb_mac_p.cuh) over a.n_rows rows, or the IR-matrix step k_mac_mx
+// (irb_mac_mx.cuh) over a.n_rows output rows in units of whole groups.  One launch, at most one CTA per unit.
+template <int M, bool PER, int INS = 0, int OUTS = 0>
+int launch_persistent(irb::MacArgs a, int num_sms, cudaStream_t st) {
     if (a.n_rows <= 0) return 0;
     if (!a.work) return fail(IRB_ERR_STATE, "persistent block step without a work counter");
     const int ctas = persistent_ctas_per_sm() * num_sms;
-    plan_units(a.n_rows, irb::Tile<M>::ROWS, ctas, irbh::g_tuning.unit_narrowing != 0, a.unit_n);
-    const int n_units = a.unit_n[0] + a.unit_n[1] + a.unit_n[2] + a.unit_n[3];
-    const int grid = std::min(n_units, ctas);
-    const size_t smem = sizeof(irb::PSmem<M, PERROW>);
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        CK(cudaFuncSetAttribute(irb::k_mac_p<M, PERROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        CK(cudaFuncSetAttribute(irb::k_mac_p<M, PERROW>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        // two CTAs per SM is what the kernel is built for (ring depth, register budget): refuse to run silently at half of it
-        int resident = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, irb::k_mac_p<M, PERROW>, irb::kThreads + 32, smem));
-        if (resident < 2) return fail(IRB_ERR_CUDA, "k_mac_p<%d>: only %d CTA per SM fits (registers / shared memory), 2 expected", M, resident);
-        configured_dev = dev;
+    void (*k)(irb::MacArgs);
+    size_t smem;
+    if constexpr (INS == 0) {
+        plan_units(a.n_rows, irb::Tile<M>::ROWS, ctas, irbh::g_tuning.unit_narrowing != 0, a.unit_n);
+        k = irb::k_mac_p<M, PER>;
+        smem = sizeof(irb::PSmem<M, PER>);
+    } else {
+        using C = irb::MxCfg<M, INS, OUTS, PER>;
+        a.unit_n[0] = (a.n_rows / OUTS + C::GROUPS - 1) / C::GROUPS; a.unit_n[1] = a.unit_n[2] = a.unit_n[3] = 0;
+        k = irb::k_mac_mx<M, INS, OUTS, PER>;
+        smem = sizeof(irb::MxSmem<M, INS, OUTS, PER>);
     }
-    irb::k_mac_p<M, PERROW><<<grid, irb::kThreads + 32, smem, st>>>(a);
-    g_launches++;
-    CK(cudaGetLastError());
-    return 0;
-}
-// the IR-matrix block step (irb_mac_mx.cuh): a.n_rows output rows, units of whole groups, one launch
-template <int M, int INS, int OUTS, bool PG>
-int launch_mac_mx_t(irb::MacArgs a, int num_sms, cudaStream_t st) {
-    using C = irb::MxCfg<M, INS, OUTS, PG>;
-    if (a.n_rows <= 0) return 0;
-    if (!a.work) return fail(IRB_ERR_STATE, "matrix block step without a work counter");
-    const int ctas = persistent_ctas_per_sm() * num_sms;
-    const int n_groups = a.n_rows / OUTS;
-    a.unit_n[0] = (n_groups + C::GROUPS - 1) / C::GROUPS; a.unit_n[1] = a.unit_n[2] = a.unit_n[3] = 0;
-    const int grid = std::min(a.unit_n[0], ctas);
-    const size_t smem = sizeof(irb::MxSmem<M, INS, OUTS, PG>);
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        CK(cudaFuncSetAttribute(irb::k_mac_mx<M, INS, OUTS, PG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        CK(cudaFuncSetAttribute(irb::k_mac_mx<M, INS, OUTS, PG>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        int resident = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, irb::k_mac_mx<M, INS, OUTS, PG>, irb::kThreads + 32, smem));
-        if (resident < 2) return fail(IRB_ERR_CUDA, "k_mac_mx<%d, %d, %d>: only %d CTA per SM fits (registers / shared memory), 2 expected", M, INS, OUTS, resident);
-        configured_dev = dev;
-    }
-    irb::k_mac_mx<M, INS, OUTS, PG><<<grid, irb::kThreads + 32, smem, st>>>(a);
+    const int grid = std::min(a.unit_n[0] + a.unit_n[1] + a.unit_n[2] + a.unit_n[3], ctas);
+    if (int rc = kernel_setup((const void*) k, INS == 0 ? "k_mac_p" : "k_mac_mx", M, smem, true, 2)) return rc;
+    k<<<grid, irb::kThreads + 32, smem, st>>>(a);
     g_launches++;
     CK(cudaGetLastError());
     return 0;
 }
 template <int M, int INS, int OUTS>
 int launch_mac_mx_pg(const irb::MacArgs& a, bool pergroup, int num_sms, cudaStream_t st) {
-    return pergroup ? launch_mac_mx_t<M, INS, OUTS, true>(a, num_sms, st) : launch_mac_mx_t<M, INS, OUTS, false>(a, num_sms, st);
+    return pergroup ? launch_persistent<M, true, INS, OUTS>(a, num_sms, st) : launch_persistent<M, false, INS, OUTS>(a, num_sms, st);
 }
 template <int M>
 int launch_mac_mx_m(const irb::MacArgs& a, int ins, int outs, bool pergroup, int num_sms, cudaStream_t st) {
@@ -259,13 +262,7 @@ int launch_mac_tma(const irb::MacArgs& a, cudaStream_t st) {
     const int grid = (a.n_rows + irb::Tile<M>::ROWS - 1) / irb::Tile<M>::ROWS;
     if (grid <= 0) return 0;
     const size_t smem = sizeof(irb::TmaSmem<M>);
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        CK(cudaFuncSetAttribute(irb::k_mac_tma<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        configured_dev = dev;
-    }
+    if (int rc = kernel_setup((const void*) irb::k_mac_tma<M>, "k_mac_tma", M, smem, false, 0)) return rc;
     irb::k_mac_tma<M><<<grid, irb::kThreads + 32, smem, st>>>(a);
     g_launches++;
     CK(cudaGetLastError());
@@ -276,13 +273,7 @@ int launch_mac_u(const irb::MacArgs& a, cudaStream_t st) {
     const int grid = (a.n_rows + irb::Tile<M>::ROWS - 1) / irb::Tile<M>::ROWS;
     if (grid <= 0) return 0;
     const size_t smem = sizeof(irb::MacSmem<M, U>);
-    static thread_local int configured_dev = -1;
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        CK(cudaFuncSetAttribute(irb::k_mac<M, U, INV, FUSE, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        configured_dev = dev;
-    }
+    if (int rc = kernel_setup((const void*) irb::k_mac<M, U, INV, FUSE, WIDE>, "k_mac", M, smem, false, 0)) return rc;
     irb::k_mac<M, U, INV, FUSE, WIDE><<<grid, irb::kThreads + 32, smem, st>>>(a);
     g_launches++;
     CK(cudaGetLastError());
@@ -295,16 +286,8 @@ int launch_slots_t(const irb::MacArgs& a, int cl, cudaStream_t st) {
     const int tiles = (a.n_rows + rpt - 1) / rpt;
     if (tiles <= 0) return 0;
     const size_t smem = sizeof(irb::SlotSmem<M>);
-    static thread_local int configured_dev = -1;
-    static thread_local int usable[17] = {0};
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    if (configured_dev != dev) {
-        CK(cudaFuncSetAttribute(irb::k_mac_slots<M, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-        CK(cudaFuncSetAttribute(irb::k_mac_slots<M, INV>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        configured_dev = dev;
-        for (int& u : usable) u = 0;
-    }
+    const void* k = (const void*) irb::k_mac_slots<M, INV>;
+    if (int rc = kernel_setup(k, "k_mac_slots", M, smem, false, 0, true)) return rc;
     cudaLaunchConfig_t cfg{};
     cfg.blockDim = dim3(irb::kThreads + 32); cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute at[1];
@@ -313,17 +296,23 @@ int launch_slots_t(const irb::MacArgs& a, int cl, cudaStream_t st) {
     cfg.attrs = at; cfg.numAttrs = 1;
     // the largest cluster this device can co-schedule, found once per (device, size): a partitioned or busy GPU may not
     // have 16 SMs free in one GPC; the kernel reads its cluster size at run time, so a smaller one just splits less
-    if (usable[cl] == 0) {
-        int c = cl;
-        for (; c > 1; c /= 2) {
-            cfg.gridDim = dim3((unsigned) c); at[0].val.clusterDim.x = (unsigned) c;
-            int n = 0;
-            if (cudaOccupancyMaxActiveClusters(&n, irb::k_mac_slots<M, INV>, &cfg) == cudaSuccess && n > 0) break;
-            cudaGetLastError();
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    {
+        std::lock_guard<std::mutex> lk(g_setup_mu);
+        int& usable = g_setup[{k, dev, cl}];
+        if (usable == 0) {
+            int c = cl;
+            for (; c > 1; c /= 2) {
+                cfg.gridDim = dim3((unsigned) c); at[0].val.clusterDim.x = (unsigned) c;
+                int n = 0;
+                if (cudaOccupancyMaxActiveClusters(&n, irb::k_mac_slots<M, INV>, &cfg) == cudaSuccess && n > 0) break;
+                cudaGetLastError();
+            }
+            usable = c;
         }
-        usable[cl] = c;
+        cl = usable;
     }
-    cl = usable[cl];
     cfg.gridDim = dim3((unsigned) (tiles * cl)); at[0].val.clusterDim.x = (unsigned) cl;
     CK(cudaLaunchKernelEx(&cfg, irb::k_mac_slots<M, INV>, a));
     g_launches++;
@@ -334,7 +323,7 @@ int launch_mac_t(const irb::MacArgs& a, bool slots, int cl, int num_sms, cudaStr
     if constexpr (INV && M >= kPersistMinM) {
         // the fused streaming block step as ONE persistent launch (shared-IR tiles or per-stream IRs)
         if (a.head && a.in && a.work && a.blocks_per_chan == 1 && a.head_back == 0 && a.split_in == 1 && cl == 1)
-            return slots ? launch_mac_p<M, true>(a, num_sms, st) : launch_mac_p<M, false>(a, num_sms, st);
+            return slots ? launch_persistent<M, true>(a, num_sms, st) : launch_persistent<M, false>(a, num_sms, st);
     }
     if (slots) return launch_slots_t<M, INV>(a, cl, st);
     if constexpr (INV) {

@@ -455,10 +455,37 @@ __device__ __forceinline__ long long fdl_row_offset(const MacArgs& a, int chan, 
 }
 template <int M> __device__ __forceinline__ long long fdl_slot_stride(const MacArgs& a) { return a.fdl_slot_stride ? a.fdl_slot_stride : M; }
 
-// consumer release of a TMA-filled ring stage by the warp's elected lane (after the warp-wide fence.proxy.async + __syncwarp)
-__device__ __forceinline__ void mbar_release_stage(uint64_t* b, uint32_t dep, const MacArgs& a) {
-    if (a.release_dep) mbar_arrive_after(b, dep & a.zero);
-    else mbar_arrive(b);
+// ---- steps shared by the streaming block-step kernels (k_mac<FUSE>, k_mac_tma, k_mac_slots, k_mac_p, k_mac_mx) ----------
+
+// ac += xv * h for one float4 (two packed bins) of a partition product, bin0: the float4 holds bin 0, the packed {DC, Nyquist}
+// pair, which takes two real products instead of a complex one.  This fmaf sequence, in ascending partition order, is what
+// makes the block-step kernels bit-identical to one another; k_mac and k_mac_slots call it, k_mac_tma, k_mac_p and
+// k_mac_mx spell it out (as a call it changes their instruction schedule).
+__device__ __forceinline__ void cmac4(float4& ac, const float4& xv, const float4& h, bool bin0) {
+    const float h0i = bin0 ? 0.f : h.y, h0q = bin0 ? h.y : h.x;
+    ac.x = fmaf(xv.x, h.x, fmaf(-xv.y, h0i, ac.x));
+    ac.y = fmaf(xv.y, h0q, fmaf(xv.x, h0i, ac.y));
+    ac.z = fmaf(xv.z, h.z, fmaf(-xv.w, h.w, ac.z));
+    ac.w = fmaf(xv.w, h.z, fmaf(xv.z, h.w, ac.w));
+}
+
+// Barriers of an n-stage ring, set up by one thread: full[i] completes on the producer's expect_tx and the bytes of its bulk
+// copies, empty[i] on one arrive of each compute warp.  The fence makes the initialised barriers visible to the async proxy.
+__device__ __forceinline__ void ring_init(uint64_t* full, uint64_t* empty, int n) {
+    for (int i = 0; i < n; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], kThreads / 32); }
+    mbar_fence_init();
+}
+
+// A compute warp's release of a TMA-filled ring stage it has read: every lane orders its ld.shared of the stage ahead of the
+// bulk copy that refills it (fence.proxy.async, if release_fence), then the warp's first lane arrives, carrying a data
+// dependency on the values read from the stage if release_dep (mbar_arrive_after).
+__device__ __forceinline__ void release_stage(uint64_t* b, uint32_t dep, const MacArgs& a, int tid) {
+    if (a.release_fence) fence_proxy_async_smem();
+    __syncwarp();
+    if ((tid & 31) == 0) {
+        if (a.release_dep) mbar_arrive_after(b, dep & a.zero);
+        else mbar_arrive(b);
+    }
 }
 
 // Shared-IR kernel: the whole tile is bound to one IR and a ring stage holds U consecutive partitions of it.
@@ -492,10 +519,7 @@ __global__ void __launch_bounds__(kThreads + 32, U == 1 ? 3 : 2) k_mac(const Mac
     }
     const int ngroups = (pmax + U - 1) / U;
 
-    if (tid == 0) {
-        for (int i = 0; i < kStages; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.empty[i], kThreads / 32); }
-        mbar_fence_init();
-    }
+    if (tid == 0) ring_init(sm.full, sm.empty, kStages);
     __syncthreads();
 
     if (tid >= kThreads) {
@@ -647,23 +671,12 @@ __global__ void __launch_bounds__(kThreads + 32, U == 1 ? 3 : 2) k_mac(const Mac
                     const int c = L::f4(c0, vv);
                     const float4 h = *reinterpret_cast<const float4*>(&sm.h[st][u][2 * c]);
                     dep |= __float_as_uint(h.x);
-                    // bin 0 is the packed {DC, Nyquist} pair: two real products instead of a complex one
-                    const float h0i = c == 0 ? 0.f : h.y, h0q = c == 0 ? h.y : h.x;
 #pragma unroll
-                    for (int s = 0; s < L::K; ++s) {
-                        const float4 xv = x[u][s][vv];
-                        float4& ac = acc[s][vv];
-                        ac.x = fmaf(xv.x, h.x, fmaf(-xv.y, h0i, ac.x));
-                        ac.y = fmaf(xv.y, h0q, fmaf(xv.x, h0i, ac.y));
-                        ac.z = fmaf(xv.z, h.z, fmaf(-xv.w, h.w, ac.z));
-                        ac.w = fmaf(xv.w, h.z, fmaf(xv.z, h.w, ac.w));
-                    }
+                    for (int s = 0; s < L::K; ++s) cmac4(acc[s][vv], x[u][s][vv], h, c == 0);
                 }
             }
         }
-        if (a.release_fence) fence_proxy_async_smem();
-        __syncwarp();
-        if ((tid & 31) == 0) mbar_release_stage(&sm.empty[st], dep, a);
+        release_stage(&sm.empty[st], dep, a, tid);
     };
 
     if (ngroups > 0) load_group(xa, 0);
@@ -741,10 +754,7 @@ __global__ void __launch_bounds__(kThreads + 32, M <= 1024 ? 3 : 2) k_mac_tma(co
     const int ir = a.ir_of_chan ? a.ir_of_chan[row0] : 0;
     const int np = a.nparts[ir];
 
-    if (tid == 0) {
-        for (int i = 0; i < kTmaStages; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.empty[i], kThreads / 32); }
-        mbar_fence_init();
-    }
+    if (tid == 0) ring_init(sm.full, sm.empty, kTmaStages);
     if (tid < T::ROWS) {
         int hd = -1;
         if (row0 + tid < a.n_rows) { hd = a.head[row0 + tid] - a.head_back; if (hd < 0) hd += a.ring; }
@@ -862,9 +872,7 @@ __global__ void __launch_bounds__(kThreads + 32, M <= 1024 ? 3 : 2) k_mac_tma(co
                 ac.w = fmaf(xv.w, h.z, fmaf(xv.z, h.w, ac.w));
             }
         }
-        if (a.release_fence) fence_proxy_async_smem();
-        __syncwarp();
-        if ((tid & 31) == 0) mbar_release_stage(&sm.empty[st], dep, a);
+        release_stage(&sm.empty[st], dep, a, tid);
     }
 
     bar_compute();                                        // every warp is through its last group: stage 0 is the tile again
@@ -933,8 +941,7 @@ __global__ void __launch_bounds__(kThreads + 32, 1) k_mac_slots(const MacArgs a)
     stamp(a, 0);
 
     if (tid == 0) {
-        for (int i = 0; i < kSlotStages; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.empty[i], kThreads / 32); }
-        mbar_fence_init();
+        ring_init(sm.full, sm.empty, kSlotStages);
         sm.ngroups = 0;
     }
     __syncthreads();
@@ -1110,18 +1117,10 @@ __global__ void __launch_bounds__(kThreads + 32, 1) k_mac_slots(const MacArgs a)
                     if (g >= nvalid[s]) continue;          // this slot's range is shorter: its stage entry was not filled
                     const float4 h = *reinterpret_cast<const float4*>(&sm.h[st][s * L::G + g_][2 * c]);
                     dep |= __float_as_uint(h.x);
-                    const float h0i = c == 0 ? 0.f : h.y, h0q = c == 0 ? h.y : h.x;    // bin 0 = packed {DC, Nyquist}
-                    const float4 xv = x[s][vv];
-                    float4& ac = acc[s][vv];
-                    ac.x = fmaf(xv.x, h.x, fmaf(-xv.y, h0i, ac.x));
-                    ac.y = fmaf(xv.y, h0q, fmaf(xv.x, h0i, ac.y));
-                    ac.z = fmaf(xv.z, h.z, fmaf(-xv.w, h.w, ac.z));
-                    ac.w = fmaf(xv.w, h.z, fmaf(xv.z, h.w, ac.w));
+                    cmac4(acc[s][vv], x[s][vv], h, c == 0);
                 }
             }
-            if (a.release_fence) fence_proxy_async_smem();
-            __syncwarp();
-            if ((tid & 31) == 0) mbar_release_stage(&sm.empty[st], dep, a);
+            release_stage(&sm.empty[st], dep, a, tid);
         };
         // kSlotDepth groups of FDL loads stay in flight (round 1 kept one), the IR ring holds kSlotStages partitions: the 6 or 7
         // partitions a slot has on the latency path are requested at once.

@@ -69,9 +69,8 @@ __global__ void __launch_bounds__(kThreads + 32, 2) k_mac_p(const MacArgs a) {
     }
 
     if (tid == 0) {
-        for (int i = 0; i < C::NS; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.empty[i], kThreads / 32); }
         for (int i = 0; i < 2; ++i) { mbar_init(&sm.u_full[i], 1); mbar_init(&sm.u_empty[i], kThreads / 32); }
-        mbar_fence_init();
+        ring_init(sm.full, sm.empty, C::NS);
     }
     __syncthreads();
 
@@ -269,9 +268,7 @@ __global__ void __launch_bounds__(kThreads + 32, 2) k_mac_p(const MacArgs a) {
                     }
                 }
                 if (g + 1 < np) {
-                    if (a.release_fence) fence_proxy_async_smem();
-                    __syncwarp();
-                    if ((tid & 31) == 0) mbar_release_stage(&sm.empty[st], dep, a);
+                    release_stage(&sm.empty[st], dep, a, tid);
                 } else {
                     hold = st;                            // the last stage of the unit is kept: its FDL area becomes the tile
                 }
