@@ -237,6 +237,36 @@ int irb_deconvolve_batch(const float* nums, int batch, int len_num, const float*
  * accepted too, and goes through staged device-to-device copies. */
 int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing,
                                 int include_phase, int include_amplitude, float* out_dev);
+/* fp::ir::IRchop followed, when `normalize`, by fp::tools::normalize(goal_db) on each row x[0, len) of x_dev[batch][len]
+ * (device memory) -> out_dev[batch][ir_length] (device memory); positions (null, or device memory) [batch][2] = {q, start}:
+ * the peak's index (the system delay of a capture) and the first sample of the cut.  The rule, the facade's (fp_b200.cpp):
+ *   peak = max |x_i| accumulated as std::max(m, fabs(x_i)) from m = 0 (NaN samples are ignored, an Inf makes the peak Inf);
+ *   q = the first index with fabs(x_q) == peak, 0 when there is none (every sample NaN);
+ *   below(i) := linTodB(fabs(x_i)) - linTodB(peak) < threshold_db in float, linTodB(v) = v == 0 ? -333 : 20 * ln(v) / ln(10)
+ *   evaluated left to right in float, ln(v) = (float) log((double) v) (the correctly rounded float log; see below);
+ *   walked = 0 when consecutive <= 0, else the smallest k >= consecutive such that below(s_{k-consecutive}) .. below(s_{k-1})
+ *   all hold, s_j = (q - j) mod len, capped at ir_length; start = (q - walked) mod len;
+ *   out = the ir_length samples from start (wrapping past len - 1 to 0); samples [ir_length-1-ir_length/4, ir_length-1) times
+ *   (float) (1.0 - (double) (float(i') * step)) (the last sample is not faded, as in the reference), then samples [0, walked/4)
+ *   times float(i') * step; i' is the offset in the fade, step = (float) (1.0 / fade length) (tools::linearFade);
+ *   normalize: every sample times goal / max|out|, goal = dBToLin(goal_db) in float (a silent row gives NaN, as the facade).
+ * The log: glibc's logf is not correctly rounded (on about 417 000 of the 2^31 positive floats it differs from the correctly
+ * rounded result; linTodB then differs on about 326 000), and the device's own logf has a different error set, so the device
+ * uses the correctly rounded float log, computed as log((double) v) rounded to float (with glibc's double log that formula is the
+ * nearest float to ln(v) on every positive float except five hard cases, 0x3c413d3a, 0x41178feb, 0x4c5d65a5, 0x65d890d3 and
+ * 0x6f31a8ec).  A row's cut can therefore differ from the host facade's only when the level of one of its walked samples, or of
+ * its peak, is one of those inputs AND that 1-ulp difference flips a threshold decision.  Everything else (the peak, the cut,
+ * the fades, the gain) is the facade's arithmetic bit for bit (NaN samples stay NaN; the payload is the device's).
+ * IRB_ERR_ARG before any CUDA call: a null x_dev or out_dev, batch < 1, len < 1, ir_length < 1 or > len.  Any 4-byte aligned
+ * pointers; irb_last_compute_ms() is the device time of the call. */
+int irb_ir_chop_batch_device(const float* x_dev, int batch, int len, int ir_length, float threshold_db, int consecutive, int normalize, float goal_db,
+                             float* out_dev, int* positions);
+/* irb_deconvolve_batch followed by the chop above, inside the sub-batch pipeline: host (or pinned) nums in, out[batch][ir_length]
+ * and positions (null, or host memory [batch][2]) back; the [batch][N] results never leave the device.  Row b is bit-identical to
+ * irb_deconvolve_batch's row b chopped by irb_ir_chop_batch_device.  IRB_ERR_ARG before any CUDA call for the division's own
+ * rejections and ir_length < 1 or > N.  irb_last_compute_ms() covers the chop as part of the kernel sections. */
+int irb_deconvolve_chop_batch(const float* nums, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
+                              int include_amplitude, int ir_length, float threshold_db, int consecutive, int normalize, float goal_db, float* out, int* positions);
 /* fp::ir::invertFilter (fp/ir.hpp:20, fp/ir.cpp:13-18); out[nextPowerOfTwo(len)] */
 int irb_invert_filter(const float* x, int len, int sample_rate, float* out);
 /* fp::convolution::averagingFilter (fp/convolution.hpp:44, fp/convolution.cpp:406-546), in place on an interleaved

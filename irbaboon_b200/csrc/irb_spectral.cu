@@ -1,7 +1,7 @@
 // irb_spectral.cu -- host side of the single-large-FFT entry points of include/irb_b200.h:
 // irb_convolve_nonperiodic, irb_convolve_batch(_device), irb_deconvolve(_batch), irb_averaging_filter, irb_fft_transform,
-// irb_fft_inv_transform, irb_invert_filter, irb_ess_generate.  Every arithmetic step is a kernel of
-// irb_spectral.cuh; the host only sizes buffers, copies and launches.
+// irb_fft_inv_transform, irb_invert_filter, irb_ess_generate, irb_ir_chop_batch_device, irb_deconvolve_chop_batch.  Every
+// arithmetic step is a kernel of irb_spectral.cuh or irb_chop.cuh; the host only sizes buffers, copies and launches.
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
@@ -9,6 +9,7 @@
 #include <cstring>
 #include <vector>
 
+#include "irb_chop.cuh"
 #include "irb_common.hpp"
 #include "irb_spectral.cuh"
 #include "irb_tuning.hpp"
@@ -255,6 +256,50 @@ int fft_size_for(int len, int* N) {
     return 0;
 }
 
+// fp::ir::IRchop (+ fp::tools::normalize) of rows of a batch (irb_chop.cuh); positions: [rows][2] device memory, or null
+struct ChopSpec {
+    int ir_length;
+    float threshold_db;
+    int consecutive, normalize;
+    float goal_lin;               // tools::dBToLin(goal_db), computed here on the host as the facade does
+    int* positions;               // the caller's [batch][2], or null
+};
+
+// every argument error of the chop, before any CUDA call; len: the samples of each row the chop reads
+int chop_spec(int len, int ir_length, float threshold_db, int consecutive, int normalize, float goal_db, int* positions, ChopSpec* c) {
+    if (ir_length < 1 || ir_length > len) return fail(IRB_ERR_ARG, "ir_length %d outside [1, %d]: the IR is cut from rows of %d samples", ir_length, len, len);
+    *c = ChopSpec{ir_length, threshold_db, consecutive, normalize != 0, std::pow(10.0f, goal_db / 20.0f), positions};
+    return 0;
+}
+
+// chunks per row of the peak pass: about 8 CTAs per SM over the batch, at least 8192 samples per chunk
+int chop_chunks(int rows, long long len, long long* chunk_len) {
+    constexpr long long kTargetCtas = 148 * 8, kMinChunk = 8192;
+    long long chunks = std::max(1LL, std::min((kTargetCtas + rows - 1) / rows, (len + kMinChunk - 1) / kMinChunk));
+    *chunk_len = ((len + chunks - 1) / chunks + 3) & ~3LL;
+    return (int) ((len + *chunk_len - 1) / *chunk_len);
+}
+
+// bytes of the peak pass's partial results for rows x chunks
+size_t chop_part_bytes(int rows, int chunks) { return (sizeof(long long) + sizeof(float)) * (size_t) rows * chunks; }
+
+// rows of x[rows][len] (device) -> out[rows][c.ir_length] and pos[rows][2] (device, or null); chunks / chunk_len from chop_chunks,
+// part: chop_part_bytes(rows, chunks)
+int launch_chop(const float* x, int rows, long long len, int chunks, long long chunk_len, const ChopSpec& c, float* out, int* pos, void* part, cudaStream_t st) {
+    long long* part_i = static_cast<long long*>(part);
+    float* part_m = reinterpret_cast<float*>(part_i + (size_t) rows * chunks);
+    const bool vec = (uintptr_t) x % 16 == 0 && len % 4 == 0;
+    if (vec) irb::k_chop_peak<true><<<(unsigned) ((long long) rows * chunks), irb::kChopPeakThreads, 0, st>>>(x, len, chunks, chunk_len, part_m, part_i);
+    else irb::k_chop_peak<false><<<(unsigned) ((long long) rows * chunks), irb::kChopPeakThreads, 0, st>>>(x, len, chunks, chunk_len, part_m, part_i);
+    g_launches++;
+    CK(cudaGetLastError());
+    irb::ChopArgs a{x, len, chunks, part_m, part_i, c.ir_length, c.consecutive, c.normalize, c.threshold_db, c.goal_lin, out, pos};
+    irb::k_chop_cut<<<(unsigned) rows, irb::kChopCutThreads, 0, st>>>(a);
+    g_launches++;
+    CK(cudaGetLastError());
+    return 0;
+}
+
 }  // namespace
 
 // One batched spectral product, the core of the batched division and of the (batched) linear convolution:
@@ -269,6 +314,7 @@ struct BatchJob {
     bool divide;
     OutWindow win;
     float* out;
+    const ChopSpec* chop = nullptr;              // division only: out[batch][ir_length] holds each row cut by the chop
     long long out_row() const { return win.len >= 0 ? win.len : N; }
 };
 
@@ -287,7 +333,7 @@ static int batch_staged(const BatchJob& J, double sample_rate, int smoothing, in
     CK(cudaSetDevice(dev));
     Plan plan;
     if ((rc = plan.init(dev, M))) return rc;
-    struct Slot { DevBuf dn, Zn, dy, dy2, tmp, dh, Zh, Bh; cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr, t0 = nullptr, t1 = nullptr;
+    struct Slot { DevBuf dn, Zn, dy, dy2, tmp, dh, Zh, Bh, dc, dpos, dpart; cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr, t0 = nullptr, t1 = nullptr;
                   bool dn_busy = false, dy_busy = false, timed = false;
                   ~Slot() { for (cudaEvent_t e : {ev_in, ev_done, ev_out, t0, t1}) if (e) cudaEventDestroy(e); } } slot[4];   // [2], [3]: the smoothing path's last phase
     // smoothing runs in up to kLanes groups of captures at once, each on its own compute stream with its own spectrum array and
@@ -324,6 +370,8 @@ static int batch_staged(const BatchJob& J, double sample_rate, int smoothing, in
     const int ngroups = (batch + grp - 1) / grp, nlanes = std::min(ngroups, lanes_pref);
     const float smooth_per_avg = 1.0 / 13.0;                                          // fp/convolution.cpp:390 (a float there)
     const int nslots = batch > sub ? 2 : 1;
+    long long chop_chunk_len = 0;
+    const int chop_chunks_n = J.chop ? chop_chunks(sub, N, &chop_chunk_len) : 0;
     for (int i = 0; i < (smoothing ? 2 * nslots : nslots); ++i) {
         Slot& q = slot[i < nslots ? i : 2 + (i - nslots)];
         const bool first = i < nslots, last = !smoothing || !first;                // which phase(s) of the pipeline the slot serves
@@ -332,6 +380,9 @@ static int batch_staged(const BatchJob& J, double sample_rate, int smoothing, in
             return rc;
         if (!fused && (rc = q.tmp.alloc(sizeof(float2) * (size_t) M * sub, false))) return rc;
         if (last && !include_phase && (rc = q.dy2.alloc(sizeof(float) * (size_t) N * sub, false))) return rc;
+        if (last && J.chop && ((rc = q.dc.alloc(sizeof(float) * (size_t) J.chop->ir_length * sub, false)) || (rc = q.dpos.alloc(sizeof(int) * 2 * (size_t) sub, false)) ||
+                               (rc = q.dpart.alloc(chop_part_bytes(sub, chop_chunks_n), false))))
+            return rc;
         if (per_item && ((rc = q.dh.alloc(sizeof(float) * lde * sub, true)) || (rc = q.Zh.alloc(sizeof(float2) * (size_t) M * sub, false)) ||
                          (fused && (rc = q.Bh.alloc(sizeof(float2) * (size_t) M * sub, false)))))
             return rc;
@@ -391,7 +442,7 @@ static int batch_staged(const BatchJob& J, double sample_rate, int smoothing, in
         CK(cudaStreamWaitEvent(cs, q.ev_in, 0));
         return 0;
     };
-    // inverse-transformed sub-batch in q.dy -> (half swap) -> host
+    // inverse-transformed sub-batch in q.dy -> (half swap) -> (chop) -> host
     auto download = [&](Slot& q, int b0, int nb, cudaStream_t cs) -> int {
         const float* res = q.dy.as<float>();
         if (!include_phase) {                                                        // ir::shifteroo, fp/convolution.cpp:400
@@ -399,11 +450,18 @@ static int batch_staged(const BatchJob& J, double sample_rate, int smoothing, in
             LAUNCHED();
             res = q.dy2.as<float>();
         }
+        if (J.chop) { int rc2 = launch_chop(res, nb, N, chop_chunks_n, chop_chunk_len, *J.chop, q.dc.as<float>(), q.dpos.as<int>(), q.dpart.p, cs); if (rc2) return rc2; }
         if (smoothing) { int rc2 = spans.close(cs); if (rc2) return rc2; }
         else CK(cudaEventRecord(q.t1, cs));
         CK(cudaEventRecord(q.ev_done, cs));
         CK(cudaStreamWaitEvent(sg_out.s, q.ev_done, 0));
-        CK(cudaMemcpyAsync(J.out + (size_t) b0 * out_row, res, sizeof(float) * (size_t) out_row * nb, cudaMemcpyDefault, sg_out.s));
+        if (J.chop) {                                                                // only the IRs (and their positions) leave the device
+            const long long Lw = J.chop->ir_length;
+            CK(cudaMemcpyAsync(J.out + (size_t) b0 * Lw, q.dc.p, sizeof(float) * (size_t) Lw * nb, cudaMemcpyDefault, sg_out.s));
+            if (J.chop->positions) CK(cudaMemcpyAsync(J.chop->positions + 2 * (size_t) b0, q.dpos.p, sizeof(int) * 2 * (size_t) nb, cudaMemcpyDefault, sg_out.s));
+        } else {
+            CK(cudaMemcpyAsync(J.out + (size_t) b0 * out_row, res, sizeof(float) * (size_t) out_row * nb, cudaMemcpyDefault, sg_out.s));
+        }
         CK(cudaEventRecord(q.ev_out, sg_out.s));
         q.dy_busy = true;
         return 0;
@@ -704,6 +762,43 @@ int irb_deconvolve_batch_device(const float* nums_dev, int batch, int len_num, c
     if (!(plan.big() && !smoothing && include_phase && len_num % 2 == 0 && aligned))
         return batch_staged(J, sample_rate, smoothing, include_phase, include_amplitude, true);
     return batch_direct(J, plan);
+}
+
+int irb_deconvolve_chop_batch(const float* nums, int batch, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase,
+                              int include_amplitude, int ir_length, float threshold_db, int consecutive, int normalize, float goal_db, float* out, int* positions) {
+    BatchJob J;
+    ChopSpec c;
+    int rc;
+    if ((rc = deconvolve_job(nums, batch, len_num, den, len_den, out, &J)) || (rc = chop_spec(J.N, ir_length, threshold_db, consecutive, normalize, goal_db, positions, &c)))
+        return rc;
+    J.chop = &c;
+    return batch_staged(J, sample_rate, smoothing, include_phase, include_amplitude, false);
+}
+
+int irb_ir_chop_batch_device(const float* x_dev, int batch, int len, int ir_length, float threshold_db, int consecutive, int normalize, float goal_db, float* out_dev,
+                             int* positions) {
+    if (!x_dev || !out_dev) return fail(IRB_ERR_ARG, "null argument");
+    if (batch < 1 || len < 1) return fail(IRB_ERR_ARG, "empty input");
+    ChopSpec c;
+    int rc;
+    if ((rc = chop_spec(len, ir_length, threshold_db, consecutive, normalize, goal_db, positions, &c))) return rc;
+    CK(cudaSetDevice(irbh::current_device()));
+    long long chunk_len = 0;
+    const int chunks = chop_chunks(batch, len, &chunk_len);
+    DevBuf part;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    struct EvGuard { cudaEvent_t &a, &b; ~EvGuard() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); } } evg{e0, e1};
+    irbh::StreamGuard sg;
+    if ((rc = sg.create()) || (rc = part.alloc(chop_part_bytes(batch, chunks), false))) return rc;
+    CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
+    CK(cudaEventRecord(e0, sg.s));
+    if ((rc = launch_chop(x_dev, batch, len, chunks, chunk_len, c, out_dev, positions, part.p, sg.s))) return rc;
+    CK(cudaEventRecord(e1, sg.s));
+    CK(cudaEventSynchronize(e1));
+    float ms = 0.f;
+    CK(cudaEventElapsedTime(&ms, e0, e1));
+    irbh::set_last_compute_ms((double) ms);
+    return 0;
 }
 
 int irb_deconvolve(const float* num, int len_num, const float* den, int len_den, double sample_rate, int smoothing, int include_phase, int include_amplitude,

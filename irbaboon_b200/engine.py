@@ -90,6 +90,9 @@ _SIGS = {
     "irb_deconvolve": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_deconvolve_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_deconvolve_batch_device": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
+    "irb_ir_chop_batch_device": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_int, ctypes.c_int, ctypes.c_float, _vp, _vp]),
+    "irb_deconvolve_chop_batch": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                 ctypes.c_int, ctypes.c_float, ctypes.c_int, ctypes.c_int, ctypes.c_float, _vp, _vp]),
     "irb_invert_filter": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _vp]),
     "irb_averaging_filter": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_double, ctypes.c_double, ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "irb_fft_transform": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp]),
@@ -399,6 +402,45 @@ def deconvolve_batch_device(nums_ptr, batch, len_num, den, out_ptr, sample_rate=
     den = np.ascontiguousarray(den, np.float32).reshape(-1)
     _ck(lib().irb_deconvolve_batch_device(_vp(int(nums_ptr)), int(batch), int(len_num), _ptr(den), len(den), float(sample_rate), int(smoothing), int(include_phase),
                                           int(include_amplitude), _vp(int(out_ptr))))
+
+
+def _check_chop(batch, length, ir_length):
+    if int(batch) < 1 or int(length) < 1:
+        raise ValueError("batch %r and row length %r must be at least 1" % (batch, length))
+    if not 1 <= int(ir_length) <= int(length):
+        raise ValueError("ir_length %r outside [1, %d]: the IR is cut from rows of %d samples" % (ir_length, int(length), int(length)))
+
+
+def ir_chop_batch_device(x_ptr, batch, len, ir_length, out_ptr, threshold_db=-60.0, consecutive=50, normalize=True, goal_db=0.0, positions_ptr=None):
+    """irb_ir_chop_batch_device: fp::ir::IRchop (+ fp::tools::normalize(goal_db)) of every row of x[batch][len] -> out[batch][ir_length];
+    x_ptr, out_ptr and positions_ptr ([batch][2] int32 {peak index, start}, optional) are raw DEVICE pointers (ints)."""
+    _check_chop(batch, len, ir_length)
+    if not x_ptr or not out_ptr:
+        raise ValueError("x_ptr and out_ptr must be device pointers")
+    _ck(lib().irb_ir_chop_batch_device(_vp(int(x_ptr)), int(batch), int(len), int(ir_length), float(threshold_db), int(consecutive), int(bool(normalize)),
+                                       float(goal_db), _vp(int(out_ptr)), _vp(int(positions_ptr)) if positions_ptr else None))
+
+
+def deconvolve_chop_batch(nums, den, ir_length, sample_rate=48000.0, smoothing=False, include_phase=True, include_amplitude=True, threshold_db=-60.0,
+                          consecutive=50, normalize=True, goal_db=0.0, out=None, return_positions=False):
+    """irb_deconvolve_chop_batch: deconvolve_batch(nums, den, ...) with every row cut by ir_chop_batch_device on the device
+    -> out[batch][ir_length] (and, with return_positions, int32 [batch][2] {peak index, start})."""
+    nums = np.ascontiguousarray(nums, np.float32)
+    nums = nums[None, :] if nums.ndim == 1 else nums
+    den = np.ascontiguousarray(den, np.float32).reshape(-1)
+    if nums.ndim != 2 or len(den) < 1:
+        raise ValueError("nums must be [batch][len_num] and den a non-empty [len_den], got %r and %r" % (nums.shape, den.shape))
+    N = next_pow2(max(nums.shape[1], len(den)))
+    _check_chop(nums.shape[0], N, ir_length)
+    if out is None:
+        out = np.empty((nums.shape[0], int(ir_length)), np.float32)
+    elif not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.shape == (nums.shape[0], int(ir_length)) and out.flags.c_contiguous and out.flags.writeable):
+        raise ValueError("out must be a writable C-contiguous float32 array of shape %r" % ((nums.shape[0], int(ir_length)),))
+    pos = np.empty((nums.shape[0], 2), np.int32) if return_positions else None
+    _ck(lib().irb_deconvolve_chop_batch(_ptr(nums), nums.shape[0], nums.shape[1], _ptr(den), len(den), float(sample_rate), int(smoothing), int(include_phase),
+                                        int(include_amplitude), int(ir_length), float(threshold_db), int(consecutive), int(bool(normalize)), float(goal_db),
+                                        _ptr(out), _ptr(pos) if pos is not None else None))
+    return (out, pos) if return_positions else out
 
 
 def invert_filter(x, sample_rate=48000):

@@ -19,6 +19,11 @@ AudioBuffer<float> createIRFilt(AudioBuffer<float>& irTarget, AudioBuffer<float>
 // an IR cut to irLength around its peak (ir::IRchop) and normalised to 0 dB (tools::normalize): library functions of
 // fp/ir.hpp and fp/tools.hpp composed for convenience -- the plug-in itself never calls IRchop
 AudioBuffer<float> chopAndNormalize(AudioBuffer<float>& ir, int irLength, float thresholdLeveldB, int consecutiveSamplesBelowThreshold);
+// the batched form of captureToIR + chopAndNormalize: one capture per channel of `captures`, all divided by sweepForDeconv, cut and
+// normalised on the GPU (irb_deconvolve_chop_batch) -> one IR of irLength samples per channel; only the IRs leave the device.
+// smoothing = false skips the 1/13-octave smoothing the plug-in applies.
+AudioBuffer<float> capturesToIRs(AudioBuffer<float>& captures, AudioBuffer<float>& sweepForDeconv, double sampleRate, int irLength, float thresholdLeveldB,
+                                 int consecutiveSamplesBelowThreshold, bool smoothing = true);
 
 }  // namespace b200
 }  // namespace fp

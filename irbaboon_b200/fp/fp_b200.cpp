@@ -746,6 +746,16 @@ AudioBuffer<float> chopAndNormalize(AudioBuffer<float>& ir, int irLength, float 
     tools::normalize(&out, 0.0f, false);
     return out;
 }
+AudioBuffer<float> capturesToIRs(AudioBuffer<float>& captures, AudioBuffer<float>& sweepForDeconv, double sampleRate, int irLength, float thresholdLeveldB,
+                                 int consecutiveSamplesBelowThreshold, bool smoothing) {
+    const int batch = captures.getNumChannels(), n = captures.getNumSamples();
+    std::vector<float> x = pack(captures);
+    AudioBuffer<float> out(batch, irLength);
+    if (irb_deconvolve_chop_batch(x.data(), batch, n, sweepForDeconv.getReadPointer(0), sweepForDeconv.getNumSamples(), sampleRate, smoothing, 1, 1, irLength,
+                                  thresholdLeveldB, consecutiveSamplesBelowThreshold, 1, 0.0f, out.getWritePointer(0), nullptr) != IRB_OK)
+        raise("fp::b200::capturesToIRs");
+    return out;
+}
 
 }  // namespace b200
 }  // namespace fp
