@@ -87,6 +87,24 @@ int irb_engine_set_ir(irb_engine* e, int ir_id, const float* left, const float* 
  * keep it) and, if nothing was loaded before, starts from cleared spectra as prepareToPlay does (:225-226).  Taps beyond
  * n_partitions*block_size are never read; shorter IRs are zero-extended. */
 int irb_engine_stage_ir(irb_engine* e, int ir_id, const float* left, const float* right, int n_taps, int n_partitions);
+/* n IRs in one call.  Row j (taps + j*ld, and right + j*ld when right != NULL, folded to (L+R)/2) holds n_taps[j] taps
+ * (n_taps == NULL: ld taps each) for IR ir_ids[j].  taps/right: host memory (pageable or pinned) or device memory of the
+ * engine's device, any 4-byte alignment (both of one kind).  Row j's result is exactly what irb_engine_set_ir / _stage_ir of
+ * that row gives, and rows are applied in order j = 0, 1, ....  Returns when the spectra are in place (one sync of the engine's
+ * stream).  Device taps are read on the engine's stream (irb_engine_set_stream): a writer on another stream orders its write
+ * before the call, as for _process_device.  Host taps go through a bounded staging area (at most 64 MB per side and chunk, two
+ * chunks in flight, from the workspace pool when the rows exceed the engine's own buffer), the upload of one chunk overlapping
+ * the transform of the previous one.
+ * One kernel (k_ir_load) per chunk transforms every partition of every row, writes every copy of the spectra, clears the ring
+ * partitions past each IR's last and, for staged IRs, writes the zero-extended taps into their round-robin buffers.
+ * All or nothing: every argument error is IRB_ERR_ARG, returned before any CUDA call and before anything is loaded -- a null
+ * engine, ir_ids or taps; n < 1; an id outside [0, n_irs) or repeated; n_taps[j] < 1; ld < n_taps[j]; for _set_irs
+ * n_taps[j] > block_size * max_partitions; for _stage_irs more partitions than max_partitions by stage_ir's rule per row.  Then
+ * the pointers are classified: device memory of another device, or taps and right of different kinds, are IRB_ERR_ARG too.
+ * irb_engine_set_ir / _stage_ir are the one-row calls of these. */
+int irb_engine_set_irs(irb_engine* e, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps);
+int irb_engine_stage_irs(irb_engine* e, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps,
+                         int n_partitions);
 /* channels [chan_begin, chan_end) convolve with ir_id.  When every kernel tile (irb_engine_tile_channels()
  * consecutive channels) is bound to one IR the tile shares the staged IR spectra; otherwise every channel stages its own
  * partitions (twice the memory traffic).  Either way a block step is one launch of the persistent kernel. */
@@ -189,6 +207,12 @@ int irb_group_device_count(const irb_group* g);
 int irb_group_channel_range(const irb_group* g, int index, int* begin, int* end);
 int irb_group_set_ir(irb_group* g, int ir_id, const float* left, const float* right, int n_taps);
 int irb_group_stage_ir(irb_group* g, int ir_id, const float* left, const float* right, int n_taps, int n_partitions);
+/* host memory only; private-IR groups (n_irs == 0) send each row to the device that owns channel ir_ids[j], shared-IR groups
+ * send every row to every device; every device's copies and kernels are enqueued before the first wait (as irb_group_process).
+ * Arguments as irb_engine_set_irs / _stage_irs; device memory is IRB_ERR_ARG.  irb_group_set_ir / _stage_ir are their one-row calls. */
+int irb_group_set_irs(irb_group* g, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps);
+int irb_group_stage_irs(irb_group* g, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps,
+                        int n_partitions);
 int irb_group_bind(irb_group* g, int chan_begin, int chan_end, int ir_id);
 int irb_group_reset(irb_group* g);
 int irb_group_process(irb_group* g, const float* in_host, float* out_host, int n_blocks);

@@ -28,6 +28,8 @@ int irbx_engine_mac_only_device(irb_engine* e, float* acc_dev);
  * stores at [16 b + phase] the %globaltimer (ns) at kernel start, after the set-up, after the forward transform, after the partition loop, before and after
  * each cluster barrier and at the end.  NULL switches it off (the default). */
 int irbx_engine_set_stamps(irb_engine* e, unsigned long long* stamps_dev);
+/* identical copies of the IR spectra the engine keeps (the h_reps the block steps read and every IR load writes) */
+int irbx_engine_ir_copies(const irb_engine* e);
 /* With the same pointer set (at least 4096 x 4 uint64), the persistent block-step kernel k_mac_p logs per launch, at
  * [4 (launch % 4096) + {0,1,2,3}], CTA 0's {%globaltimer at start, SM cycle counter at start, %globaltimer at end, cycle counter at end}:
  * cycles / ns is the SM clock the step ran at. */

@@ -12,7 +12,7 @@ _ROOT = os.path.dirname(_HERE)
 CSRC = os.path.join(_HERE, "csrc")
 LIB = os.path.join(_HERE, "libirb_b200.so")
 SOURCES = ["irb_engine.cu", "irb_spectral.cu", "irb_benchaids.cu"]
-HEADERS = ["irb_chop.cuh", "irb_fft.cuh", "irb_kernels.cuh", "irb_mac_p.cuh", "irb_mac_mx.cuh", "irb_spectral.cuh", "irb_common.hpp", "irb_tuning.hpp",
+HEADERS = ["irb_chop.cuh", "irb_fft.cuh", "irb_ir_load.cuh", "irb_kernels.cuh", "irb_mac_p.cuh", "irb_mac_mx.cuh", "irb_spectral.cuh", "irb_common.hpp", "irb_tuning.hpp",
            os.path.join(_ROOT, "include", "irb_b200.h"), os.path.join(_ROOT, "include", "irb_b200_bench.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [

@@ -89,6 +89,7 @@ int irbx_get_tuning(const char* name) {
 
 int irbx_engine_mac_only_device(irb_engine* e, float* acc_dev) { return irbh::engine_mac_only(e, acc_dev); }
 int irbx_engine_set_stamps(irb_engine* e, unsigned long long* stamps_dev) { return irbh::engine_set_stamps(e, stamps_dev); }
+int irbx_engine_ir_copies(const irb_engine* e) { return irbh::engine_ir_copies(e); }
 
 int irbx_hbm_read_probe(size_t bytes, int iters, int write_every, int store_kind, double* gbs) {
     if (!gbs || iters < 1 || bytes < (1u << 20)) return fail(IRB_ERR_ARG, "bad argument");

@@ -113,4 +113,4 @@ inline int next_pow2(int x) {                                  // tools::nextPow
 }  // namespace irbh
 
 struct irb_engine;
-namespace irbh { int engine_mac_only(irb_engine* e, float* acc_dev); int engine_set_stamps(irb_engine* e, unsigned long long* dev); }
+namespace irbh { int engine_mac_only(irb_engine* e, float* acc_dev); int engine_set_stamps(irb_engine* e, unsigned long long* dev); int engine_ir_copies(const irb_engine* e); }

@@ -18,6 +18,7 @@
 
 #include "irb_common.hpp"
 #include "irb_kernels.cuh"
+#include "irb_ir_load.cuh"
 #include "irb_mac_p.cuh"
 #include "irb_mac_mx.cuh"
 #include "irb_tuning.hpp"
@@ -381,18 +382,19 @@ struct irb_engine {
     cudaStream_t own_stream = nullptr, stream = nullptr;
     const float2* W = nullptr;
     DevBuf fdl, H, ov, head, ir_of_chan, nparts, io_in[2], io_out[2], taps;
+    // IR loads (irb_engine_set_irs / _stage_irs): the item table of k_ir_load, grown on demand; the pooled staging of a load from
+    // host memory larger than `taps`, held until the load is waited for; upload / transform events of its two staging slots
+    DevBuf ld_tab;
+    size_t ld_tab_cap = 0;
+    std::unique_ptr<irbh::ScratchBuf> ld_stage;
+    cudaEvent_t ld_ev[4] = {nullptr, nullptr, nullptr, nullptr};
     DevBuf work;                       // k_mac_p: {next unit, finished CTAs}, cleared by the kernel itself
     unsigned long long* stamps = nullptr;   // measurement only (irbx_engine_set_stamps): phase time stamps of the latency-path kernel
     int h_reps = 1;                    // identical copies of the IR spectra H (MacArgs::h_reps): [rep][ir][partition][M]
     long long h_rep_stride() const { return (long long) n_irs * ring * M; }
-    // clear / replicate the spectra of one IR across the copies (copy 0 is the one every writer fills)
+    // clear the spectra of one IR in every copy
     int ir_clear_all(int ir, cudaStream_t st) {
         for (int r = 0; r < h_reps; ++r) CK(cudaMemsetAsync(H.as<float2>() + r * h_rep_stride() + (size_t) ir * ring * M, 0, sizeof(float2) * (size_t) M * ring, st));
-        return 0;
-    }
-    int ir_replicate(int ir, cudaStream_t st) {
-        const float2* src = H.as<float2>() + (size_t) ir * ring * M;
-        for (int r = 1; r < h_reps; ++r) CK(cudaMemcpyAsync(H.as<float2>() + r * h_rep_stride() + (size_t) ir * ring * M, src, sizeof(float2) * (size_t) M * ring, cudaMemcpyDeviceToDevice, st));
         return 0;
     }
     std::vector<int> h_ir_of_chan, h_nparts;
@@ -439,6 +441,7 @@ struct irb_engine {
     ~irb_engine() {
         for (auto ev : tev) cudaEventDestroy(ev);
         for (auto ev : ev_grp) if (ev) cudaEventDestroy(ev);
+        for (auto ev : ld_ev) if (ev) cudaEventDestroy(ev);
         for (int i = 0; i < 2; ++i) {
             if (ev_in[i]) cudaEventDestroy(ev_in[i]);
             if (ev_done[i]) cudaEventDestroy(ev_done[i]);
@@ -777,37 +780,9 @@ int irb_engine_reset(irb_engine* e) {
     return 0;
 }
 
+// One-row calls of irb_engine_set_irs / _stage_irs (their checks, their launch; same results and errors as ever).
 int irb_engine_set_ir(irb_engine* e, int ir_id, const float* left, const float* right, int n_taps) {
-    if (!e || !left) return fail(IRB_ERR_ARG, "engine or taps null");
-    if (ir_id < 0 || ir_id >= e->n_irs) return fail(IRB_ERR_ARG, "ir_id %d outside [0, %d)", ir_id, e->n_irs);
-    if (n_taps < 1 || (long long) n_taps > (long long) e->B * e->ring) return fail(IRB_ERR_ARG, "n_taps %d outside [1, %lld]", n_taps, (long long) e->B * e->ring);
-    CK(cudaSetDevice(e->device));
-    const int P = (int) std::ceil((float) n_taps / (float) e->B);          // fp/convolution.cpp:52
-    float* dl = e->taps.as<float>();
-    float* dr = dl + (size_t) e->B * e->ring;
-    CK(cudaMemcpyAsync(dl, left, sizeof(float) * n_taps, cudaMemcpyHostToDevice, e->stream));
-    if (right) CK(cudaMemcpyAsync(dr, right, sizeof(float) * n_taps, cudaMemcpyHostToDevice, e->stream));
-    float2* Hd = e->H.as<float2>() + (size_t) ir_id * e->ring * e->M;
-    int rc = e->ir_clear_all(ir_id, e->stream);
-    if (rc) return rc;
-    irb::FwdArgs f{};
-    f.src = dl; f.src2 = right ? dr : nullptr; f.src_chan_stride = 0; f.L = n_taps; f.B = e->B;
-    f.blocks_per_chan = P; f.n_rows = P; f.dst = Hd; f.dst_chan_stride = 0; f.head = nullptr; f.ring = e->ring; f.W = e->W;
-    if ((rc = launch_fwd(e->M, f, e->stream))) return rc;
-    e->launches += 1;
-    if ((rc = e->ir_replicate(ir_id, e->stream))) return rc;
-    if (e->rr_buf[ir_id]) {            // a staged (round-robin) IR: the refresh must keep producing these taps
-        float* rb = e->rr_buf[ir_id]->as<float>();
-        CK(cudaMemsetAsync(rb, 0, sizeof(float) * (size_t) e->B * e->ring, e->stream));
-        if (right) { irb::k_fold_mono<<<(n_taps + 255) / 256, 256, 0, e->stream>>>(dl, dr, rb, n_taps); g_launches++; CK(cudaGetLastError()); }
-        else CK(cudaMemcpyAsync(rb, dl, sizeof(float) * n_taps, cudaMemcpyDeviceToDevice, e->stream));
-        if (P != e->h_nparts[ir_id]) CK(cudaMemsetAsync(e->rr_pos.as<int>() + ir_id, 0, sizeof(int), e->stream));
-    }
-    if (P != e->h_nparts[ir_id]) e->plan_dirty = true;
-    e->h_nparts[ir_id] = P;
-    CK(cudaMemcpyAsync(e->nparts.as<int>() + ir_id, &e->h_nparts[ir_id], sizeof(int), cudaMemcpyHostToDevice, e->stream));
-    CK(cudaStreamSynchronize(e->stream));
-    return 0;
+    return irb_engine_set_irs(e, 1, &ir_id, left, right, n_taps, &n_taps);
 }
 
 // "IRtoConvolve = this buffer" (PluginProcessor.cpp:411-414): nothing is transformed here; every following block step
@@ -815,50 +790,7 @@ int irb_engine_set_ir(irb_engine* e, int ir_id, const float* left, const float* 
 // by partition over nparts blocks.  The first call for an IR fixes its partition count (n_partitions, or
 // ceil(n_taps / block_size) when 0) and starts from cleared spectra, as prepareToPlay does (:225-226).
 int irb_engine_stage_ir(irb_engine* e, int ir_id, const float* left, const float* right, int n_taps, int n_partitions) {
-    if (!e || !left) return fail(IRB_ERR_ARG, "engine or taps null");
-    if (ir_id < 0 || ir_id >= e->n_irs) return fail(IRB_ERR_ARG, "ir_id %d outside [0, %d)", ir_id, e->n_irs);
-    if (n_taps < 1) return fail(IRB_ERR_ARG, "n_taps %d < 1", n_taps);
-    int P = n_partitions > 0 ? n_partitions : (e->h_nparts[ir_id] > 0 ? e->h_nparts[ir_id] : (int) std::ceil((float) n_taps / (float) e->B));
-    if (P > e->ring) return fail(IRB_ERR_ARG, "%d partitions exceed max_partitions %d", P, e->ring);
-    CK(cudaSetDevice(e->device));
-    const size_t cap = (size_t) e->B * e->ring;
-    const bool first = !e->rr_buf[ir_id];
-    if (first) {
-        std::unique_ptr<DevBuf> b(new (std::nothrow) DevBuf);
-        if (!b) return fail(IRB_ERR_ARG, "out of host memory");
-        int rc = b->alloc(sizeof(float) * cap, false);
-        if (rc) return rc;
-        e->rr_buf[ir_id] = std::move(b);
-        e->bytes += sizeof(float) * cap;
-        const float* ptr = e->rr_buf[ir_id]->as<float>();
-        CK(cudaMemcpyAsync(e->rr_ptrs.as<const float*>() + ir_id, &ptr, sizeof(ptr), cudaMemcpyHostToDevice, e->stream));
-        e->h_rr_list.push_back(ir_id);
-        CK(cudaMemcpyAsync(e->rr_list.p, e->h_rr_list.data(), sizeof(int) * e->h_rr_list.size(), cudaMemcpyHostToDevice, e->stream));
-    }
-    const int keep = (int) std::min<size_t>((size_t) n_taps, (size_t) P * e->B);      // taps beyond the partitions are never read
-    float* rb = e->rr_buf[ir_id]->as<float>();
-    CK(cudaMemsetAsync(rb, 0, sizeof(float) * cap, e->stream));
-    if (right) {
-        float* dl = e->taps.as<float>();
-        float* dr = dl + cap;
-        CK(cudaMemcpyAsync(dl, left, sizeof(float) * keep, cudaMemcpyHostToDevice, e->stream));
-        CK(cudaMemcpyAsync(dr, right, sizeof(float) * keep, cudaMemcpyHostToDevice, e->stream));
-        irb::k_fold_mono<<<(keep + 255) / 256, 256, 0, e->stream>>>(dl, dr, rb, keep);
-        g_launches++;
-        CK(cudaGetLastError());
-    } else {
-        CK(cudaMemcpyAsync(rb, left, sizeof(float) * keep, cudaMemcpyHostToDevice, e->stream));
-    }
-    if (P != e->h_nparts[ir_id]) {
-        if (e->h_nparts[ir_id] == 0)               // nothing was ever loaded for this IR: its partitions fade in from cleared spectra
-            { int rc2 = e->ir_clear_all(ir_id, e->stream); if (rc2) return rc2; }
-        CK(cudaMemsetAsync(e->rr_pos.as<int>() + ir_id, 0, sizeof(int), e->stream));
-        e->h_nparts[ir_id] = P;
-        CK(cudaMemcpyAsync(e->nparts.as<int>() + ir_id, &e->h_nparts[ir_id], sizeof(int), cudaMemcpyHostToDevice, e->stream));
-        e->plan_dirty = true;
-    }
-    CK(cudaStreamSynchronize(e->stream));
-    return 0;
+    return irb_engine_stage_irs(e, 1, &ir_id, left, right, n_taps, &n_taps, n_partitions);
 }
 
 int irb_engine_bind(irb_engine* e, int chan_begin, int chan_end, int ir_id) {
@@ -1043,6 +975,295 @@ int engine_process_enqueue(irb_engine* e, const void* in_host, int in_fmt, void*
     return 0;
 }
 }  // namespace
+
+}  // extern "C"
+
+// ---- IR loads: irb_engine_set_irs / _stage_irs and the group forms, one k_ir_load launch per chunk (irb_ir_load.cuh) ----------
+namespace {
+constexpr size_t kLoadSlotBytes = 64ull << 20;        // host sources: taps staged per chunk and side; two chunks in flight
+
+// the partition count set_ir has always used: float ceil (fp/convolution.cpp:52)
+int parts_for(int n_taps, int B) { return (int) std::ceil((float) n_taps / (float) B); }
+
+// One load into one engine: row j (local IR ids[j]) is row rows[j] of the caller's array taps / right with stride ld.
+struct LoadSpec {
+    std::vector<int> ids, rows;
+    const float* taps = nullptr;
+    const float* right = nullptr;
+    long long ld = 0;
+    const int* n_taps = nullptr;       // [caller rows]; null: ld taps each
+    int src_rows = 0;                  // rows of the caller's array: the last one may end at its own n_taps (no read past it)
+    bool stage = false;
+    int n_partitions = 0;
+    int taps_of(int j) const { return n_taps ? n_taps[rows[j]] : (int) ld; }
+};
+
+// stage_ir's partition rule for a row
+int stage_parts(const irb_engine* e, int ir, int nt, int n_partitions) {
+    return n_partitions > 0 ? n_partitions : (e->h_nparts[ir] > 0 ? e->h_nparts[ir] : parts_for(nt, e->B));
+}
+
+// the argument errors a load's rows carry whatever the engine: null ids or taps, n < 1, a row without taps or longer than ld,
+// a repeated id.  Checked before the engine itself, so that they are reported without a device.
+int rows_check(int n, const int* ids, const float* taps, long long ld, const int* n_taps) {
+    if (!ids || !taps) return fail(IRB_ERR_ARG, "ir_ids or taps null");
+    if (n < 1) return fail(IRB_ERR_ARG, "n %d < 1", n);
+    if (!n_taps && ld > 0x7fffffffLL) return fail(IRB_ERR_ARG, "ld %lld: rows of more than 2^31 - 1 taps", ld);
+    for (int j = 0; j < n; ++j) {
+        const long long nt = n_taps ? n_taps[j] : ld;
+        if (nt < 1) return fail(IRB_ERR_ARG, "n_taps[%d] = %lld < 1", j, nt);
+        if (ld < nt) return fail(IRB_ERR_ARG, "ld %lld < n_taps[%d] = %lld", ld, j, nt);
+    }
+    std::vector<std::pair<int, int>> v((size_t) n);
+    for (int j = 0; j < n; ++j) v[j] = {ids[j], j};
+    std::sort(v.begin(), v.end());
+    for (int j = 1; j < n; ++j)
+        if (v[j].first == v[j - 1].first) return fail(IRB_ERR_ARG, "ir_ids[%d] = %d repeats ir_ids[%d]", v[j].second, v[j].first, v[j - 1].second);
+    return 0;
+}
+
+// the argument errors that depend on the engine (rows_check passed): an id outside [0, n_irs), more taps or partitions than the ring
+int load_check(const irb_engine* e, const LoadSpec& s) {
+    for (size_t j = 0; j < s.ids.size(); ++j) {
+        const int ir = s.ids[j], nt = s.taps_of((int) j);
+        if (ir < 0 || ir >= e->n_irs) return fail(IRB_ERR_ARG, "ir_ids[%d] = %d outside [0, %d)", s.rows[j], ir, e->n_irs);
+        if (!s.stage && (long long) nt > (long long) e->B * e->ring)
+            return fail(IRB_ERR_ARG, "n_taps[%d] = %d outside [1, %lld]", s.rows[j], nt, (long long) e->B * e->ring);
+        if (s.stage) {
+            const int P = stage_parts(e, ir, nt, s.n_partitions);
+            if (P > e->ring) return fail(IRB_ERR_ARG, "row %d: %d partitions exceed max_partitions %d", s.rows[j], P, e->ring);
+        }
+    }
+    return 0;
+}
+
+// where the taps are: 1 device memory the engine's kernels read in place (its own device, or managed), 0 host memory
+// (pageable or pinned), -1 device memory of another device
+int taps_location(const void* p, int dev) {
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return 0; }
+    if (at.type == cudaMemoryTypeManaged) return 1;
+    if (at.type == cudaMemoryTypeDevice) return at.device == dev ? 1 : -1;
+    return 0;
+}
+int sources_location(const float* taps, const float* right, int dev, int* loc) {
+    const int a = taps_location(taps, dev), b = right ? taps_location(right, dev) : a;
+    if (a < 0 || b < 0) return fail(IRB_ERR_ARG, "taps in device memory of another device than the engine's %d", dev);
+    if (a != b) return fail(IRB_ERR_ARG, "taps and right must both be host memory or both device memory");
+    *loc = a;
+    return 0;
+}
+
+template <int M>
+int launch_ir_load_t(const irb::IrLoadArgs& a, long long grid, cudaStream_t st) {
+    irb::k_ir_load<M><<<(unsigned) grid, irb::kThreads, 0, st>>>(a);
+    g_launches++;
+    CK(cudaGetLastError());
+    return 0;
+}
+int launch_ir_load(int M, const irb::IrLoadArgs& a, long long grid, cudaStream_t st) { IRB_DISPATCH_M(M, launch_ir_load_t<MM>(a, grid, st)); }
+
+// Enqueue a checked load on the engine's stream; engine_load_wait completes it.  Everything that can fail for want of memory (new
+// round-robin buffers, a larger item table, pooled staging, events) is acquired first, into locals: a failure there returns
+// with the engine exactly as it was.  Only then does the host state change (partition counts, round-robin buffers and list, with
+// set_ir's / stage_ir's per-IR rules), the device tables rr_ptrs, rr_list and nparts follow, and after them the copies and kernels.
+// Host taps go through staging in chunks of whole rows: the upload of chunk k+1 (copy stream s_in) overlaps the transform of chunk
+// k (the engine's stream).  Device taps are read in place by one launch.
+int engine_load_enqueue(irb_engine* e, const LoadSpec& s, bool on_dev) {
+    CK(cudaSetDevice(e->device));
+    if (e->pipe_pending) { int rc = engine_process_wait(e); if (rc) return rc; }      // s_in and the stream are free
+    const int n = (int) s.ids.size(), B = e->B;
+    const long long cap = (long long) B * e->ring;
+    // ---- plan, from the state as it is: per row the samples read, partitions, a spectra row, a cleared ring (first staging),
+    // a round-robin buffer row, an rr_pos restart
+    std::vector<int> len(n), P(n);
+    std::vector<char> xf(n), clr(n), rr(n), restart(n), fresh(n);
+    int lo = e->n_irs, hi = -1, n_fresh = 0;
+    for (int j = 0; j < n; ++j) {
+        const int ir = s.ids[j], nt = s.taps_of(j);
+        lo = std::min(lo, ir); hi = std::max(hi, ir);
+        if (!s.stage) {
+            P[j] = parts_for(nt, B); len[j] = nt; xf[j] = 1; rr[j] = e->rr_buf[ir] != nullptr;
+        } else {
+            P[j] = stage_parts(e, ir, nt, s.n_partitions);
+            len[j] = (int) std::min<long long>(nt, (long long) P[j] * B);      // taps beyond the partitions are never read
+            rr[j] = 1;
+            clr[j] = P[j] != e->h_nparts[ir] && e->h_nparts[ir] == 0;         // nothing was ever loaded: partitions fade in from cleared spectra
+            fresh[j] = !e->rr_buf[ir];
+            n_fresh += fresh[j];
+        }
+        restart[j] = rr[j] && P[j] != e->h_nparts[ir];
+    }
+    // chunks of whole rows [j0, j1), row k of a chunk staged at k * w (w: the longest row of the chunk); device taps: one chunk
+    struct Chunk { int j0, j1, w; size_t tab, n_x, n_s; long long grid; };
+    std::vector<Chunk> chunks;
+    const size_t slot = on_dev ? 0 : std::max(kLoadSlotBytes / sizeof(float), (size_t) *std::max_element(len.begin(), len.end()));
+    for (int j = 0; j < n;) {
+        Chunk c{j, j, 0, 0, 0, 0, 0};
+        while (c.j1 < n && (on_dev || (size_t) (c.j1 - c.j0 + 1) * (size_t) std::max(c.w, len[c.j1]) <= slot)) c.w = std::max(c.w, len[c.j1++]);
+        chunks.push_back(c);
+        j = c.j1;
+    }
+    std::vector<irb::IrLoadItem> tab;
+    const long long rows_per_tile = tile_rows(e->M), pieces = (cap + irb::kPiece - 1) / irb::kPiece;
+    for (auto& c : chunks) {
+        c.tab = tab.size();
+        auto off = [&](int j) { return on_dev ? (long long) s.rows[j] * s.ld : (long long) (j - c.j0) * c.w; };
+        for (int j = c.j0; j < c.j1; ++j)
+            if (xf[j] || clr[j]) tab.push_back({off(j), len[j], s.ids[j], xf[j] ? P[j] : 0, 0});
+        c.n_x = tab.size() - c.tab;
+        for (int j = c.j0; j < c.j1; ++j)
+            if (rr[j]) tab.push_back({off(j), len[j], s.ids[j], restart[j] ? 1 : 0, 0});
+        c.n_s = tab.size() - c.tab - c.n_x;
+        c.grid = ((long long) c.n_x * e->ring + rows_per_tile - 1) / rows_per_tile + (long long) c.n_s * pieces;
+        if (c.grid > 0x7fffffffLL) return fail(IRB_ERR_ARG, "a load of %lld tiles exceeds one launch", c.grid);
+    }
+    // a row stride above the copy engine's largest pitch: one copy per row instead of 2-D copies
+    int max_pitch = 0;
+    CK(cudaDeviceGetAttribute(&max_pitch, cudaDevAttrMaxPitch, e->device));
+    const bool pitched = (long long) sizeof(float) * s.ld <= (long long) max_pitch;
+    // ---- acquire: every allocation of the load, into locals
+    std::vector<std::unique_ptr<DevBuf>> bufs((size_t) n);
+    for (int j = 0; j < n; ++j) {
+        if (!fresh[j]) continue;
+        bufs[j].reset(new (std::nothrow) DevBuf);
+        if (!bufs[j]) return fail(IRB_ERR_ARG, "out of host memory");
+        if (int rc = bufs[j]->alloc(sizeof(float) * (size_t) cap, false)) { cudaGetLastError(); return rc; }      // an OOM is not left pending
+    }
+    DevBuf new_tab;
+    size_t new_tab_cap = 0;
+    if (tab.size() > e->ld_tab_cap) {
+        new_tab_cap = std::max<size_t>(tab.size(), 1024);
+        if (int rc = new_tab.alloc(sizeof(irb::IrLoadItem) * new_tab_cap, false)) { cudaGetLastError(); return rc; }
+    }
+    const int sides = s.right ? 2 : 1;
+    const bool multi = chunks.size() > 1;
+    std::unique_ptr<irbh::ScratchBuf> staging;
+    float* stage_base = nullptr;
+    size_t side_stride = 0, slot_stride = 0;             // floats between the sides of a slot, between the slots
+    if (!on_dev) {                                       // the engine's own buffer when one chunk fits it, else two slots per side from the pool
+        const size_t need = multi ? slot : (size_t) (chunks[0].j1 - chunks[0].j0) * chunks[0].w;
+        if (!multi && need <= (size_t) cap) {
+            stage_base = e->taps.as<float>(); side_stride = (size_t) cap;
+        } else {
+            staging.reset(new (std::nothrow) irbh::ScratchBuf);
+            if (!staging) return fail(IRB_ERR_ARG, "out of host memory");
+            if (int rc = staging->alloc(sizeof(float) * need * sides * (multi ? 2 : 1), false)) { cudaGetLastError(); return rc; }
+            stage_base = staging->as<float>(); side_stride = need; slot_stride = need * sides;
+        }
+        if (multi && !e->ld_ev[3]) {
+            cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+            for (auto& x : ev)
+                if (cudaEventCreateWithFlags(&x, cudaEventDisableTiming) != cudaSuccess) {
+                    for (auto y : ev) if (y) cudaEventDestroy(y);
+                    return fail(IRB_ERR_CUDA, "event creation failed: %s", cudaGetErrorString(cudaGetLastError()));
+                }
+            std::copy(ev, ev + 4, e->ld_ev);
+        }
+    }
+    if (new_tab_cap) {                                   // the old table's last reader finished with the previous load's wait
+        std::swap(e->ld_tab.p, new_tab.p);
+        e->ld_tab_cap = new_tab_cap;
+    }
+    // ---- commit the host state; nothing below allocates
+    std::vector<int> list = e->h_rr_list;
+    for (int j = 0; j < n; ++j) if (fresh[j]) list.push_back(s.ids[j]);
+    if (n_fresh) {
+        std::vector<const float*> ptrs((size_t) e->n_irs, nullptr);
+        for (int ir = 0; ir < e->n_irs; ++ir) if (e->rr_buf[ir]) ptrs[ir] = e->rr_buf[ir]->as<float>();
+        for (int j = 0; j < n; ++j) if (fresh[j]) ptrs[s.ids[j]] = bufs[j]->as<float>();
+        CK(cudaMemcpyAsync(e->rr_ptrs.p, ptrs.data(), sizeof(float*) * ptrs.size(), cudaMemcpyHostToDevice, e->stream));
+        CK(cudaMemcpyAsync(e->rr_list.p, list.data(), sizeof(int) * list.size(), cudaMemcpyHostToDevice, e->stream));
+    }
+    for (int j = 0; j < n; ++j) {
+        const int ir = s.ids[j];
+        if (fresh[j]) { e->rr_buf[ir] = std::move(bufs[j]); e->bytes += sizeof(float) * (size_t) cap; }
+        if (P[j] != e->h_nparts[ir]) e->plan_dirty = true;
+        e->h_nparts[ir] = P[j];
+    }
+    e->h_rr_list.swap(list);
+    e->ld_stage = std::move(staging);                    // held until engine_load_wait: copies and kernels read it
+    CK(cudaMemcpyAsync(e->nparts.as<int>() + lo, e->h_nparts.data() + lo, sizeof(int) * (size_t) (hi - lo + 1), cudaMemcpyHostToDevice, e->stream));
+    if (!tab.empty()) CK(cudaMemcpyAsync(e->ld_tab.p, tab.data(), sizeof(irb::IrLoadItem) * tab.size(), cudaMemcpyHostToDevice, e->stream));
+    // ---- copies and kernels
+    const cudaStream_t cs = multi ? e->s_in : e->stream;
+    for (size_t ci = 0; ci < chunks.size(); ++ci) {
+        const Chunk& c = chunks[ci];
+        const int q = (int) (ci & 1);
+        irb::IrLoadArgs a{};
+        a.items = e->ld_tab.as<irb::IrLoadItem>() + c.tab; a.n_x = (int) c.n_x; a.n_s = (int) c.n_s;
+        a.B = B; a.ring = e->ring; a.H = e->H.as<float2>(); a.ir_stride = (long long) e->ring * e->M;
+        a.h_reps = e->h_reps; a.h_rep_stride = e->h_rep_stride(); a.W = e->W;
+        a.rr_taps = e->rr_ptrs.as<float* const>(); a.rr_pos = e->rr_pos.as<int>();
+        if (on_dev) {
+            a.src = s.taps; a.src2 = s.right;
+        } else {
+            float* dst = stage_base + q * slot_stride;
+            if (multi && ci >= 2) CK(cudaStreamWaitEvent(cs, e->ld_ev[2 + q], 0));      // the transform two chunks back has read this slot
+            for (int side = 0; side < sides; ++side) {
+                const float* src = side ? s.right : s.taps;
+                float* d = dst + side * side_stride;
+                // runs of consecutive caller rows, one 2-D copy each; the caller's last row alone, at its own length
+                for (int j = c.j0; j < c.j1;) {
+                    int k = j + 1;
+                    while (pitched && k < c.j1 && s.rows[k] == s.rows[k - 1] + 1 && s.rows[k] != s.src_rows - 1) ++k;
+                    if (k == j + 1) CK(cudaMemcpyAsync(d + (size_t) (j - c.j0) * c.w, src + (long long) s.rows[j] * s.ld, sizeof(float) * len[j], cudaMemcpyHostToDevice, cs));
+                    else CK(cudaMemcpy2DAsync(d + (size_t) (j - c.j0) * c.w, sizeof(float) * c.w, src + (long long) s.rows[j] * s.ld, sizeof(float) * s.ld,
+                                              sizeof(float) * c.w, k - j, cudaMemcpyHostToDevice, cs));
+                    j = k;
+                }
+            }
+            if (multi) {
+                CK(cudaEventRecord(e->ld_ev[q], cs));
+                CK(cudaStreamWaitEvent(e->stream, e->ld_ev[q], 0));
+            }
+            a.src = dst; a.src2 = s.right ? dst + side_stride : nullptr;
+        }
+        if (c.grid > 0) {
+            if (int rc = launch_ir_load(e->M, a, c.grid, e->stream)) return rc;
+            e->launches += 1;
+        }
+        if (multi) CK(cudaEventRecord(e->ld_ev[2 + q], e->stream));
+    }
+    return 0;
+}
+// the load's work is in place: both streams drained (an early error can leave copies running on s_in), then the pooled staging
+// goes back to the pool
+int engine_load_wait(irb_engine* e) {
+    CK(cudaSetDevice(e->device));
+    const cudaError_t ci = cudaStreamSynchronize(e->s_in);
+    const cudaError_t ce = cudaStreamSynchronize(e->stream);
+    e->ld_stage.reset();
+    CK(ci);
+    CK(ce);
+    return 0;
+}
+
+int engine_load(irb_engine* e, int n, const int* ids, const float* taps, const float* right, long long ld, const int* n_taps, bool stage, int n_partitions) {
+    int rc = rows_check(n, ids, taps, ld, n_taps);
+    if (rc) return rc;
+    if (!e) return fail(IRB_ERR_ARG, "engine is null");
+    LoadSpec s;
+    s.ids.assign(ids, ids + n);
+    s.rows.resize(n);
+    for (int j = 0; j < n; ++j) s.rows[j] = j;
+    s.taps = taps; s.right = right; s.ld = ld; s.n_taps = n_taps; s.src_rows = n; s.stage = stage; s.n_partitions = n_partitions;
+    if ((rc = load_check(e, s))) return rc;
+    int loc = 0;
+    if ((rc = sources_location(taps, right, e->device, &loc))) return rc;
+    rc = engine_load_enqueue(e, s, loc == 1);
+    const int w = engine_load_wait(e);
+    return rc ? rc : w;
+}
+}  // namespace
+
+extern "C" {
+int irb_engine_set_irs(irb_engine* e, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps) {
+    return engine_load(e, n, ir_ids, taps, right, ld, n_taps, false, 0);
+}
+int irb_engine_stage_irs(irb_engine* e, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps, int n_partitions) {
+    return engine_load(e, n, ir_ids, taps, right, ld, n_taps, true, n_partitions);
+}
 
 // Streams come and go: only channels [0, n_active) take part in the following block steps (their FDL rings advance, the
 // others keep their state untouched); in/out arrays of the process calls are then [n_blocks][n_active][block_size].
@@ -1345,24 +1566,46 @@ int irb_group_channel_range(const irb_group* g, int index, int* begin, int* end)
 }
 // shared IRs (n_irs > 0): ir_id on every device.  Private IRs (n_irs == 0): ir_id is the CHANNEL whose IR this is.
 int irb_group_set_ir(irb_group* g, int ir_id, const float* left, const float* right, int n_taps) {
-    if (!g) return fail(IRB_ERR_ARG, "group is null");
-    if (g->private_irs) {
-        if (ir_id < 0 || ir_id >= g->n_chans) return fail(IRB_ERR_ARG, "channel %d outside [0, %d)", ir_id, g->n_chans);
-        const int i = g->owner(ir_id);
-        return irb_engine_set_ir(g->eng[i], ir_id - g->begin[i], left, right, n_taps);
-    }
-    for (auto* e : g->eng) { int rc = irb_engine_set_ir(e, ir_id, left, right, n_taps); if (rc) return rc; }
-    return 0;
+    return irb_group_set_irs(g, 1, &ir_id, left, right, n_taps, &n_taps);
 }
 int irb_group_stage_ir(irb_group* g, int ir_id, const float* left, const float* right, int n_taps, int n_partitions) {
+    return irb_group_stage_irs(g, 1, &ir_id, left, right, n_taps, &n_taps, n_partitions);
+}
+}  // extern "C"
+namespace {
+// rows of a private-IR group go to the device owning channel ir_ids[j] (as its local IR), rows of a shared-IR group to every
+// device; all checks first, then every device's copies and kernels, then the waits
+int group_load(irb_group* g, int n, const int* ids, const float* taps, const float* right, long long ld, const int* n_taps, bool stage, int n_partitions) {
+    int rc = rows_check(n, ids, taps, ld, n_taps);
+    if (rc) return rc;
     if (!g) return fail(IRB_ERR_ARG, "group is null");
-    if (g->private_irs) {
-        if (ir_id < 0 || ir_id >= g->n_chans) return fail(IRB_ERR_ARG, "channel %d outside [0, %d)", ir_id, g->n_chans);
-        const int i = g->owner(ir_id);
-        return irb_engine_stage_ir(g->eng[i], ir_id - g->begin[i], left, right, n_taps, n_partitions);
+    std::vector<LoadSpec> s(g->eng.size());
+    for (auto& x : s) { x.taps = taps; x.right = right; x.ld = ld; x.n_taps = n_taps; x.src_rows = n; x.stage = stage; x.n_partitions = n_partitions; }
+    for (int j = 0; j < n; ++j) {
+        if (g->private_irs) {
+            if (ids[j] < 0 || ids[j] >= g->n_chans) return fail(IRB_ERR_ARG, "ir_ids[%d]: channel %d outside [0, %d)", j, ids[j], g->n_chans);
+            const int i = g->owner(ids[j]);
+            s[i].ids.push_back(ids[j] - g->begin[i]); s[i].rows.push_back(j);
+        } else {
+            for (auto& x : s) { x.ids.push_back(ids[j]); x.rows.push_back(j); }
+        }
     }
-    for (auto* e : g->eng) { int rc = irb_engine_stage_ir(e, ir_id, left, right, n_taps, n_partitions); if (rc) return rc; }
-    return 0;
+    for (size_t i = 0; i < s.size(); ++i) if ((rc = s[i].ids.empty() ? 0 : load_check(g->eng[i], s[i]))) return rc;
+    int loc = 0;
+    if ((rc = sources_location(taps, right, g->eng[0]->device, &loc))) return rc;
+    if (loc != 0) return fail(IRB_ERR_ARG, "irb_group_* loads take host memory: the taps are device memory");
+    size_t started = 0;
+    for (; started < s.size() && !rc; ++started) rc = s[started].ids.empty() ? 0 : engine_load_enqueue(g->eng[started], s[started], false);
+    for (size_t i = 0; i < started; ++i) { const int w = s[i].ids.empty() ? 0 : engine_load_wait(g->eng[i]); if (!rc) rc = w; }
+    return rc;
+}
+}  // namespace
+extern "C" {
+int irb_group_set_irs(irb_group* g, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps) {
+    return group_load(g, n, ir_ids, taps, right, ld, n_taps, false, 0);
+}
+int irb_group_stage_irs(irb_group* g, int n, const int* ir_ids, const float* taps, const float* right, long long ld, const int* n_taps, int n_partitions) {
+    return group_load(g, n, ir_ids, taps, right, ld, n_taps, true, n_partitions);
 }
 int irb_group_bind(irb_group* g, int chan_begin, int chan_end, int ir_id) {
     if (!g) return fail(IRB_ERR_ARG, "group is null");
@@ -1413,6 +1656,7 @@ int engine_set_stamps(irb_engine* e, unsigned long long* dev) {
     e->g_sig.n_rr = -1;                // a captured graph baked the old pointer in: re-capture
     return 0;
 }
+int engine_ir_copies(const irb_engine* e) { return e ? e->h_reps : fail(IRB_ERR_ARG, "engine is null"); }
 // the pure FDL multiply-accumulate (no forward / inverse FFT) on the current state into n_channels * M complex
 int engine_mac_only(irb_engine* e, float* acc_dev) {
     if (!e || !acc_dev) return fail(IRB_ERR_ARG, "null argument");

@@ -42,6 +42,8 @@ _SIGS = {
     "irb_engine_set_stream": (ctypes.c_int, [_vp, _vp]),
     "irb_engine_set_ir": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int]),
     "irb_engine_stage_ir": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, ctypes.c_int]),
+    "irb_engine_set_irs": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, _vp, ctypes.c_longlong, _vp]),
+    "irb_engine_stage_irs": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, _vp, ctypes.c_longlong, _vp, ctypes.c_int]),
     "irb_engine_mac_plan": (ctypes.c_int, [_vp, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]),
     "irb_engine_set_mac_split": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int]),
     "irb_engine_set_fused_step": (ctypes.c_int, [_vp, ctypes.c_int]),
@@ -78,6 +80,8 @@ _SIGS = {
     "irb_group_channel_range": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]),
     "irb_group_set_ir": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int]),
     "irb_group_stage_ir": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, ctypes.c_int, ctypes.c_int]),
+    "irb_group_set_irs": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, _vp, ctypes.c_longlong, _vp]),
+    "irb_group_stage_irs": (ctypes.c_int, [_vp, ctypes.c_int, _vp, _vp, _vp, ctypes.c_longlong, _vp, ctypes.c_int]),
     "irb_group_bind": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "irb_group_reset": (ctypes.c_int, [_vp]),
     "irb_group_process": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int]),
@@ -107,6 +111,7 @@ _BENCH_SIGS = {
     "irbx_get_tuning": (ctypes.c_int, [ctypes.c_char_p]),
     "irbx_engine_mac_only_device": (ctypes.c_int, [_vp, _vp]),
     "irbx_engine_set_stamps": (ctypes.c_int, [_vp, _vp]),
+    "irbx_engine_ir_copies": (ctypes.c_int, [_vp]),
     "irbx_hbm_read_probe": (ctypes.c_int, [ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)]),
     "irbx_copy_probe_create": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_int, ctypes.c_size_t, ctypes.c_int]),
     "irbx_copy_probe_run": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_size_t, ctypes.POINTER(ctypes.c_double)]),
@@ -195,6 +200,57 @@ def _pcm_output(shape, fmt, out):
 def _planar(a):
     a = np.ascontiguousarray(a, dtype=np.float32)
     return a[None, :] if a.ndim == 1 else a
+
+
+def _ir_rows(ir_ids, taps, n_taps, right, ld, allow_ptr=True):
+    """The arguments of irb_*_set_irs / _stage_irs: -> (n, ids, taps, right, ld, n_taps, arrays to keep alive).  taps / right are
+    host arrays [n][ld] (a 1-D array is one row), or raw device pointers (ints, e.g. tensor.data_ptr()) with ld given."""
+    ids = np.ascontiguousarray(np.asarray(ir_ids, dtype=np.int64).reshape(-1), np.int32)
+    if not np.array_equal(ids, np.asarray(ir_ids, dtype=np.int64).reshape(-1)):
+        raise ValueError("ir_ids do not fit int32")
+    n = ids.size
+    if n < 1:
+        raise ValueError("ir_ids is empty: a load takes at least one row")
+    keep = [ids]
+    if isinstance(taps, (int, np.integer)):
+        if not allow_ptr:
+            raise ValueError("a group loads from host arrays only, not from a pointer")
+        if ld is None:
+            raise ValueError("ld is needed with a pointer taps")
+        if right is not None and not isinstance(right, (int, np.integer)):
+            raise ValueError("right must be a pointer too when taps is one")
+        if not taps or (right is not None and not right):
+            raise ValueError("null taps or right pointer")
+        tp, rp, ld = _vp(int(taps)), (_vp(int(right)) if right is not None else None), int(ld)
+    else:
+        t = np.ascontiguousarray(taps, np.float32)
+        t = t[None, :] if t.ndim == 1 else t
+        if t.ndim != 2 or t.shape[0] != n:
+            raise ValueError("taps must be [n][ld] with one row per IR id (%d), got shape %r" % (n, np.shape(taps)))
+        if ld is not None and int(ld) != t.shape[1]:
+            raise ValueError("ld=%r contradicts taps of shape %r" % (ld, t.shape))
+        ld = t.shape[1]
+        keep.append(t)
+        tp, rp = _ptr(t), None
+        if right is not None:
+            if isinstance(right, (int, np.integer)):
+                raise ValueError("right must be a host array when taps is one")
+            r = np.ascontiguousarray(right, np.float32)
+            r = r[None, :] if r.ndim == 1 else r
+            if r.shape != t.shape:
+                raise ValueError("right must have the shape of taps %r, got %r" % (t.shape, r.shape))
+            keep.append(r)
+            rp = _ptr(r)
+    nt = None
+    if n_taps is not None:
+        nt = np.ascontiguousarray(np.asarray(n_taps, dtype=np.int64).reshape(-1), np.int64)
+        if nt.size != n:
+            raise ValueError("n_taps needs one entry per row (%d), got %d" % (n, nt.size))
+        if nt.min() < -2**31 or nt.max() >= 2**31:
+            raise ValueError("n_taps do not fit int32")
+        nt = nt.astype(np.int32)
+        keep.append(nt)
+    return n, _ptr(ids), tp, rp, ld, (_ptr(nt) if nt is not None else None), keep
 
 
 def device_count():
@@ -541,6 +597,18 @@ class Engine:
         else:
             raise ValueError("IR must be mono or stereo")
 
+    def set_irs(self, ir_ids, taps, n_taps=None, right=None, ld=None):
+        """Load n IRs in one call (irb_engine_set_irs): row j of taps ([n][ld] host float32, or a raw device pointer with ld
+        given) holds n_taps[j] taps (default: ld) of IR ir_ids[j]; right (same kind) folds a stereo IR to (L+R)/2.  Row j's
+        spectra are exactly those of set_ir on that row."""
+        n, ids, tp, rp, ld, nt, _keep = _ir_rows(ir_ids, taps, n_taps, right, ld)
+        _ck(lib().irb_engine_set_irs(self._h, n, ids, tp, rp, ld, nt))
+
+    def stage_irs(self, ir_ids, taps, n_taps=None, right=None, ld=None, n_partitions=0):
+        """stage_ir for n IRs in one call (irb_engine_stage_irs); arguments as set_irs."""
+        n, ids, tp, rp, ld, nt, _keep = _ir_rows(ir_ids, taps, n_taps, right, ld)
+        _ck(lib().irb_engine_stage_irs(self._h, n, ids, tp, rp, ld, nt, int(n_partitions)))
+
     def mac_plan(self):
         """(slots_kernel, split_in, cluster) of the next block step's MAC launch."""
         a, b, c = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
@@ -611,6 +679,11 @@ class Engine:
     def set_stamps(self, dev_ptr):
         """bench-only: device array of 16 uint64 for the phase time stamps of the latency-path kernel (0 / None: off)"""
         _ck(lib().irbx_engine_set_stamps(self._h, _vp(int(dev_ptr or 0))))
+
+    @property
+    def ir_copies(self):
+        """bench-only: identical copies of the IR spectra the engine keeps (every load writes all of them)"""
+        return _ck(lib().irbx_engine_ir_copies(self._h))
 
     def set_active_channels(self, n_active):
         """Only channels [0, n_active) take part in the following block steps; I/O arrays are then [n_blocks][n_active][B]."""
@@ -769,6 +842,16 @@ class Group:
     def stage_ir(self, ir_id, taps, n_partitions=0):
         t = np.ascontiguousarray(_planar(taps)[0])
         _ck(lib().irb_group_stage_ir(self._h, int(ir_id), _ptr(t), None, len(t), int(n_partitions)))
+
+    def set_irs(self, ir_ids, taps, n_taps=None, right=None):
+        """irb_group_set_irs: host arrays only (taps / right [n][ld] float32); private-IR groups: ir_ids are channels."""
+        n, ids, tp, rp, ld, nt, _keep = _ir_rows(ir_ids, taps, n_taps, right, None, allow_ptr=False)
+        _ck(lib().irb_group_set_irs(self._h, n, ids, tp, rp, ld, nt))
+
+    def stage_irs(self, ir_ids, taps, n_taps=None, right=None, n_partitions=0):
+        """irb_group_stage_irs: host arrays only, as set_irs."""
+        n, ids, tp, rp, ld, nt, _keep = _ir_rows(ir_ids, taps, n_taps, right, None, allow_ptr=False)
+        _ck(lib().irb_group_stage_irs(self._h, n, ids, tp, rp, ld, nt, int(n_partitions)))
 
     def bind(self, chan_begin, chan_end, ir_id):
         _ck(lib().irb_group_bind(self._h, int(chan_begin), int(chan_end), int(ir_id)))

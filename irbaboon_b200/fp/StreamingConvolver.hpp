@@ -25,6 +25,8 @@ public:
 
     // mono IR (channel 0) or stereo IR folded to (L+R)/2, as convolvePeriodic does for mono audio
     void setIR(int irId, const AudioBuffer<float>& ir, bool foldStereo = false);
+    // many IRs in one call (irb_engine_set_irs): channel c of irs becomes IR firstId + c, each mono
+    void setIRs(int firstId, const AudioBuffer<float>& irs);
     void bind(int channelBegin, int channelEnd, int irId);
     void reset();
     // one block per call: buffer holds `channels` channels of exactly blockSize samples, processed in place
@@ -58,7 +60,8 @@ public:
     MatrixConvolver& operator=(const MatrixConvolver&) = delete;
 
     // An IR file: a mono one sets IR irId; one with ins*outs channels sets IRs irId .. irId + ins*outs - 1 from its channels
-    // (a stereo file is the {L, R} pair of a (1, 2) matrix, a four-channel file the LL, LR, RL, RR of a (2, 2) matrix)
+    // (a stereo file is the {L, R} pair of a (1, 2) matrix, a four-channel file the LL, LR, RL, RR of a (2, 2) matrix), in one
+    // irb_engine_set_irs call
     void setIR(int irId, const AudioBuffer<float>& ir);
     void bindMatrix(int groupBegin, int groupEnd, const std::vector<int>& irIds);    // irIds[i*outs + o]
     void reset();
@@ -90,6 +93,8 @@ public:
     MultiGpuConvolver(const MultiGpuConvolver&) = delete;
     MultiGpuConvolver& operator=(const MultiGpuConvolver&) = delete;
     void setIR(int irId, const AudioBuffer<float>& ir, bool foldStereo = false);
+    // many IRs in one call (irb_group_set_irs): channel c of irs becomes IR (or, with numIRs == 0, channel) firstId + c, each mono
+    void setIRs(int firstId, const AudioBuffer<float>& irs);
     void bind(int channelBegin, int channelEnd, int irId);
     void reset();
     void process(const float* in, float* out, int nBlocks);   // dense [nBlocks][channels][blockSize] host arrays

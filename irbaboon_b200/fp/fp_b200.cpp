@@ -27,6 +27,23 @@ std::vector<float> pack(const AudioBuffer<float>& b) {
     return v;
 }
 
+// the channels of an IR file as the rows [channels][ld] of irb_*_set_irs: in place when they are evenly spaced, else packed
+struct IrRows {
+    std::vector<float> packed;
+    std::vector<int> ids, taps;
+    const float* data = nullptr;
+    long long ld = 0;
+    IrRows(const AudioBuffer<float>& b, int firstId) {
+        const int ch = b.getNumChannels(), n = b.getNumSamples();
+        for (int c = 0; c < ch; ++c) { ids.push_back(firstId + c); taps.push_back(n); }
+        data = b.getReadPointer(0);
+        ld = ch > 1 ? (long long) (b.getReadPointer(1) - data) : n;
+        bool even = ld >= n;
+        for (int c = 2; c < ch && even; ++c) even = b.getReadPointer(c) - b.getReadPointer(c - 1) == ld;
+        if (!even) { packed = pack(b); data = packed.data(); ld = n; }
+    }
+};
+
 }  // namespace
 
 namespace fp {
@@ -144,6 +161,10 @@ void StreamingConvolver::setIR(int irId, const AudioBuffer<float>& ir, bool fold
     const float* r = (foldStereo && ir.getNumChannels() == 2) ? ir.getReadPointer(1) : nullptr;
     if (irb_engine_set_ir(engine, irId, ir.getReadPointer(0), r, ir.getNumSamples()) != IRB_OK) raise("irb_engine_set_ir");
 }
+void StreamingConvolver::setIRs(int firstId, const AudioBuffer<float>& irs) {
+    const IrRows r(irs, firstId);
+    if (irb_engine_set_irs(engine, (int) r.ids.size(), r.ids.data(), r.data, nullptr, r.ld, r.taps.data()) != IRB_OK) raise("irb_engine_set_irs");
+}
 void StreamingConvolver::bind(int channelBegin, int channelEnd, int irId) {
     if (irb_engine_bind(engine, channelBegin, channelEnd, irId) != IRB_OK) raise("irb_engine_bind");
 }
@@ -177,8 +198,8 @@ void MatrixConvolver::setIR(int irId, const AudioBuffer<float>& ir) {
     const int ch = ir.getNumChannels();
     if (ch != 1 && ch != ins * outs)
         throw std::invalid_argument("MatrixConvolver::setIR: an IR file has 1 channel or one per IR of the matrix (" + std::to_string(ins * outs) + ")");
-    for (int c = 0; c < ch; ++c)
-        if (irb_engine_set_ir(engine, irId + c, ir.getReadPointer(c), nullptr, ir.getNumSamples()) != IRB_OK) raise("irb_engine_set_ir");
+    const IrRows r(ir, irId);
+    if (irb_engine_set_irs(engine, ch, r.ids.data(), r.data, nullptr, r.ld, r.taps.data()) != IRB_OK) raise("irb_engine_set_irs");
 }
 void MatrixConvolver::bindMatrix(int groupBegin, int groupEnd, const std::vector<int>& irIds) {
     if ((int) irIds.size() != ins * outs) throw std::invalid_argument("MatrixConvolver::bindMatrix: one IR id per input and output (ins*outs)");
@@ -209,6 +230,10 @@ MultiGpuConvolver::~MultiGpuConvolver() { irb_group_destroy(group); }
 void MultiGpuConvolver::setIR(int irId, const AudioBuffer<float>& ir, bool foldStereo) {
     const float* r = (foldStereo && ir.getNumChannels() == 2) ? ir.getReadPointer(1) : nullptr;
     if (irb_group_set_ir(group, irId, ir.getReadPointer(0), r, ir.getNumSamples()) != IRB_OK) raise("irb_group_set_ir");
+}
+void MultiGpuConvolver::setIRs(int firstId, const AudioBuffer<float>& irs) {
+    const IrRows r(irs, firstId);
+    if (irb_group_set_irs(group, (int) r.ids.size(), r.ids.data(), r.data, nullptr, r.ld, r.taps.data()) != IRB_OK) raise("irb_group_set_irs");
 }
 void MultiGpuConvolver::bind(int channelBegin, int channelEnd, int irId) {
     if (irb_group_bind(group, channelBegin, channelEnd, irId) != IRB_OK) raise("irb_group_bind");
